@@ -285,6 +285,31 @@ def csv_decode_bench(eng, B, iters=20):
     return out
 
 
+# ------------------------------------------------------------------------------------------- outputs of the timed path
+DUMP_MAX_ROWS, DUMP_BLOCK = 32768, 1024
+
+
+def dump_outputs(eng, loss, out_dir):
+    """What the timed path hands its caller after its last step: the loss of that step (loss.npy) and the trained
+    state, every variable and optimizer slot as <name>.npy ("emb/m" -> emb.m.npy), float32.  A tensor of more than
+    DUMP_MAX_ROWS rows is stored as DUMP_MAX_ROWS / DUMP_BLOCK blocks of DUMP_BLOCK consecutive rows at offsets drawn
+    from a fixed seed, in ascending order: the same rows for every tensor of the same height and on every run (6.5 MB
+    for the default workload, about 32 MB at k = 64: under 64 MB).  Reading the state applies the optimizer steps that
+    are still deferred (dfm_flush),
+    outside the timed region.  Sharded runs store rank 0's shard."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().cpu().numpy().astype(np.float32))
+    for var in eng.variable_names():
+        for name in [var] + [var + "/" + s for s in eng.slot_names(var)]:
+            rows, _ = eng.tensor_shape(name)
+            if rows <= DUMP_MAX_ROWS:
+                a = eng.get_tensor(name)
+            else:
+                starts = np.sort(np.random.default_rng(0).choice(rows // DUMP_BLOCK, DUMP_MAX_ROWS // DUMP_BLOCK, replace=False))
+                a = np.concatenate([eng.get_tensor(name, int(s) * DUMP_BLOCK, DUMP_BLOCK) for s in starts])
+            np.save(os.path.join(out_dir, name.replace("/", ".") + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------- one measured workload
 def measure(name, args, world, rank, local, peaks, primary=True, zipf=None):
     """Times one workload on this rank's GPU (all ranks call it for the primary workload).  Returns the JSON dict on
@@ -378,6 +403,10 @@ def measure(name, args, world, rank, local, peaks, primary=True, zipf=None):
     torch.cuda.synchronize()
     last_loss = float(loss_buf.item())
     unique_rows = eng.last_unique_rows
+    if primary and not zipf and args.dump_outputs:
+        if rank == 0:
+            dump_outputs(eng, loss_buf, args.dump_outputs)
+        barrier()
 
     # ---------------- end-to-end through the host-buffer entry point (e2e)
     nh = len(packed_host)
@@ -585,6 +614,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs[2]/[1]/[0] blocks at N=1")
     ap.add_argument("--no-zipf", action="store_true", help="skip the Zipf(1.05) block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss of the last one and the trained state (large tables as a "
+                         "fixed, seeded sample of rows) to DIR/<name>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     name = args.workload or DEFAULT_WORKLOAD

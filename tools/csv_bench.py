@@ -1,5 +1,5 @@
 import sys, time, tempfile, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from recommender_tensorflow_b200.trainers import ml_100k
 from recommender_tensorflow_b200.engine import DeepFMEngine

@@ -1,5 +1,5 @@
-import ctypes as C, sys, torch
-sys.path.insert(0, "/root/repo")
+import ctypes as C, os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from recommender_tensorflow_b200 import _lib
 lib = _lib.load()
 for (M, N, K) in [(65536, 256, 384), (65536, 128, 256), (65536, 256, 128), (65536, 384, 256)]:
