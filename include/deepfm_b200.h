@@ -45,7 +45,12 @@ extern "C" {
 #define DFM_MAX_HIDDEN   8
 
 /* column kinds — tf.feature_column.categorical_column_with_* (trainers/ml_100k.py:19-35) */
-enum { DFM_COL_HASH = 0, DFM_COL_BUCKETIZED = 1, DFM_COL_VOCAB = 2, DFM_COL_IDENTITY = 3 };
+enum { DFM_COL_HASH = 0, DFM_COL_BUCKETIZED = 1, DFM_COL_VOCAB = 2, DFM_COL_IDENTITY = 3,
+       /* tf.feature_column.crossed_column: model column whose ids are sparse_cross_hashed over source columns */
+       DFM_COL_CROSSED = 4,
+       /* a raw int32 / string feature used as it is; allowed only among dfm_config.src */
+       DFM_COL_RAW = 5 };
+#define DFM_MAX_CROSS_KEYS 8   /* constituents of one crossed column */
 /* raw column dtypes — what tf.decode_csv yields (trainers/ml_100k.py:11-15,45) */
 enum { DFM_INT32 = 0, DFM_FLOAT32 = 1, DFM_STRING = 2 };
 /* optimizers — trainers/model_utils.py:57-66 */
@@ -71,6 +76,15 @@ typedef struct {
      * the present slots (embedding_column combiner='mean'), the linear term their SUM (linear_model
      * sparse_combiner='sum'); an empty bag contributes zeros.  0 or 1 = single-valued. */
     int32_t            width;
+    /* crossed column (kind DFM_COL_CROSSED, tf.feature_column.crossed_column): for every combination of one value of each
+     * constituent, id = FingerprintCat64 chain over the constituents' values seeded with hash_key, mod num_buckets
+     * (TF-1.12 sparse_cross_hashed).  keys[n_keys] index dfm_config.src in HASHING order (sparse constituents first:
+     * categorical and multivalent raw sources, then single-valued raw sources; the caller orders them, the library
+     * does not).  2 <= n_keys <= DFM_MAX_CROSS_KEYS.  hash_key 0 = TF's default 0xDECAFCAFFE.  width is derived: the
+     * product of the constituents' widths.  The column's own cat_data entry is not read and may be NULL. */
+    int32_t            n_keys;
+    const int32_t*     keys;
+    uint64_t           hash_key;
 } dfm_column;
 
 /* tf.train.*Optimizer(learning_rate) hyper-parameters (trainers/model_utils.py:57-66; TF defaults) */
@@ -106,14 +120,21 @@ typedef struct {
     /* params["activation"] (trainers/deep_fm.py:22,100; default tf.nn.relu): DFM_ACT_*.  Anything but ReLU runs the
      * general CUDA-core tower (the fused and tensor-core towers are built around the ReLU mask). */
     int32_t           activation;
+    /* source columns: the inputs of crossed columns.  Kinds DFM_COL_RAW (int32 or string value, crossed as it is; width
+     * > 1 makes it a sparse multivalent key whose -1 / '' padding slots are absent), DFM_COL_BUCKETIZED, DFM_COL_VOCAB,
+     * DFM_COL_IDENTITY.  They own no table and have no place in model order; their raw data is
+     * dfm_raw_batch.cat_data[n_cat + s] / cat_offsets[n_cat + s].  n_cat + n_src <= DFM_MAX_CAT. */
+    int32_t           n_src;
+    const dfm_column* src;
 } dfm_config;
 
 /* One batch of raw (un-hashed) feature columns = what input_fn's parse_csv yields
  * (trainers/ml_100k.py:44-49) for the columns the model consumes. */
 typedef struct {
     int32_t               batch_size;
-    const void* const*    cat_data;     /* [n_cat]: int32[B] | float32[B] | uint8 bytes (strings) */
-    const int32_t* const* cat_offsets;  /* [n_cat]: int32[B+1] byte offsets for string columns, else NULL */
+    const void* const*    cat_data;     /* [n_cat + n_src]: int32[B] | float32[B] | uint8 bytes (strings); the entry
+                                           of a crossed column is ignored (may be NULL), source columns follow cat */
+    const int32_t* const* cat_offsets;  /* [n_cat + n_src]: int32[B+1] byte offsets for string columns, else NULL */
     const float* const*   num_data;     /* [n_num]: float32[B] */
     const float*          labels;       /* [B] 0/1 (rating >= cutoff, trainers/ml_100k.py:48); NULL for forward */
 } dfm_raw_batch;

@@ -12,7 +12,8 @@ DFM_OK = 0
 ERRORS = {-1: "INVALID_ARG", -2: "CUDA", -3: "OUT_OF_RANGE", -4: "UNSUPPORTED", -5: "NCCL", -6: "NOT_FOUND", -7: "PARSE", -8: "PEER"}
 MAX_CAT, MAX_NUM, MAX_HIDDEN = 64, 64, 8
 
-COL_KIND = {"hash": 0, "bucketized": 1, "vocab": 2, "identity": 3}
+COL_KIND = {"hash": 0, "bucketized": 1, "vocab": 2, "identity": 3, "crossed": 4, "raw": 5}
+MAX_CROSS_KEYS = 8
 DTYPE = {"int32": 0, "float32": 1, "string": 2}
 OPT_KIND = {"Adam": 0, "Adagrad": 1, "Ftrl": 2, "SGD": 3, "RMSProp": 4}
 LOSS_RED = {"mean": 0, "sum": 1}
@@ -21,7 +22,8 @@ LOSS_RED = {"mean": 0, "sum": 1}
 class Column(C.Structure):
     _fields_ = [("name", C.c_char_p), ("kind", C.c_int32), ("dtype", C.c_int32), ("num_buckets", C.c_int64),
                 ("boundaries", C.POINTER(C.c_float)), ("n_boundaries", C.c_int32),
-                ("vocab", C.POINTER(C.c_char_p)), ("vocab_size", C.c_int32), ("num_oov", C.c_int32), ("width", C.c_int32)]
+                ("vocab", C.POINTER(C.c_char_p)), ("vocab_size", C.c_int32), ("num_oov", C.c_int32), ("width", C.c_int32),
+                ("n_keys", C.c_int32), ("keys", C.POINTER(C.c_int32)), ("hash_key", C.c_uint64)]
 
 
 class Optimizer(C.Structure):
@@ -35,7 +37,8 @@ class Config(C.Structure):
                 ("use_linear", C.c_int32), ("use_mf", C.c_int32), ("use_dnn", C.c_int32),
                 ("loss_reduction", C.c_int32), ("opt_deep", Optimizer), ("opt_linear", Optimizer),
                 ("max_batch", C.c_int32), ("device", C.c_int32), ("rank", C.c_int32), ("world", C.c_int32),
-                ("nccl_comm", C.c_void_p), ("dropout", C.c_float), ("dropout_seed", C.c_uint64), ("activation", C.c_int32)]
+                ("nccl_comm", C.c_void_p), ("dropout", C.c_float), ("dropout_seed", C.c_uint64), ("activation", C.c_int32),
+                ("n_src", C.c_int32), ("src", C.POINTER(Column))]
 ACTIVATIONS = {"relu": 0, "tanh": 1, "sigmoid": 2, "identity": 3, "linear": 3, None: 3}
 
 

@@ -90,6 +90,8 @@ struct HostStage {          // one in-flight host batch (double buffered)
 struct dfm_handle {
     int dc = 0, dn = 0, K = 0, L = 0;
     int dcs = 0;                 // value slots per sample = sum of column widths (== dc without multivalent columns)
+    int n_src = 0;               // source columns of crossed columns: cols[dc + s], raw data cat_data[dc + s]
+    bool has_cross = false;      // a crossed column among the model columns: transform_kernel<.., CROSS = true>
     bool has_bags = false;
     // tiny-vocabulary columns reduced densely instead of through the sort (embed_kernels.cuh: tiny_reduce_kernel)
     int n_tiny = 0, n_big = 0, n_tiny_rows = 0, tiny_blocks_max = 0, tiny_group_rows = 0;
@@ -320,8 +322,36 @@ static void free_all(dfm_handle* h) {
 extern "C" void dfm_destroy(dfm_handle* h) { free_all(h); }
 
 static int create_impl(const dfm_config* cfg, dfm_handle* h) {
-    if (cfg->n_cat < 0 || cfg->n_cat > DFM_MAX_CAT || cfg->n_num < 0 || cfg->n_num > DFM_MAX_NUM)
+    if (cfg->n_cat < 0 || cfg->n_cat > DFM_MAX_CAT || cfg->n_num < 0 || cfg->n_num > DFM_MAX_NUM || cfg->n_src < 0 ||
+        cfg->n_cat + cfg->n_src > DFM_MAX_CAT)
         FAIL(DFM_ERR_INVALID_ARG, "too many feature columns");
+    if (cfg->n_src > 0 && !cfg->src) FAIL(DFM_ERR_INVALID_ARG, "src is null");
+    // crossed columns and their sources (TF-1.12 feature_column.py crossed_column / sparse_cross_op.cc)
+    for (int s = 0; s < cfg->n_src; ++s) {
+        const dfm_column& c = cfg->src[s];
+        if (c.kind == DFM_COL_HASH)
+            FAIL(DFM_ERR_INVALID_ARG, "categorical_column_with_hash_bucket is not supported for crossing. Hashing before crossing "
+                                      "will increase probability of collision. Instead, use the feature name as a string.");
+        if (c.kind == DFM_COL_RAW && c.dtype != DFM_INT32 && c.dtype != DFM_STRING)
+            FAIL(DFM_ERR_INVALID_ARG, "a raw feature of a crossed column must be int32 or string (sparse_cross takes int64 / string)");
+        if (c.kind != DFM_COL_RAW && c.kind != DFM_COL_BUCKETIZED && c.kind != DFM_COL_VOCAB && c.kind != DFM_COL_IDENTITY)
+            FAIL(DFM_ERR_INVALID_ARG, "Unsupported key type. All keys must be either string, or categorical column except "
+                                      "_HashedCategoricalColumn.");
+    }
+    for (int f = 0; f < cfg->n_cat; ++f) {
+        const dfm_column& c = cfg->cat[f];
+        if (c.kind == DFM_COL_RAW) FAIL(DFM_ERR_INVALID_ARG, "a raw column is allowed only as a source column of a cross");
+        if (c.kind != DFM_COL_CROSSED) continue;
+        if (c.num_buckets < 1) FAIL(DFM_ERR_INVALID_ARG, "hash_bucket_size must be > 1.");
+        if (c.n_keys < 2 || !c.keys) FAIL(DFM_ERR_INVALID_ARG, "keys must be a list with length > 1.");
+        if (c.n_keys > DFM_MAX_CROSS_KEYS) FAIL(DFM_ERR_UNSUPPORTED, "a crossed column has at most 8 keys");
+        int64_t width = 1;
+        for (int i = 0; i < c.n_keys; ++i) {
+            if (c.keys[i] < 0 || c.keys[i] >= cfg->n_src) FAIL(DFM_ERR_INVALID_ARG, "crossed column key outside [0, n_src)");
+            width *= std::max(1, cfg->src[c.keys[i]].width);
+            if (width > 4 * DFM_MAX_CAT) FAIL(DFM_ERR_UNSUPPORTED, "too many value slots (sum of column widths)");
+        }
+    }
     // trainers/deep_fm.py:31-34
     if (cfg->n_cat + cfg->n_num == 0)
         FAIL(DFM_ERR_INVALID_ARG, "At least 1 feature column of categorical_columns or numeric_columns must be specified.");
@@ -369,16 +399,35 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     h->row_off.assign(h->dc + 1, 0);
     std::vector<int32_t> slot_col, slot_j, field_slot0;
     uint64_t R = 0;
-    for (int f = 0; f < h->dc; ++f) {
-        const dfm_column& c = cfg->cat[f];
+    h->n_src = cfg->n_src;
+    for (int f = 0; f < h->dc + h->n_src; ++f) {
+        const bool is_src = f >= h->dc;          // a source column: no table, no slots, no place in model order
+        const dfm_column& c = is_src ? cfg->src[f - h->dc] : cfg->cat[f];
         ColDev d{};
         d.kind = c.kind; d.dtype = c.dtype;
         d.width = std::max(1, c.width);
-        if (d.width > 1) h->has_bags = true;
-        for (int j = 0; j < d.width; ++j) { slot_col.push_back(f); slot_j.push_back(j); }
-        field_slot0.push_back((int32_t)slot_col.size() - d.width);
+        if (c.kind == DFM_COL_CROSSED) {
+            h->has_cross = true;
+            d.width = 1;
+            d.n_keys = c.n_keys;
+            d.hash_key = c.hash_key ? c.hash_key : 0xDECAFCAFFEull;     // sparse_ops.py _DEFAULT_HASH_KEY
+            for (int i = 0; i < c.n_keys && i < DFM_MAX_CROSS_KEYS; ++i) {      // n_keys was checked above
+                d.keys[i] = (uint8_t)(h->dc + c.keys[i]);
+                d.width *= std::max(1, cfg->src[c.keys[i]].width);
+            }
+        }
+        if (!is_src) {
+            if (d.width > 1) h->has_bags = true;
+            for (int j = 0; j < d.width; ++j) { slot_col.push_back(f); slot_j.push_back(j); }
+            field_slot0.push_back((int32_t)slot_col.size() - d.width);
+        }
         uint64_t nb = 0;
         switch (c.kind) {
+            case DFM_COL_CROSSED:
+                nb = (uint64_t)c.num_buckets;
+                break;
+            case DFM_COL_RAW:
+                break;
             case DFM_COL_HASH:
                 if (c.num_buckets <= 0) FAIL(DFM_ERR_INVALID_ARG, "hash column needs num_buckets > 0");
                 if (c.dtype == DFM_FLOAT32) FAIL(DFM_ERR_UNSUPPORTED, "hash column over float32 keys");
@@ -412,6 +461,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
         d.nb_rcp = nb >= 2 ? (uint64_t)(((unsigned __int128)1 << 64) / nb) : 0;
         h->cols.push_back(d);
         h->col_names.push_back(c.name ? c.name : "");
+        if (is_src) continue;
         if (R > 0xffffffffull) FAIL(DFM_ERR_UNSUPPORTED, "more than 2^32 table rows on one device");
         h->row_off[f] = (uint32_t)R;
         R += nb;
@@ -554,6 +604,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     const int64_t Bm = h->max_batch, n = Bm * std::max(h->dcs, 1);
     if (h->has_bags && dalloc(h, &h->inv_cnt, (size_t)Bm * h->dc)) return DFM_ERR_CUDA;
     CK(cudaFuncSetAttribute(transform_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
+    CK(cudaFuncSetAttribute(transform_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
     if (n >= (1ll << 31)) FAIL(DFM_ERR_UNSUPPORTED, "max_batch * n_cat must be < 2^31");
     if (dalloc(h, &h->ids, n)) return DFM_ERR_CUDA;
     if (alloc_ws(h, h->ws, n, K, h->world > 1)) return DFM_ERR_CUDA;
@@ -901,7 +952,7 @@ extern "C" int dfm_init_random(dfm_handle* h, uint64_t seed) {
 // -------------------------------------------------------------------------------- step pieces
 static BatchPtrs make_ptrs(const dfm_handle* h, const dfm_raw_batch* b) {
     BatchPtrs bp{};
-    for (int f = 0; f < h->dc; ++f) {
+    for (int f = 0; f < h->dc + h->n_src; ++f) {
         bp.cat[f] = b->cat_data ? b->cat_data[f] : nullptr;
         bp.off[f] = b->cat_offsets ? b->cat_offsets[f] : nullptr;
     }
@@ -910,11 +961,19 @@ static BatchPtrs make_ptrs(const dfm_handle* h, const dfm_raw_batch* b) {
     return bp;
 }
 
+// identity of a batch for the prefetch paths: its first raw column pointer (a crossed column has none of its own)
+static const void* batch_tag(const dfm_handle* h, const void* const* cat) {
+    for (int f = 0; f < h->dc + h->n_src; ++f)
+        if (h->cols[f].kind != DFM_COL_CROSSED) return cat[f];
+    return nullptr;
+}
+
 static int check_batch(dfm_handle* h, const dfm_raw_batch* b, bool need_labels) {
     if (!b) FAIL(DFM_ERR_INVALID_ARG, "null batch");
     if (b->batch_size <= 0 || b->batch_size > h->max_batch) FAIL(DFM_ERR_INVALID_ARG, "batch_size outside (0, max_batch]");
     if (h->dc && !b->cat_data) FAIL(DFM_ERR_INVALID_ARG, "cat_data is null");
-    for (int f = 0; f < h->dc; ++f) {
+    for (int f = 0; f < h->dc + h->n_src; ++f) {
+        if (h->cols[f].kind == DFM_COL_CROSSED) continue;           // computed from its source columns
         if (!b->cat_data[f]) FAIL(DFM_ERR_INVALID_ARG, "missing feature column: " + h->col_names[f]);
         if (h->cols[f].dtype == DFM_STRING && (!b->cat_offsets || !b->cat_offsets[f]))
             FAIL(DFM_ERR_INVALID_ARG, "missing string offsets for column: " + h->col_names[f]);
@@ -936,7 +995,7 @@ template <int K>
 static void launch_transform(dfm_handle* h, const BatchPtrs& bp, int B, bool with_keys, int32_t* ids_out, cudaStream_t st,
                              bool with_claim = false) {
     if (h->dc == 0) return;
-    transform_kernel<32><<<cdiv(B, 32), 256, (size_t)32 * h->dcs * 4, st>>>(
+    (h->has_cross ? transform_kernel<32, true> : transform_kernel<32, false>)<<<cdiv(B, 32), 256, (size_t)32 * h->dcs * 4, st>>>(
         bp, h->d_cols, h->d_bounds, h->d_voc_bytes, h->d_voc_offs, B, h->dcs, h->has_bags ? h->d_slot_col : nullptr,
         h->has_bags ? h->d_slot_j : nullptr, h->d_row_off, (uint32_t)h->R, ids_out,
         with_keys ? h->ws.keys[with_claim ? 1 : 0] : nullptr, with_keys ? h->ws.vals[with_claim ? 1 : 0] : nullptr, h->d_err,
@@ -1598,7 +1657,7 @@ static int train_fused(dfm_handle* h, const BatchPtrs& bp, int B, float* loss_ou
         const int64_t l0 = h->launches;
         const StepOpts so = step_opts(h);
         Phase ph(h, st);
-        const bool prefetched = h->prefetch_B == B && h->dc > 0 && h->prefetch_tag == bp.cat[0];
+        const bool prefetched = h->prefetch_B == B && h->dc > 0 && h->prefetch_tag == batch_tag(h, bp.cat);
         if (h->prefetch_B >= 0 && !prefetched) h->prefetch_B = -1;
         // record-staged step: once-only rows are updated inside the kernel (the claim table is filled by the transform,
         // so a prefetched batch - ids computed earlier, no claims - takes the older kernel)
@@ -1686,7 +1745,7 @@ static int train_impl(dfm_handle* h, const BatchPtrs& bp, int B, float* loss_out
     const StepOpts so = step_opts(h);
     Phase ph(h, st);
     // ids, sort and segments of this batch may have been computed ahead of time on the side stream (dfm_prefetch_batch)
-    const bool prefetched = h->prefetch_B == B && h->dc > 0 && h->prefetch_tag == bp.cat[0];
+    const bool prefetched = h->prefetch_B == B && h->dc > 0 && h->prefetch_tag == batch_tag(h, bp.cat);
     if (h->prefetch_B >= 0 && !prefetched) h->prefetch_B = -1;            // a different batch arrived: drop the prefetch
     if (prefetched) {
         CK(cudaStreamWaitEvent(st, h->ev_prefetch, 0));
@@ -1883,7 +1942,7 @@ extern "C" int dfm_prefetch_batch(dfm_handle* h, const dfm_raw_batch* b, void* a
     std::swap(h->ws, h->ws_next); std::swap(h->ids, h->ids_next);
     if (rc) return rc;
     CK(cudaEventRecord(h->ev_prefetch, h->side_stream));
-    h->prefetch_B = B; h->prefetch_tag = bp.cat[0];
+    h->prefetch_B = B; h->prefetch_tag = batch_tag(h, bp.cat);
     CK(cudaGetLastError());
     return DFM_OK;
 }
@@ -2582,7 +2641,7 @@ extern "C" int dfm_xchg_train_step_next(dfm_handle* h, const dfm_raw_batch* b, c
     CK(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     if (h->x_pf_valid) {
-        if (b->batch_size != h->x_pf_B || (h->dc > 0 && b->cat_data[0] != h->x_pf_tag))
+        if (b->batch_size != h->x_pf_B || (h->dc > 0 && batch_tag(h, b->cat_data) != h->x_pf_tag))
             FAIL(DFM_ERR_INVALID_ARG, "dfm_xchg_train_step_next: the batch announced as next_batch must be trained next");
         h->x_pf_valid = false;
         CK(cudaStreamWaitEvent(st, h->ev_xpf_done, 0));
@@ -2597,7 +2656,7 @@ extern "C" int dfm_xchg_train_step_next(dfm_handle* h, const dfm_raw_batch* b, c
         CK(cudaStreamWaitEvent(h->side_stream, h->ev_xpf_fork, 0));
         if ((rc = dfm_xchg_begin(h, next_b, h->side_stream))) return rc;
         CK(cudaEventRecord(h->ev_xpf_done, h->side_stream));
-        h->x_pf_valid = true; h->x_pf_B = next_b->batch_size; h->x_pf_tag = h->dc > 0 ? next_b->cat_data[0] : nullptr;
+        h->x_pf_valid = true; h->x_pf_B = next_b->batch_size; h->x_pf_tag = h->dc > 0 ? batch_tag(h, next_b->cat_data) : nullptr;
     }
     return DFM_OK;
 }
@@ -2610,7 +2669,8 @@ static int stage_batch(dfm_handle* h, const dfm_raw_batch* b, HostStage& sg, boo
     std::vector<Seg> segs;
     const int B = b->batch_size;
     out = BatchPtrs{};
-    for (int f = 0; f < h->dc; ++f) {
+    for (int f = 0; f < h->dc + h->n_src; ++f) {
+        if (h->cols[f].kind == DFM_COL_CROSSED) continue;          // no raw data of its own: the sources are staged
         const size_t nv = (size_t)B * h->cols[f].width;      // values of this column in the batch (multivalent: B * width)
         if (h->cols[f].dtype == DFM_STRING) {
             const int32_t* off = b->cat_offsets[f];

@@ -10,6 +10,10 @@ struct ColDev {
     uint64_t nb_rcp;        // floor(2^64 / nb) (nb >= 2; 0: use the plain modulo): fingerprint % nb without a 64-bit division
     int32_t  bnd_off, bnd_cnt;
     int32_t  voc_off, voc_cnt, num_oov, width;   // width: value slots per sample (multivalent column), >= 1
+    // crossed column: constituents = cols[keys[0..n_keys)] (source columns, hashing order), chain seeded with hash_key
+    uint64_t hash_key;
+    int32_t  n_keys;
+    uint8_t  keys[DFM_MAX_CROSS_KEYS];
 };
 
 // raw batch as kernel parameter (pointer tables by value: no H2D copy of pointer arrays)

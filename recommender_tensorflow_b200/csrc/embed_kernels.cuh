@@ -267,12 +267,64 @@ __device__ __forceinline__ int32_t transform_one(const BatchPtrs& bp, const ColD
     }
 }
 
+// Crossed column (TF-1.12 sparse_cross_hashed, reached through tf.feature_column.crossed_column): slot j of sample b is
+// one combination of constituent value slots, j read as a mixed-radix number over the constituents' widths (first key
+// most significant, the order of TF's product iterator).  f(v) per constituent, chained with FingerprintCat64 from the
+// hash key (core/kernels/sparse_cross_op.cc HashCrosser):
+//   raw string -> Fingerprint64(bytes);  raw int32 -> (uint64)(int64)v;  categorical -> (uint64)(int64)id
+// Absent values make the combination absent (-1): padding slots ('' / -1) of a multivalent raw key (a SparseTensor in
+// TF), and ids a categorical key drops (empty string, identity -1).  A single-valued raw key is a dense tensor in TF and
+// drops nothing.  A vocabulary key without OOV buckets maps an unknown string to the id -1, which TF keeps and crosses.
+// Only the CROSS instantiation of transform_kernel contains this code, so models without crossed columns run the
+// kernel as it was.  The key loop is not unrolled (transform_one is inlined into it once).
+__device__ __forceinline__ int32_t transform_cross(const BatchPtrs& bp, const ColDev* __restrict__ cols, int f, int b,
+                                                   int j, const float* __restrict__ bounds,
+                                                   const uint8_t* __restrict__ voc_bytes,
+                                                   const int32_t* __restrict__ voc_offs, int* err) {
+    const ColDev& c = cols[f];
+    uint64_t h = c.hash_key;
+    int stride = c.width;
+    const int n_keys = c.n_keys;
+#pragma unroll 1
+    for (int i = 0; i < n_keys; ++i) {
+        {
+            const int s = c.keys[i];
+            const ColDev k = cols[s];
+            stride /= k.width;
+            const int d = j / stride;
+            j -= d * stride;
+            const int vi = b * k.width + d;
+            uint64_t v;
+            if (k.kind == DFM_COL_RAW) {
+                if (k.dtype == DFM_STRING) {
+                    const int32_t* off = bp.off[s];
+                    const int a = off[vi], e = off[vi + 1];
+                    if (e <= a && k.width > 1) return -1;
+                    v = fh::fp64_mem(reinterpret_cast<const uint8_t*>(bp.cat[s]) + a, e - a);
+                } else {
+                    const int32_t x = reinterpret_cast<const int32_t*>(bp.cat[s])[vi];
+                    if (x == -1 && k.width > 1) return -1;
+                    v = (uint64_t)(int64_t)x;
+                }
+            } else {
+                if (k.kind == DFM_COL_VOCAB && bp.off[s][vi + 1] <= bp.off[s][vi]) return -1;
+                const int32_t id = transform_one(bp, k, s, vi, bounds, voc_bytes, voc_offs, err);
+                if (id < 0 && k.kind != DFM_COL_VOCAB) return -1;
+                v = (uint64_t)(int64_t)id;
+            }
+            h = fh::fp_cat64(h, v);
+        }
+    }
+    return (int32_t)mod_buckets(h, cols[f]);
+}
+
 // One block = TILE consecutive samples x all value slots (a single-valued column has one slot, a multivalent
 // column `width`).  Phase 1: work item w -> (slot w / TILE, sample w % TILE), so a warp reads 32 consecutive
 // samples of ONE column (coalesced for single-valued columns, uniform column kind) and the columns of a sample are
 // transformed in parallel by different warps (a hashed string column costs ~100x an identity column).
 // Phase 2 writes ids / keys / payload sample-major: ids [B, n_slots], payload = payload_pack(b, slot).
-template <int TILE>
+// CROSS: the model has crossed columns (transform_cross above).
+template <int TILE, bool CROSS = false>
 __global__ void __launch_bounds__(256) transform_kernel(BatchPtrs bp, const ColDev* __restrict__ cols,
                                                         const float* __restrict__ bounds,
                                                         const uint8_t* __restrict__ voc_bytes,
@@ -291,8 +343,11 @@ __global__ void __launch_bounds__(256) transform_kernel(BatchPtrs bp, const ColD
         if (t < nb) {
             const int f = slot_col ? slot_col[slot] : slot;      // null slot tables: every column single-valued
             ColDev c = cols[f];
-            const int vi = slot_col ? (b0 + t) * c.width + slot_j[slot] : b0 + t;
-            sid[t * n_slots + slot] = transform_one(bp, c, f, vi, bounds, voc_bytes, voc_offs, err);
+            const int j = slot_col ? slot_j[slot] : 0;
+            const int vi = slot_col ? (b0 + t) * c.width + j : b0 + t;
+            sid[t * n_slots + slot] = CROSS && c.kind == DFM_COL_CROSSED
+                                          ? transform_cross(bp, cols, f, b0 + t, j, bounds, voc_bytes, voc_offs, err)
+                                          : transform_one(bp, c, f, vi, bounds, voc_bytes, voc_offs, err);
         }
     }
     __syncthreads();

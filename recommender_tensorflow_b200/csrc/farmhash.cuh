@@ -168,4 +168,15 @@ __device__ __forceinline__ int itoa16(int32_t v, uint64_t& lo, uint64_t& hi) {
     return len;
 }
 
+// FingerprintCat64 (TF-1.12 core/lib/hash/hash.h): the combiner sparse_cross_hashed chains over the constituents of a
+// feature cross, h = FingerprintCat64(h, f(v)) starting from the hash key
+__device__ __forceinline__ uint64_t fp_cat64(uint64_t fp1, uint64_t fp2) {
+    constexpr uint64_t kMul = 0xc6a4a7935bd1e995ULL;
+    uint64_t r = fp1 ^ kMul;
+    r ^= smix(fp2 * kMul) * kMul;
+    r *= kMul;
+    r = smix(r) * kMul;
+    return smix(r);
+}
+
 }  // namespace fh

@@ -32,7 +32,9 @@ class GpuCsvReader:
         if engine.num_columns:
             raise ValueError("GpuCsvReader: numeric (float) model columns are not supported, the CSV schema is int32 / string")
         wanted = {}
-        for s in engine.specs:
+        for s in engine.raw_specs:          # model columns and the source columns of crossed ones
+            if s["kind"] == "crossed":
+                continue
             if s["width"] != 1:
                 raise ValueError("GpuCsvReader: multivalent column %r has no CSV encoding in the reference" % s["source"])
             wanted[s["source"]] = s["dtype"]
@@ -119,11 +121,13 @@ class GpuCsvReader:
 
     def _batch(self, n):
         eng = self.eng
-        nc = max(len(eng.specs), 1)
+        nc = max(len(eng.raw_specs), 1)
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
         num = (C.c_void_p * 1)()
-        for i, s in enumerate(eng.specs):
+        for i, s in enumerate(eng.raw_specs):
+            if s["kind"] == "crossed":
+                continue
             f = self._field[s["source"]]
             if s["dtype"] == "string":
                 cat[i] = self.lib.dfm_csv_str_bytes(self.h, f)

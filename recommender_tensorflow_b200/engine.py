@@ -35,6 +35,41 @@ def _torch():
     return torch
 
 
+def cross_spec(column, feature_dtypes=None, multivalent=None):
+    """Resolve a feature_column.CrossedColumn into the spec the library takes: the constituents become source specs in
+    HASHING order.  TF-1.12 `_CrossedColumn._transform_feature` flattens nested crosses (`_collect_leaf_level_keys`) and
+    `sparse_ops._sparse_cross_internal` hands SparseTensor inputs to the op before dense ones, keeping key order within
+    each group: categorical keys and multivalent raw keys are sparse, single-valued raw keys (decode_csv output) dense."""
+    from .feature_column import DEFAULT_HASH_KEY
+    fd, mv = dict(feature_dtypes or {}), dict(multivalent or {})
+    sparse, dense = [], []
+    for key in column.leaf_keys():
+        if isinstance(key, str):
+            if key not in fd:
+                raise ValueError("crossed_column %s: dtype of raw feature %r is unknown (pass it in feature_dtypes)"
+                                 % (column.name, key))
+            d = fd[key]
+            if d not in ("int32", "string"):
+                raise ValueError("crossed_column %s: raw feature %r is %s; sparse_cross takes only int64 and string inputs"
+                                 % (column.name, key, d))
+            s = dict(name=key, source=key, kind="raw", dtype=d, num_buckets=0, width=int(mv.get(key, 1)))
+            (sparse if s["width"] > 1 else dense).append(s)
+        else:
+            s = key.spec()
+            s["width"] = int(mv.get(s["source"], 1))
+            if s["kind"] == "bucketized":
+                s["dtype"] = fd.get(s["source"], key.source_column.dtype)
+                if s["dtype"] == "string":
+                    raise ValueError("bucketized column %s needs a numeric feature" % s["name"])
+            sparse.append(s)
+    keys = sparse + dense
+    if len(keys) > _lib.MAX_CROSS_KEYS:
+        raise ValueError("crossed_column %s: %d keys, at most %d are supported" % (column.name, len(keys), _lib.MAX_CROSS_KEYS))
+    width = int(np.prod([k["width"] for k in keys]))
+    return dict(name=column.name, source=None, kind="crossed", dtype=None, num_buckets=int(column.hash_bucket_size),
+                hash_key=int(column.hash_key or DEFAULT_HASH_KEY), keys=keys, width=width)
+
+
 class PackedBatch:
     """Raw feature columns of one batch laid out back to back in one arena (host pinned or device)."""
 
@@ -73,24 +108,41 @@ class DeepFMEngine:
         fd = dict(feature_dtypes or {})
         mv = dict(multivalent or {})      # raw feature key -> value slots per sample (multi-hot / multivalent column)
         self.specs = []
+        # source columns of crossed columns (deduplicated); their raw data follows the model columns' in a batch
+        self.src_specs = []
         for c in cats:
+            if c.kind == "crossed":
+                s = cross_spec(c, fd, mv)
+                s["key_idx"] = []
+                for k in s["keys"]:
+                    if k not in self.src_specs:
+                        self.src_specs.append(k)
+                    s["key_idx"].append(self.src_specs.index(k))
+                self.specs.append(s)
+                continue
             s = c.spec()
             s["width"] = int(mv.get(s["source"], 1))
             if s["kind"] == "bucketized":
                 s["dtype"] = fd.get(s["source"], c.source_column.dtype)
             self.specs.append(s)
+        # every raw column a batch carries, in cat_data order: model columns (a crossed one has none), then sources
+        self.raw_specs = self.specs + self.src_specs
         self.num_buckets = [int(s["num_buckets"]) for s in self.specs]
         self.n_slots = sum(s["width"] for s in self.specs)
         self.row_offsets = np.concatenate([[0], np.cumsum(self.num_buckets)]).astype(np.int64)
         self._keep = []
         cols = (_lib.Column * max(len(cats), 1))()
-        for i, s in enumerate(self.specs):
-            col = cols[i]
+        srcs = (_lib.Column * max(len(self.src_specs), 1))()
+        for col, s in list(zip(cols, self.specs)) + list(zip(srcs, self.src_specs)):
             col.name = s["name"].encode()
             col.kind = _lib.COL_KIND[s["kind"]]
-            col.dtype = _lib.DTYPE[s["dtype"]]
+            col.dtype = _lib.DTYPE[s["dtype"] or "int32"]
             col.num_buckets = s["num_buckets"]
             col.width = s["width"]
+            if s["kind"] == "crossed":
+                arr = (C.c_int32 * len(s["key_idx"]))(*s["key_idx"])
+                self._keep.append(arr)
+                col.n_keys, col.keys, col.hash_key = len(s["key_idx"]), C.cast(arr, C.POINTER(C.c_int32)), s["hash_key"]
             if s["kind"] == "bucketized":
                 arr = (C.c_float * len(s["boundaries"]))(*s["boundaries"])
                 self._keep.append(arr)
@@ -107,8 +159,8 @@ class DeepFMEngine:
                           C.cast(hid, C.POINTER(C.c_int32)), int(self.use_linear), int(self.use_mf), int(self.use_dnn),
                           _lib.LOSS_RED[loss_reduction], _opt_struct(self.opt_deep), _opt_struct(self.opt_linear),
                           self.max_batch, self.device, self.rank, self.world, None, self.dropout, self.dropout_seed,
-                          _lib.ACTIVATIONS[self.activation])
-        self._keep += [cols, hid]
+                          _lib.ACTIVATIONS[self.activation], len(self.src_specs), C.cast(srcs, C.POINTER(_lib.Column)))
+        self._keep += [cols, srcs, hid]
         handle = C.c_void_p()
         rc = self.lib.dfm_create(C.byref(cfg), C.byref(handle))
         if rc != _lib.DFM_OK:
@@ -360,7 +412,9 @@ class DeepFMEngine:
         """-> list of (kind, index, ndarray) in arena order; kind in cat|off|num|lab."""
         segs = []
         B = None
-        for f, s in enumerate(self.specs):
+        for f, s in enumerate(self.raw_specs):
+            if s["kind"] == "crossed":
+                continue
             raw = features[s["source"]]
             if s["dtype"] == "string":
                 if isinstance(raw, tuple):
@@ -425,7 +479,7 @@ class DeepFMEngine:
             arena, base = host, host.data_ptr()
         else:
             arena, base = hv, hv.ctypes.data
-        nc, nn = max(len(self.specs), 1), max(len(self.num_columns), 1)
+        nc, nn = max(len(self.raw_specs), 1), max(len(self.num_columns), 1)
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
         num = (C.c_void_p * nn)()
@@ -448,7 +502,7 @@ class DeepFMEngine:
     def repack_like(self, pb, arena):
         """A PackedBatch over another arena (torch uint8 tensor, host pinned or device) with pb's column layout."""
         base = arena.data_ptr()
-        nc, nn = max(len(self.specs), 1), max(len(self.num_columns), 1)
+        nc, nn = max(len(self.raw_specs), 1), max(len(self.num_columns), 1)
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
         num = (C.c_void_p * nn)()

@@ -85,6 +85,40 @@ class IdentityCategoricalColumn(namedtuple("IdentityCategoricalColumn", ["key", 
         return dict(name=self.name, source=self.key, kind="identity", dtype="int32", num_buckets=self.num_buckets)
 
 
+class CrossedColumn(namedtuple("CrossedColumn", ["keys", "hash_bucket_size", "hash_key"]), _Cat):
+    """tf.feature_column.crossed_column (TF-1.12 feature_column.py `_CrossedColumn`).  Its ids are
+    sparse_cross_hashed(inputs, num_buckets=hash_bucket_size, hash_key=hash_key or DEFAULT_HASH_KEY) over the
+    Cartesian product of the constituents' bags; the engine resolves the keys into source columns
+    (engine.cross_spec) and the transform runs on the device."""
+    kind = "crossed"
+
+    def leaf_keys(self):
+        """`_collect_leaf_level_keys`: nested crosses flattened, key order kept."""
+        out = []
+        for k in self.keys:
+            out += k.leaf_keys() if isinstance(k, CrossedColumn) else [k]
+        return out
+
+    @property
+    def name(self):
+        return "_X_".join(sorted(k if isinstance(k, str) else k.name for k in self.leaf_keys()))
+
+    @property
+    def num_buckets(self):
+        return self.hash_bucket_size
+
+    @property
+    def source(self):
+        return None
+
+    def spec(self):
+        raise TypeError("a crossed column is resolved against the raw feature dtypes: use engine.cross_spec")
+
+
+# sparse_ops.sparse_cross_hashed's default hash_key (TF-1.12 python/ops/sparse_ops.py `_DEFAULT_HASH_KEY`)
+DEFAULT_HASH_KEY = 0xDECAFCAFFE
+
+
 class EmbeddingColumn(namedtuple("EmbeddingColumn", ["categorical_column", "dimension"])):
     @property
     def name(self):
@@ -140,6 +174,25 @@ def categorical_column_with_identity(key, num_buckets, default_value=None):
     if num_buckets < 1:
         raise ValueError("num_buckets {} < 1, column_name {}".format(num_buckets, key))
     return IdentityCategoricalColumn(key, int(num_buckets))
+
+
+def crossed_column(keys, hash_bucket_size, hash_key=None):
+    """TF-1.12 tf.feature_column.crossed_column, with its argument checks and messages."""
+    if not hash_bucket_size or hash_bucket_size < 1:
+        raise ValueError("hash_bucket_size must be > 1. hash_bucket_size: {}".format(hash_bucket_size))
+    if not keys or len(keys) < 2:
+        raise ValueError("keys must be a list with length > 1. Given: {}".format(keys))
+    for key in keys:
+        if not isinstance(key, (str, _Cat)):
+            raise ValueError("Unsupported key type. All keys must be either string, or categorical column except "
+                             "_HashedCategoricalColumn. Given: {}".format(key))
+        if isinstance(key, HashedCategoricalColumn):
+            raise ValueError("categorical_column_with_hash_bucket is not supported for crossing. Hashing before crossing "
+                             "will increase probability of collision. Instead, use the feature name as a string. "
+                             "Given: {}".format(key))
+    if hash_key is not None and not 0 <= int(hash_key) < 1 << 64:
+        raise ValueError("hash_key must be a uint64. Given: {}".format(hash_key))
+    return CrossedColumn(tuple(keys), int(hash_bucket_size), None if hash_key is None else int(hash_key))
 
 
 def embedding_column(categorical_column, dimension):
