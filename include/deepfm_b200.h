@@ -85,6 +85,21 @@ typedef struct {
     int32_t            n_keys;
     const int32_t*     keys;
     uint64_t           hash_key;
+    /* vocabulary column, packed (tf.feature_column.categorical_column_with_vocabulary_list / _file).  dtype DFM_STRING:
+     * entry j is the bytes vocab_data[vocab_offsets[j] .. vocab_offsets[j + 1]) (vocab_offsets has vocab_size + 1
+     * monotone entries, total bytes < 2^31); used when `vocab` is NULL.  dtype DFM_INT32: vocab_int[vocab_size] int64
+     * keys, matched against the sign-extended raw value (-1 is dropped before the lookup).  vocab_size >= 1.  A lookup
+     * probes a device hash table keyed on the 64-bit fingerprint (strings: Fingerprint64, confirmed by a byte compare)
+     * or on the key itself (ints); on duplicated entries the first occurrence wins. */
+    const uint8_t*     vocab_data;
+    const int64_t*     vocab_offsets;
+    const int64_t*     vocab_int;
+    /* has_default != 0: vocabulary column - an unknown key maps to default_value (-1 = dropped, else in
+     * [0, vocab_size); not together with num_oov > 0); identity column - a value outside [0, num_buckets) maps to
+     * default_value (in [0, num_buckets)) instead of failing with DFM_ERR_OUT_OF_RANGE.  0: unknown vocabulary keys
+     * are dropped (-1), out-of-range identity values are an error. */
+    int64_t            default_value;
+    int32_t            has_default;
 } dfm_column;
 
 /* tf.train.*Optimizer(learning_rate) hyper-parameters (trainers/model_utils.py:57-66; TF defaults) */

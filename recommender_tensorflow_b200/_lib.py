@@ -23,7 +23,9 @@ class Column(C.Structure):
     _fields_ = [("name", C.c_char_p), ("kind", C.c_int32), ("dtype", C.c_int32), ("num_buckets", C.c_int64),
                 ("boundaries", C.POINTER(C.c_float)), ("n_boundaries", C.c_int32),
                 ("vocab", C.POINTER(C.c_char_p)), ("vocab_size", C.c_int32), ("num_oov", C.c_int32), ("width", C.c_int32),
-                ("n_keys", C.c_int32), ("keys", C.POINTER(C.c_int32)), ("hash_key", C.c_uint64)]
+                ("n_keys", C.c_int32), ("keys", C.POINTER(C.c_int32)), ("hash_key", C.c_uint64),
+                ("vocab_data", C.c_void_p), ("vocab_offsets", C.POINTER(C.c_int64)), ("vocab_int", C.POINTER(C.c_int64)),
+                ("default_value", C.c_int64), ("has_default", C.c_int32)]
 
 
 class Optimizer(C.Structure):

@@ -113,6 +113,8 @@ struct dfm_handle {
     Table tb{};               // one record per row: w | {lin w, s1, s2, last_step} | slot1 | slot2 (dfm_types.cuh)
 
     ColDev* d_cols = nullptr; float* d_bounds = nullptr; uint8_t* d_voc_bytes = nullptr; int32_t* d_voc_offs = nullptr;
+    longlong2* d_vtab = nullptr;     // hash tables of the table-looked-up vocabulary columns, back to back
+    bool has_vtab = false;           // such a column exists: transform_kernel<.., VTAB = true>
     uint32_t* d_row_off = nullptr;
 
     std::vector<DenseT> dense;
@@ -278,7 +280,7 @@ static int64_t pad32(int64_t x) { return (x + 31) / 32 * 32; }
 static void free_all(dfm_handle* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    void* ptrs[] = {h->d_cols, h->d_bounds, h->d_voc_bytes, h->d_voc_offs, h->d_row_off, h->tb.rec, h->dw,
+    void* ptrs[] = {h->d_cols, h->d_bounds, h->d_voc_bytes, h->d_voc_offs, h->d_vtab, h->d_row_off, h->tb.rec, h->dw,
                     h->ds1, h->ds2, h->dg, h->ids, h->h0, h->s, h->zacc, h->logits, h->dz, h->dE, h->splitk, h->colpart, h->head_part,
                     h->d_loss, h->d_dzsum, h->d_err, h->num_partial, h->num_scratch, h->fused_done, h->claim, h->once_lk, h->sum_h0, h->sum_s, h->sum_lin, h->sum_mf, h->sum_hidden, h->sum_dnn, h->sum_logits, h->sum_limits, h->sum_stats, h->sum_buckets, h->up_partial, h->w0_partial, h->tc_w, h->head_gpart, h->d_slot_col, h->d_slot_j, h->d_field_slot0, h->inv_cnt, h->uidx,
                     h->req_rows, h->d_counts};
@@ -321,6 +323,125 @@ static void free_all(dfm_handle* h) {
 
 extern "C" void dfm_destroy(dfm_handle* h) { free_all(h); }
 
+// String vocabularies up to this size are scanned (embed_kernels.cuh transform_one); larger ones, and every integer
+// vocabulary, are looked up through a hash table (vocab_probe).  DFM_VOCAB_PATH=scan|table forces string vocabularies
+// onto one path (A/B runs and tests).
+constexpr int VOCAB_SCAN_MAX = 8;
+
+static const uint8_t* vocab_entry(const dfm_column& c, int j, int64_t* len) {
+    if (c.vocab) { *len = (int64_t)strlen(c.vocab[j]); return reinterpret_cast<const uint8_t*>(c.vocab[j]); }
+    *len = c.vocab_offsets[j + 1] - c.vocab_offsets[j];
+    return c.vocab_data + c.vocab_offsets[j];
+}
+
+// vocabulary and identity columns (cat and src), before any CUDA call (TF-1.12 feature_column.py argument checks where
+// TF has one)
+static int check_vocab_columns(const dfm_config* cfg, dfm_handle* h) {
+    int64_t total = 0;
+    for (int f = 0; f < cfg->n_cat + cfg->n_src; ++f) {
+        const dfm_column& c = f < cfg->n_cat ? cfg->cat[f] : cfg->src[f - cfg->n_cat];
+        const std::string nm = c.name ? c.name : "";
+        if (c.kind == DFM_COL_IDENTITY && c.has_default && (c.default_value < 0 || c.default_value >= c.num_buckets))
+            FAIL(DFM_ERR_INVALID_ARG, "default_value " + std::to_string(c.default_value) + " not in range [0, " +
+                                          std::to_string(c.num_buckets) + "), column_name " + nm);
+        if (c.kind != DFM_COL_VOCAB) continue;
+        if (c.vocab_size < 1) FAIL(DFM_ERR_INVALID_ARG, "vocabulary column " + nm + " needs vocab_size >= 1");
+        if (c.num_oov < 0) FAIL(DFM_ERR_INVALID_ARG, "Invalid num_oov_buckets " + std::to_string(c.num_oov) + " in " + nm + ".");
+        const bool str_voc = c.vocab || c.vocab_data || c.vocab_offsets;
+        if (c.dtype == DFM_STRING) {
+            if (!str_voc && c.vocab_int) FAIL(DFM_ERR_INVALID_ARG, "dtype string and vocabulary dtype int64 do not match in " + nm);
+            if (!c.vocab && !(c.vocab_data && c.vocab_offsets))
+                FAIL(DFM_ERR_INVALID_ARG, "string vocabulary column " + nm + " needs vocab or vocab_data + vocab_offsets");
+            if (!c.vocab) {
+                if (c.vocab_offsets[0] < 0) FAIL(DFM_ERR_INVALID_ARG, "vocab_offsets of " + nm + " must start at >= 0");
+                for (int j = 0; j < c.vocab_size; ++j)
+                    if (c.vocab_offsets[j + 1] < c.vocab_offsets[j]) FAIL(DFM_ERR_INVALID_ARG, "vocab_offsets of " + nm + " are not monotone");
+            }
+            for (int j = 0; j < c.vocab_size; ++j) {
+                int64_t len;
+                vocab_entry(c, j, &len);
+                total += len;
+            }
+            if (total > 0x7fffffffll)
+                FAIL(DFM_ERR_UNSUPPORTED, "string vocabularies hold more than 2^31 - 1 bytes (int32 device offsets)");
+        } else if (c.dtype == DFM_INT32) {
+            if (!c.vocab_int && str_voc) FAIL(DFM_ERR_INVALID_ARG, "dtype int32 and vocabulary dtype string do not match in " + nm);
+            if (!c.vocab_int) FAIL(DFM_ERR_INVALID_ARG, "integer vocabulary column " + nm + " needs vocab_int");
+        } else {
+            FAIL(DFM_ERR_UNSUPPORTED, "vocabulary column " + nm + " needs string or int32 input");
+        }
+        if (c.has_default) {
+            if (c.num_oov > 0) FAIL(DFM_ERR_INVALID_ARG, "Can't specify both num_oov_buckets and default_value in " + nm + ".");
+            if (c.default_value != -1 && (c.default_value < 0 || c.default_value >= c.vocab_size))
+                FAIL(DFM_ERR_INVALID_ARG, "default_value " + std::to_string(c.default_value) + " of " + nm +
+                                              " must be -1 or in [0, vocab_size)");
+        }
+    }
+    return DFM_OK;
+}
+
+// Hash tables of the table-looked-up vocabulary columns (vocab_probe): capacity = the power of two >= 2 V, placement on
+// the host in vocabulary order (a deterministic layout; a repeated entry keeps its first index).  String fingerprints
+// are computed on the device by the function the probe uses.
+static int build_vocab_tables(dfm_handle* h, const dfm_config* cfg, const std::vector<int>& vt_cols) {
+    if (vt_cols.empty()) return DFM_OK;
+    const char* bits_env = getenv("DFM_VOCAB_FP_BITS");
+    const int fp_bits = bits_env ? atoi(bits_env) : 64;
+    const uint64_t fp_mask = fp_bits >= 64 || fp_bits <= 0 ? ~0ull : (1ull << fp_bits) - 1;
+    std::vector<uint64_t> base;
+    uint64_t total = 0;
+    for (int f : vt_cols) {
+        uint64_t cap = 2;
+        while (cap < 2ull * (uint64_t)h->cols[f].voc_cnt) cap <<= 1;
+        base.push_back(total);
+        total += cap;
+    }
+    std::vector<longlong2> tab(total, make_longlong2(0, -1));
+    std::vector<uint64_t> keys;
+    uint64_t* d_fp = nullptr;
+    for (size_t t = 0; t < vt_cols.size(); ++t) {
+        const int f = vt_cols[t];
+        ColDev& d = h->cols[f];
+        const dfm_column& c = f < h->dc ? cfg->cat[f] : cfg->src[f - h->dc];
+        const int V = d.voc_cnt;
+        keys.resize(V);
+        if (d.dtype == DFM_STRING) {
+            if (dalloc(h, &d_fp, (size_t)V)) return DFM_ERR_CUDA;
+            fingerprint_kernel<<<cdiv(V, 256), 256>>>(h->d_voc_bytes, h->d_voc_offs + d.voc_off, V, d_fp);
+            CK(cudaGetLastError());
+            CK(cudaMemcpy(keys.data(), d_fp, (size_t)V * 8, cudaMemcpyDeviceToHost));
+            CK(cudaFree(d_fp));
+            d_fp = nullptr;
+            for (auto& k : keys) k &= fp_mask;
+            d.fp_mask = fp_mask;
+        } else {
+            for (int j = 0; j < V; ++j) keys[j] = (uint64_t)c.vocab_int[j];
+            d.fp_mask = ~0ull;
+        }
+        const uint64_t mask = (base.size() > t + 1 ? base[t + 1] : total) - base[t] - 1;
+        longlong2* T = tab.data() + base[t];
+        for (int j = 0; j < V; ++j) {
+            uint64_t i = vocab_mix(keys[j]) & mask;
+            bool dup = false;
+            for (; T[i].y >= 0; i = (i + 1) & mask) {
+                if ((uint64_t)T[i].x != keys[j]) continue;
+                if (d.dtype != DFM_STRING) { dup = true; break; }
+                int64_t la, lb;
+                const uint8_t* a = vocab_entry(c, (int)T[i].y, &la);
+                const uint8_t* b = vocab_entry(c, j, &lb);
+                if (la == lb && memcmp(a, b, (size_t)la) == 0) { dup = true; break; }
+            }
+            if (!dup) T[i] = make_longlong2((long long)keys[j], j);
+        }
+        d.tab_mask = (uint32_t)mask;
+    }
+    if (dalloc(h, &h->d_vtab, (size_t)total)) return DFM_ERR_CUDA;
+    CK(cudaMemcpy(h->d_vtab, tab.data(), total * sizeof(longlong2), cudaMemcpyHostToDevice));
+    for (size_t t = 0; t < vt_cols.size(); ++t) h->cols[vt_cols[t]].vtab = h->d_vtab + base[t];
+    h->has_vtab = true;
+    return DFM_OK;
+}
+
 static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     if (cfg->n_cat < 0 || cfg->n_cat > DFM_MAX_CAT || cfg->n_num < 0 || cfg->n_num > DFM_MAX_NUM || cfg->n_src < 0 ||
         cfg->n_cat + cfg->n_src > DFM_MAX_CAT)
@@ -352,6 +473,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
             if (width > 4 * DFM_MAX_CAT) FAIL(DFM_ERR_UNSUPPORTED, "too many value slots (sum of column widths)");
         }
     }
+    if (int rc = check_vocab_columns(cfg, h)) return rc;
     // trainers/deep_fm.py:31-34
     if (cfg->n_cat + cfg->n_num == 0)
         FAIL(DFM_ERR_INVALID_ARG, "At least 1 feature column of categorical_columns or numeric_columns must be specified.");
@@ -398,6 +520,8 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     std::vector<int32_t> voc_offs;
     h->row_off.assign(h->dc + 1, 0);
     std::vector<int32_t> slot_col, slot_j, field_slot0;
+    std::vector<int> vt_cols;        // vocabulary columns looked up through a hash table
+    const char* vpath = getenv("DFM_VOCAB_PATH");
     uint64_t R = 0;
     h->n_src = cfg->n_src;
     for (int f = 0; f < h->dc + h->n_src; ++f) {
@@ -405,6 +529,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
         const dfm_column& c = is_src ? cfg->src[f - h->dc] : cfg->cat[f];
         ColDev d{};
         d.kind = c.kind; d.dtype = c.dtype;
+        d.dflt = -1;
         d.width = std::max(1, c.width);
         if (c.kind == DFM_COL_CROSSED) {
             h->has_cross = true;
@@ -436,6 +561,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
             case DFM_COL_IDENTITY:
                 if (c.num_buckets <= 0) FAIL(DFM_ERR_INVALID_ARG, "identity column needs num_buckets > 0");
                 if (c.dtype != DFM_INT32) FAIL(DFM_ERR_UNSUPPORTED, "identity column needs int32 input");
+                if (c.has_default) d.dflt = (int32_t)c.default_value;      // range checked by check_vocab_columns
                 nb = (uint64_t)c.num_buckets;
                 break;
             case DFM_COL_BUCKETIZED:
@@ -444,15 +570,21 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                 for (int j = 0; j < c.n_boundaries; ++j) bounds.push_back(c.boundaries[j]);
                 nb = (uint64_t)c.n_boundaries + 1;
                 break;
-            case DFM_COL_VOCAB:
-                if (c.dtype != DFM_STRING) FAIL(DFM_ERR_UNSUPPORTED, "vocabulary column needs string input");
+            case DFM_COL_VOCAB:       // checked by check_vocab_columns
                 d.voc_off = (int)voc_offs.size(); d.voc_cnt = c.vocab_size; d.num_oov = c.num_oov;
-                for (int j = 0; j < c.vocab_size; ++j) {
+                d.dflt = c.has_default ? (int32_t)c.default_value : -1;
+                if (c.dtype == DFM_STRING) {
+                    for (int j = 0; j < c.vocab_size; ++j) {
+                        voc_offs.push_back((int32_t)voc_bytes.size());
+                        int64_t len;
+                        const uint8_t* p = vocab_entry(c, j, &len);
+                        voc_bytes.insert(voc_bytes.end(), p, p + len);
+                    }
                     voc_offs.push_back((int32_t)voc_bytes.size());
-                    size_t len = strlen(c.vocab[j]);
-                    voc_bytes.insert(voc_bytes.end(), c.vocab[j], c.vocab[j] + len);
                 }
-                voc_offs.push_back((int32_t)voc_bytes.size());
+                if (c.dtype != DFM_STRING || (vpath && !strcmp(vpath, "table")) ||
+                    (!(vpath && !strcmp(vpath, "scan")) && c.vocab_size > VOCAB_SCAN_MAX))
+                    vt_cols.push_back(f);
                 nb = (uint64_t)c.vocab_size + (uint64_t)c.num_oov;
                 break;
             default: FAIL(DFM_ERR_INVALID_ARG, "unknown column kind");
@@ -491,10 +623,11 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     if (dalloc(h, &h->d_voc_bytes, voc_bytes.size())) return DFM_ERR_CUDA;
     if (dalloc(h, &h->d_voc_offs, voc_offs.size())) return DFM_ERR_CUDA;
     if (dalloc(h, &h->d_row_off, h->row_off.size())) return DFM_ERR_CUDA;
-    if (!h->cols.empty()) CK(cudaMemcpy(h->d_cols, h->cols.data(), h->cols.size() * sizeof(ColDev), cudaMemcpyHostToDevice));
     if (!bounds.empty()) CK(cudaMemcpy(h->d_bounds, bounds.data(), bounds.size() * 4, cudaMemcpyHostToDevice));
     if (!voc_bytes.empty()) CK(cudaMemcpy(h->d_voc_bytes, voc_bytes.data(), voc_bytes.size(), cudaMemcpyHostToDevice));
     if (!voc_offs.empty()) CK(cudaMemcpy(h->d_voc_offs, voc_offs.data(), voc_offs.size() * 4, cudaMemcpyHostToDevice));
+    if (int rc = build_vocab_tables(h, cfg, vt_cols)) return rc;
+    if (!h->cols.empty()) CK(cudaMemcpy(h->d_cols, h->cols.data(), h->cols.size() * sizeof(ColDev), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(h->d_row_off, h->row_off.data(), h->row_off.size() * 4, cudaMemcpyHostToDevice));
     {
         const char* env = getenv("DFM_TINY");
@@ -605,6 +738,8 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     if (h->has_bags && dalloc(h, &h->inv_cnt, (size_t)Bm * h->dc)) return DFM_ERR_CUDA;
     CK(cudaFuncSetAttribute(transform_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
     CK(cudaFuncSetAttribute(transform_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
+    CK(cudaFuncSetAttribute(transform_kernel<32, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
+    CK(cudaFuncSetAttribute(transform_kernel<32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 4 * DFM_MAX_CAT * 4));
     if (n >= (1ll << 31)) FAIL(DFM_ERR_UNSUPPORTED, "max_batch * n_cat must be < 2^31");
     if (dalloc(h, &h->ids, n)) return DFM_ERR_CUDA;
     if (alloc_ws(h, h->ws, n, K, h->world > 1)) return DFM_ERR_CUDA;
@@ -995,7 +1130,8 @@ template <int K>
 static void launch_transform(dfm_handle* h, const BatchPtrs& bp, int B, bool with_keys, int32_t* ids_out, cudaStream_t st,
                              bool with_claim = false) {
     if (h->dc == 0) return;
-    (h->has_cross ? transform_kernel<32, true> : transform_kernel<32, false>)<<<cdiv(B, 32), 256, (size_t)32 * h->dcs * 4, st>>>(
+    (h->has_vtab ? (h->has_cross ? transform_kernel<32, true, true> : transform_kernel<32, false, true>)
+                 : (h->has_cross ? transform_kernel<32, true> : transform_kernel<32, false>))<<<cdiv(B, 32), 256, (size_t)32 * h->dcs * 4, st>>>(
         bp, h->d_cols, h->d_bounds, h->d_voc_bytes, h->d_voc_offs, B, h->dcs, h->has_bags ? h->d_slot_col : nullptr,
         h->has_bags ? h->d_slot_j : nullptr, h->d_row_off, (uint32_t)h->R, ids_out,
         with_keys ? h->ws.keys[with_claim ? 1 : 0] : nullptr, with_keys ? h->ws.vals[with_claim ? 1 : 0] : nullptr, h->d_err,

@@ -14,7 +14,20 @@ struct ColDev {
     uint64_t hash_key;
     int32_t  n_keys;
     uint8_t  keys[DFM_MAX_CROSS_KEYS];
+    // vocabulary: id of an unknown key (-1 = dropped).  identity: id of a value outside [0, nb), -1 = error
+    int32_t  dflt;
+    // vocabulary looked up through its hash table (vtab != nullptr): capacity tab_mask + 1 slots, power of two >= 2 V
+    uint32_t tab_mask;
+    const longlong2* vtab;  // slot = {key (string: fingerprint & fp_mask, int: the int64 value), vocabulary index or -1 = empty}
+    uint64_t fp_mask;       // ~0; fewer bits only to test the byte comparison (DFM_VOCAB_FP_BITS)
 };
+
+// probe start of a vocabulary hash-table key: fixed 64-bit mixer (splitmix64 finaliser), the same on host and device
+__host__ __device__ __forceinline__ uint64_t vocab_mix(uint64_t k) {
+    k ^= k >> 30; k *= 0xbf58476d1ce4e5b9ull;
+    k ^= k >> 27; k *= 0x94d049bb133111ebull;
+    return k ^ (k >> 31);
+}
 
 // raw batch as kernel parameter (pointer tables by value: no H2D copy of pointer arrays)
 struct BatchPtrs {

@@ -214,6 +214,54 @@ __device__ __forceinline__ uint64_t mod_buckets(uint64_t h, const ColDev& c) {
     uint64_t r = h - __umul64hi(h, c.nb_rcp) * c.nb;
     return r >= c.nb ? r - c.nb : r;
 }
+// Vocabulary lookup through the column's open-addressing table (TF-1.12 index_table_from_tensor / _from_file: a HashTable
+// from key to index, unknown keys -> OOV bucket or default_value).  Slot = {key, index}; string keys are their
+// Fingerprint64 (the OOV bucket needs it anyway) and a fingerprint match is confirmed by comparing the bytes, so the
+// result is exact; int keys are the sign-extended value.  Linear probing from vocab_mix(key); the table is at most half
+// full, so a probe ends at an empty slot.
+__device__ __forceinline__ int32_t vocab_probe(const BatchPtrs& bp, const ColDev& c, int f, int b,
+                                            const uint8_t* __restrict__ voc_bytes, const int32_t* __restrict__ voc_offs) {
+    uint64_t key, fp = 0;
+    const uint8_t* p = nullptr;
+    int len = 0;
+    if (c.dtype == DFM_STRING) {
+        const int32_t* off = bp.off[f];
+        const int s = off[b];
+        len = off[b + 1] - s;
+        if (len <= 0) return -1;
+        p = reinterpret_cast<const uint8_t*>(bp.cat[f]) + s;
+        fp = fh::fp64_mem(p, len);
+        key = fp & c.fp_mask;
+    } else {
+        const int32_t v = reinterpret_cast<const int32_t*>(bp.cat[f])[b];
+        if (v == -1) return -1;
+        key = (uint64_t)(int64_t)v;
+    }
+    for (uint32_t i = (uint32_t)vocab_mix(key) & c.tab_mask;; i = (i + 1) & c.tab_mask) {
+        const longlong2 e = __ldg(c.vtab + i);
+        if (e.y < 0) break;
+        if ((uint64_t)e.x != key) continue;
+        if (c.dtype != DFM_STRING) return (int32_t)e.y;
+        const int vs = voc_offs[c.voc_off + (int)e.y], ve = voc_offs[c.voc_off + (int)e.y + 1];
+        if (ve - vs != len) continue;
+        bool eq = true;
+        for (int q = 0; q < len && eq; ++q) eq = voc_bytes[vs + q] == p[q];
+        if (eq) return (int32_t)e.y;
+    }
+    if (c.num_oov > 0) {
+        if (c.dtype != DFM_STRING) {        // AsString(key), as the hashed int column does
+            uint64_t lo, hi;
+            const int n = fh::itoa16((int32_t)(int64_t)key, lo, hi);
+            fp = fh::fp64_short(lo, hi, n);
+        }
+        return c.voc_cnt + (int32_t)(fp % (uint64_t)c.num_oov);
+    }
+    return c.dflt;
+}
+
+// VTAB: the model has vocabulary columns looked up through a hash table (vocab_probe); otherwise every vocabulary
+// column is a short string list and is scanned.
+template <bool VTAB>
 __device__ __forceinline__ int32_t transform_one(const BatchPtrs& bp, const ColDev& c, int f, int b,
                                                  const float* __restrict__ bounds,
                                                  const uint8_t* __restrict__ voc_bytes,
@@ -243,6 +291,7 @@ __device__ __forceinline__ int32_t transform_one(const BatchPtrs& bp, const ColD
             return cnt;
         }
         case DFM_COL_VOCAB: {
+            if (VTAB && c.vtab) return vocab_probe(bp, c, f, b, voc_bytes, voc_offs);
             const int32_t* off = bp.off[f];
             int s = off[b], e = off[b + 1];
             int len = e - s;
@@ -256,12 +305,15 @@ __device__ __forceinline__ int32_t transform_one(const BatchPtrs& bp, const ColD
                 if (eq) return j;
             }
             if (c.num_oov > 0) return c.voc_cnt + (int32_t)(fh::fp64_mem(p, len) % (uint64_t)c.num_oov);
-            return -1;
+            return c.dflt;
         }
         default: {  // identity
             int32_t v = reinterpret_cast<const int32_t*>(bp.cat[f])[b];
             if (v == -1) return -1;
-            if (v < 0 || (uint64_t)v >= c.nb) { atomicOr(err, 1); return -1; }
+            if (v < 0 || (uint64_t)v >= c.nb) {
+                if (c.dflt >= 0) return c.dflt;      // default_value
+                atomicOr(err, 1); return -1;
+            }
             return v;
         }
     }
@@ -277,6 +329,7 @@ __device__ __forceinline__ int32_t transform_one(const BatchPtrs& bp, const ColD
 // drops nothing.  A vocabulary key without OOV buckets maps an unknown string to the id -1, which TF keeps and crosses.
 // Only the CROSS instantiation of transform_kernel contains this code, so models without crossed columns run the
 // kernel as it was.  The key loop is not unrolled (transform_one is inlined into it once).
+template <bool VTAB>
 __device__ __forceinline__ int32_t transform_cross(const BatchPtrs& bp, const ColDev* __restrict__ cols, int f, int b,
                                                    int j, const float* __restrict__ bounds,
                                                    const uint8_t* __restrict__ voc_bytes,
@@ -307,8 +360,10 @@ __device__ __forceinline__ int32_t transform_cross(const BatchPtrs& bp, const Co
                     v = (uint64_t)(int64_t)x;
                 }
             } else {
-                if (k.kind == DFM_COL_VOCAB && bp.off[s][vi + 1] <= bp.off[s][vi]) return -1;
-                const int32_t id = transform_one(bp, k, s, vi, bounds, voc_bytes, voc_offs, err);
+                if (k.kind == DFM_COL_VOCAB && (k.dtype == DFM_STRING ? bp.off[s][vi + 1] <= bp.off[s][vi]
+                                                                      : reinterpret_cast<const int32_t*>(bp.cat[s])[vi] == -1))
+                    return -1;
+                const int32_t id = transform_one<VTAB>(bp, k, s, vi, bounds, voc_bytes, voc_offs, err);
                 if (id < 0 && k.kind != DFM_COL_VOCAB) return -1;
                 v = (uint64_t)(int64_t)id;
             }
@@ -323,8 +378,8 @@ __device__ __forceinline__ int32_t transform_cross(const BatchPtrs& bp, const Co
 // samples of ONE column (coalesced for single-valued columns, uniform column kind) and the columns of a sample are
 // transformed in parallel by different warps (a hashed string column costs ~100x an identity column).
 // Phase 2 writes ids / keys / payload sample-major: ids [B, n_slots], payload = payload_pack(b, slot).
-// CROSS: the model has crossed columns (transform_cross above).
-template <int TILE, bool CROSS = false>
+// CROSS: the model has crossed columns (transform_cross above).  VTAB: it has hash-table vocabularies (vocab_probe).
+template <int TILE, bool CROSS = false, bool VTAB = false>
 __global__ void __launch_bounds__(256) transform_kernel(BatchPtrs bp, const ColDev* __restrict__ cols,
                                                         const float* __restrict__ bounds,
                                                         const uint8_t* __restrict__ voc_bytes,
@@ -346,8 +401,8 @@ __global__ void __launch_bounds__(256) transform_kernel(BatchPtrs bp, const ColD
             const int j = slot_col ? slot_j[slot] : 0;
             const int vi = slot_col ? (b0 + t) * c.width + j : b0 + t;
             sid[t * n_slots + slot] = CROSS && c.kind == DFM_COL_CROSSED
-                                          ? transform_cross(bp, cols, f, b0 + t, j, bounds, voc_bytes, voc_offs, err)
-                                          : transform_one(bp, c, f, vi, bounds, voc_bytes, voc_offs, err);
+                                          ? transform_cross<VTAB>(bp, cols, f, b0 + t, j, bounds, voc_bytes, voc_offs, err)
+                                          : transform_one<VTAB>(bp, c, f, vi, bounds, voc_bytes, voc_offs, err);
         }
     }
     __syncthreads();

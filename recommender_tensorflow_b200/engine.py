@@ -70,6 +70,17 @@ def cross_spec(column, feature_dtypes=None, multivalent=None):
                 hash_key=int(column.hash_key or DEFAULT_HASH_KEY), keys=keys, width=width)
 
 
+def pack_vocabulary(vocab, dtype):
+    """A vocabulary as dfm_column takes it: strings -> (uint8 bytes, int64 offsets[V + 1]), ints -> int64[V]."""
+    if dtype != "string":
+        return np.ascontiguousarray(np.array(vocab, dtype=np.int64))
+    enc = [v if isinstance(v, bytes) else v.encode() for v in vocab]
+    offsets = np.zeros(len(enc) + 1, dtype=np.int64)
+    np.cumsum(np.fromiter(map(len, enc), dtype=np.int64, count=len(enc)), out=offsets[1:])
+    data = np.frombuffer(b"".join(enc) or b"\0", dtype=np.uint8)
+    return data, offsets
+
+
 class PackedBatch:
     """Raw feature columns of one batch laid out back to back in one arena (host pinned or device)."""
 
@@ -149,11 +160,17 @@ class DeepFMEngine:
                 col.boundaries = C.cast(arr, C.POINTER(C.c_float))
                 col.n_boundaries = len(s["boundaries"])
             if s["kind"] == "vocab":
-                arr = (C.c_char_p * len(s["vocab"]))(*[v.encode() for v in s["vocab"]])
-                self._keep.append(arr)
-                col.vocab = C.cast(arr, C.POINTER(C.c_char_p))
+                packed = pack_vocabulary(s["vocab"], s["dtype"])
+                self._keep.append(packed)
+                if s["dtype"] == "string":
+                    col.vocab_data = packed[0].ctypes.data
+                    col.vocab_offsets = packed[1].ctypes.data_as(C.POINTER(C.c_int64))
+                else:
+                    col.vocab_int = packed.ctypes.data_as(C.POINTER(C.c_int64))
                 col.vocab_size = len(s["vocab"])
                 col.num_oov = s["num_oov"]
+            if s["kind"] in ("vocab", "identity") and s.get("default_value") not in (None, -1):
+                col.default_value, col.has_default = int(s["default_value"]), 1
         hid = (C.c_int32 * max(len(self.hidden), 1))(*self.hidden)
         cfg = _lib.Config(len(cats), C.cast(cols, C.POINTER(_lib.Column)), len(nums), self.k, len(self.hidden),
                           C.cast(hid, C.POINTER(C.c_int32)), int(self.use_linear), int(self.use_mf), int(self.use_dnn),

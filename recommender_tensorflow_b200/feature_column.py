@@ -2,7 +2,10 @@
 reference uses them (trainers/ml_100k.py:18-39).  They are plain descriptors: all arithmetic
 (hashing, bucketizing, vocabulary lookup, embedding) happens in the CUDA library.
 """
+import os
 from collections import namedtuple
+
+import numpy as np
 
 
 class _Cat:
@@ -58,7 +61,9 @@ class BucketizedColumn(namedtuple("BucketizedColumn", ["source_column", "boundar
 
 
 class VocabularyListCategoricalColumn(
-        namedtuple("VocabularyListCategoricalColumn", ["key", "vocabulary_list", "num_oov_buckets"]), _Cat):
+        namedtuple("VocabularyListCategoricalColumn", ["key", "vocabulary_list", "num_oov_buckets", "dtype", "default_value"],
+                   defaults=("string", -1)), _Cat):
+    """dtype "string": vocabulary_list holds str; "int32": int keys (int64 range).  default_value -1 = dropped."""
     kind = "vocab"
 
     @property
@@ -70,11 +75,32 @@ class VocabularyListCategoricalColumn(
         return len(self.vocabulary_list) + self.num_oov_buckets
 
     def spec(self):
-        return dict(name=self.name, source=self.key, kind="vocab", dtype="string", vocab=list(self.vocabulary_list),
-                    num_oov=self.num_oov_buckets, num_buckets=self.num_buckets)
+        return dict(name=self.name, source=self.key, kind="vocab", dtype=self.dtype, vocab=list(self.vocabulary_list),
+                    num_oov=self.num_oov_buckets, default_value=self.default_value, num_buckets=self.num_buckets)
 
 
-class IdentityCategoricalColumn(namedtuple("IdentityCategoricalColumn", ["key", "num_buckets"]), _Cat):
+class VocabularyFileCategoricalColumn(
+        namedtuple("VocabularyFileCategoricalColumn",
+                   ["key", "vocabulary_file", "vocabulary_size", "num_oov_buckets", "default_value", "dtype"]), _Cat):
+    """The file is read when the engine resolves the column (spec()), as TF reads it at table initialisation."""
+    kind = "vocab"
+
+    @property
+    def name(self):
+        return self.key
+
+    @property
+    def num_buckets(self):
+        return self.vocabulary_size + self.num_oov_buckets
+
+    def spec(self):
+        vocab = read_vocabulary_file(self.vocabulary_file, self.vocabulary_size, self.dtype, self.key)
+        return dict(name=self.name, source=self.key, kind="vocab", dtype=self.dtype, vocab=vocab,
+                    num_oov=self.num_oov_buckets, default_value=self.default_value, num_buckets=self.num_buckets)
+
+
+class IdentityCategoricalColumn(namedtuple("IdentityCategoricalColumn", ["key", "num_buckets", "default_value"],
+                                           defaults=(None,)), _Cat):
     kind = "identity"
 
     @property
@@ -82,7 +108,8 @@ class IdentityCategoricalColumn(namedtuple("IdentityCategoricalColumn", ["key", 
         return self.key
 
     def spec(self):
-        return dict(name=self.name, source=self.key, kind="identity", dtype="int32", num_buckets=self.num_buckets)
+        return dict(name=self.name, source=self.key, kind="identity", dtype="int32", num_buckets=self.num_buckets,
+                    default_value=self.default_value)
 
 
 class CrossedColumn(namedtuple("CrossedColumn", ["keys", "hash_bucket_size", "hash_key"]), _Cat):
@@ -161,19 +188,141 @@ def bucketized_column(source_column, boundaries):
     return BucketizedColumn(source_column, tuple(float(x) for x in b))
 
 
+def _vocab_default(default_value, vocabulary_size, key):
+    """default_value of a vocabulary column: -1 (dropped) or a vocabulary index.  TF does not check it and would gather
+    outside the table; here anything else is rejected."""
+    d = -1 if default_value is None else int(default_value)
+    if d != -1 and not 0 <= d < vocabulary_size:
+        raise ValueError("default_value {} must be -1 or in [0, {}), column_name: {}".format(default_value, vocabulary_size, key))
+    return d
+
+
+def _vocab_dtype_name(dtype, prefix):
+    """fc_utils.assert_string_or_int: string or integer, integer raw features are int32 here."""
+    try:
+        d = _dtype_name(dtype)
+    except ValueError:
+        d = None
+    if d not in ("string", "int32"):
+        raise ValueError("{} dtype must be string or integer. dtype: {}.".format(prefix, dtype))
+    return d
+
+
 def categorical_column_with_vocabulary_list(key, vocabulary_list, dtype=None, default_value=-1, num_oov_buckets=0):
-    if not vocabulary_list:
+    """TF-1.12 tf.feature_column.categorical_column_with_vocabulary_list.  The vocabulary dtype is inferred from the
+    list as np.array(vocabulary_list).dtype does; a repeated entry keeps its first index (TF's duplicate check is not
+    reproduced)."""
+    if vocabulary_list is None or len(vocabulary_list) < 1:
         raise ValueError("vocabulary_list {} must be non-empty, column_name: {}".format(vocabulary_list, key))
+    if num_oov_buckets:
+        if default_value != -1:
+            raise ValueError("Can't specify both num_oov_buckets and default_value in {}.".format(key))
     if num_oov_buckets < 0:
         raise ValueError("Invalid num_oov_buckets {} in {}.".format(num_oov_buckets, key))
-    vocab = tuple(v.decode() if isinstance(v, bytes) else str(v) for v in vocabulary_list)
-    return VocabularyListCategoricalColumn(key, vocab, int(num_oov_buckets))
+    # np.array(vocabulary_list).dtype without materialising the array: all integers -> int64, all str / bytes -> string
+    if all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in vocabulary_list):
+        vocab_dtype, vocab_np = "int32", "int64"
+    elif all(isinstance(v, (str, bytes, np.str_, np.bytes_)) for v in vocabulary_list):
+        vocab_dtype, vocab_np = "string", "string"
+    else:
+        raise ValueError("column_name: {} vocabulary dtype must be string or integer. dtype: {}.".format(
+            key, np.array(vocabulary_list).dtype))
+    if dtype is None:
+        d = vocab_dtype
+    else:
+        d = _vocab_dtype_name(dtype, "column_name: {}".format(key))
+        if d != vocab_dtype:
+            raise ValueError("dtype {} and vocabulary dtype {} do not match, column_name: {}".format(dtype, vocab_np, key))
+    if d == "string":
+        vocab = tuple(v.decode() if isinstance(v, bytes) else str(v) for v in vocabulary_list)
+    else:
+        vocab = tuple(int(v) for v in vocabulary_list)
+        if any(not -(1 << 63) <= v < 1 << 63 for v in vocab):
+            raise ValueError("column_name: {} vocabulary holds a value outside int64".format(key))
+    return VocabularyListCategoricalColumn(key, vocab, int(num_oov_buckets), d,
+                                           _vocab_default(default_value, len(vocab), key))
+
+
+def categorical_column_with_vocabulary_file(key, vocabulary_file, vocabulary_size=None, num_oov_buckets=0,
+                                            default_value=None, dtype="string"):
+    """TF-1.12 tf.feature_column.categorical_column_with_vocabulary_file: one key per line (read_vocabulary_file)."""
+    if not vocabulary_file:
+        raise ValueError("Missing vocabulary_file in {}.".format(key))
+    if vocabulary_size is None:
+        if not os.path.exists(vocabulary_file):
+            raise ValueError("vocabulary_file in {} does not exist.".format(key))
+        with open(vocabulary_file, "rb") as f:
+            data = f.read()
+        vocabulary_size = len(_split_lines(data))
+    if vocabulary_size < 1:
+        raise ValueError("Invalid vocabulary_size in {}.".format(key))
+    if num_oov_buckets:
+        if default_value is not None:
+            raise ValueError("Can't specify both num_oov_buckets and default_value in {}.".format(key))
+        if num_oov_buckets < 0:
+            raise ValueError("Invalid num_oov_buckets {} in {}.".format(num_oov_buckets, key))
+    d = _vocab_dtype_name(dtype, "column_name: {} vocabulary".format(key))
+    return VocabularyFileCategoricalColumn(key, vocabulary_file, int(vocabulary_size),
+                                           0 if num_oov_buckets is None else int(num_oov_buckets),
+                                           _vocab_default(default_value, int(vocabulary_size), key), d)
+
+
+def _split_lines(data):
+    """io::InputBuffer::ReadLine over a whole file: lines end at '\n' (not part of the line), a trailing '\r' is
+    removed, a last line without '\n' counts, nothing follows a final '\n'."""
+    lines = data.split(b"\n")
+    if lines[-1] == b"":
+        lines.pop()
+    return [ln[:-1] if ln.endswith(b"\r") else ln for ln in lines]
+
+
+_SPACE = b" \t\n\v\f\r"
+
+
+def _strto64(b):
+    """strings::safe_strto64: surrounding whitespace allowed, an optional '-', decimal digits only, int64 range."""
+    s = b.strip(_SPACE)
+    digits = s[1:] if s.startswith(b"-") else s
+    if not digits or not digits.isdigit():
+        return None
+    v = int(s)
+    return v if -(1 << 63) <= v < (1 << 63) else None
+
+
+def read_vocabulary_file(path, vocabulary_size, dtype, key):
+    """The first vocabulary_size keys of a vocabulary file, as index_table_from_file / TextFileLineIterator reads them
+    (TF-1.12): bytes for dtype "string", int for "int32" (each line parsed as int64).  Fewer lines than vocabulary_size,
+    a repeated key or an unparsable integer line is a ValueError, as the table initialisation fails in TF."""
+    with open(path, "rb") as f:
+        lines = _split_lines(f.read())
+    if len(lines) < vocabulary_size:
+        raise ValueError("Invalid vocab_size in {}: vocabulary_size = {} but file {} has {} lines.".format(
+            key, vocabulary_size, path, len(lines)))
+    lines = lines[:vocabulary_size]
+    if dtype == "string":
+        vocab = lines
+    else:
+        vocab = []
+        for i, ln in enumerate(lines):
+            v = _strto64(ln)
+            if v is None:
+                raise ValueError("Field {!r} in line {} of {} is not a valid int64 (column {}).".format(ln, i, path, key))
+            vocab.append(v)
+    seen = set()
+    for i, v in enumerate(vocab):
+        if v in seen:
+            raise ValueError("HashTable has different value for same key. Key {!r} (line {} of {}, column {}) repeats an "
+                             "earlier line.".format(v, i, path, key))
+        seen.add(v)
+    return vocab
 
 
 def categorical_column_with_identity(key, num_buckets, default_value=None):
     if num_buckets < 1:
         raise ValueError("num_buckets {} < 1, column_name {}".format(num_buckets, key))
-    return IdentityCategoricalColumn(key, int(num_buckets))
+    if default_value is not None and (default_value < 0 or default_value >= num_buckets):
+        raise ValueError("default_value {} not in range [0, {}), column_name {}".format(default_value, num_buckets, key))
+    return IdentityCategoricalColumn(key, int(num_buckets), None if default_value is None else int(default_value))
 
 
 def crossed_column(keys, hash_bucket_size, hash_key=None):
