@@ -860,7 +860,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                 // record-staged variant: the shapes BASELINE.json names (k = 16, first hidden layer 16), unsharded
                 const int rs = K + 4 + h->emb_slots * K;
                 if (fused_rows_supported(K, m.H[0], h->dc, h->dn) && h->world > 1 && !h->has_bags && h->dropout == 0.f && h->need_emb &&
-                    getenv("DFM_NO_FUSED_ROWS") == nullptr && getenv("DFM_NO_STAGED_APPLY") == nullptr) {
+                    getenv("DFM_NO_FUSED_ROWS") == nullptr) {
                     h->fr_smem_rb = fused_rows_smem_bytes(m, K, h->dc, h->dn, K + 4);
                     if (h->fr_smem_rb <= 227 * 1024) {
                         h->fused_rows_rb = true;
@@ -1573,6 +1573,11 @@ static int tower_backward(dfm_handle* h, const BatchPtrs& bp, int B, float scale
     return DFM_OK;
 }
 
+template <int K, bool BAGS>
+static StageSrcPlain<K, BAGS> stage_src(const GradSrc<K, BAGS>& src) { StageSrcPlain<K, BAGS> s{}; s.s = src; return s; }
+template <typename SRC>
+static SRC stage_src(const SRC& src) { return src; }
+
 // deterministic segmented reduction of the sparse gradients (+ optimizer, or gradient rows out when gsum != nullptr)
 template <int K, typename SRC>
 static int sparse_update(dfm_handle* h, SegWS& ws, int64_t n, const SRC& src, const OptDev& od, const OptDev& ol, int64_t t,
@@ -1584,51 +1589,28 @@ static int sparse_update(dfm_handle* h, SegWS& ws, int64_t n, const SRC& src, co
         h->launches += 2;
     }
     if (ph) ph->next();
-    // rows are rewritten here: the non-lazy Adam decay they skipped since their last write is replayed first (to step t-1)
-    constexpr bool kBags = std::is_same<SRC, GradSrc<K, true>>::value;
-    static const bool staged_ok = getenv("DFM_NO_STAGED_APPLY") == nullptr;
-    if (!gsum && !route && !kBags && staged_ok) {
-        // table records + first gradient operand staged by cp.async, a few iterations ahead (row_apply.cuh)
-        if constexpr (std::is_same<SRC, GradSrc<K, false>>::value) {
-            using S2 = StageSrcPlain<K>;
-            static bool attr = false;
-            if (!attr) { CK(cudaFuncSetAttribute(row_apply_kernel<K, S2>, cudaFuncAttributeMaxDynamicSharedMemorySize, RowApplyCfg<K, S2>::SMEM)); attr = true; }
-            S2 s2{}; s2.s = src;
-            row_apply_kernel<K, S2><<<n > 0 ? (unsigned)h->sm_count * 2 : 1, 256, RowApplyCfg<K, S2>::SMEM, st>>>(
-                ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0, ws.piece_start, ws.seg_cnt, s2, ws.piece_sum, h->tb, h->emb_slots, od, ol,
-                (bool)h->need_emb, (bool)h->use_linear, (int)t, make_rr(h, t - 1));
-        } else if constexpr (!kBags) {
-            const int smem = RowApplyCfg<K, SRC>::SMEM + src.aux_floats() * 4;
-            if (smem > 200 * 1024) FAIL(DFM_ERR_UNSUPPORTED, "internal: staged sparse apply does not fit in shared memory");
-            static int attr = 0;
-            if (attr < smem) { CK(cudaFuncSetAttribute(row_apply_kernel<K, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr = smem; }
-            row_apply_kernel<K, SRC><<<n > 0 ? (unsigned)h->sm_count * 2 : 1, 256, smem, st>>>(
-                ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0, ws.piece_start, ws.seg_cnt, src, ws.piece_sum, h->tb, h->emb_slots, od, ol,
-                (bool)h->need_emb, (bool)h->use_linear, (int)t, make_rr(h, t - 1));
-        }
-    } else if (gsum && route && !kBags && staged_ok) {
-        // requester side of the fused exchange: staged gradient operands, rows leave as coalesced stores over NVLink
-        if constexpr (std::is_same<SRC, GradSrc<K, false>>::value) {
-            using S2 = StageSrcPlain<K>;
-            const int smem = RowGsumCfg<K, S2>::SMEM;
-            static int attr = 0;
-            if (attr < smem) { CK(cudaFuncSetAttribute(row_gsum_kernel<K, S2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr = smem; }
-            S2 s2{}; s2.s = src;
-            row_gsum_kernel<K, S2><<<n > 0 ? (unsigned)h->sm_count * 2 : 1, 256, smem, st>>>(ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0,
-                                                                                           ws.piece_start, ws.seg_cnt, s2, ws.piece_sum, route, h->fr_rb_live);
-        } else if constexpr (!kBags) {
-            const int smem = RowGsumCfg<K, SRC>::SMEM + src.aux_floats() * 4;
-            if (smem > 200 * 1024) FAIL(DFM_ERR_UNSUPPORTED, "internal: staged gradient-row kernel does not fit in shared memory");
-            static int attr = 0;
-            if (attr < smem) { CK(cudaFuncSetAttribute(row_gsum_kernel<K, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr = smem; }
-            row_gsum_kernel<K, SRC><<<n > 0 ? (unsigned)h->sm_count * 2 : 1, 256, smem, st>>>(ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0,
-                                                                                            ws.piece_start, ws.seg_cnt, src, ws.piece_sum, route, h->fr_rb_live);
-        }
+    // gradient operands of the first lookup of every row (and, applying, the table records) staged by cp.async a few
+    // iterations ahead (row_apply.cuh); the plain sources gain the staging interface, the fused one has it
+    using S = decltype(stage_src(src));
+    const S ss = stage_src(src);
+    const unsigned grid = n > 0 ? (unsigned)h->sm_count * 2 : 1;
+    if (!gsum) {
+        // rows are rewritten here: the non-lazy Adam decay they skipped since their last write is replayed first (to step t-1)
+        const int smem = RowApplyCfg<K, S>::SMEM + ss.aux_floats() * 4;
+        if (smem > 200 * 1024) FAIL(DFM_ERR_UNSUPPORTED, "internal: staged sparse apply does not fit in shared memory");
+        static int attr = 0;
+        if (attr < smem) { CK(cudaFuncSetAttribute(row_apply_kernel<K, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr = smem; }
+        row_apply_kernel<K, S><<<grid, 256, smem, st>>>(ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0, ws.piece_start, ws.seg_cnt, ss,
+                                                        ws.piece_sum, h->tb, h->emb_slots, od, ol, (bool)h->need_emb, (bool)h->use_linear,
+                                                        (int)t, make_rr(h, t - 1));
     } else {
-        row_update_kernel<K, SRC><<<n > 0 ? row_grid : 1, 256, 0, st>>>(ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0, ws.piece_start, ws.seg_cnt, src,
-                                                                   ws.piece_sum, h->tb, h->emb_slots, od, ol, (bool)h->need_emb,
-                                                                   (bool)h->use_linear, (int)t, make_rr(h, gsum ? -1 : t - 1), gsum, K + 4, route,
-                                                                   h->fr_rb_live && gsum && !route);
+        // requester side of the sharded step: gradient rows into gsum (collectives) or over NVLink into the owners' segments
+        const int smem = RowGsumCfg<K, S>::SMEM + ss.aux_floats() * 4;
+        if (smem > 200 * 1024) FAIL(DFM_ERR_UNSUPPORTED, "internal: staged gradient-row kernel does not fit in shared memory");
+        static int attr = 0;
+        if (attr < smem) { CK(cudaFuncSetAttribute(row_gsum_kernel<K, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr = smem; }
+        row_gsum_kernel<K, S><<<grid, 256, smem, st>>>(ws.urow, ws.uval, ws.svals(), ws.row_start, ws.row_piece0, ws.piece_start, ws.seg_cnt, ss,
+                                                       ws.piece_sum, route, gsum, h->fr_rb_live);
     }
     h->launches++;
     if (ph) ph->next();

@@ -1057,204 +1057,29 @@ __global__ void __launch_bounds__(256) piece_reduce_kernel(const uint32_t* __res
     }
 }
 
-// level 2 + optimizer: one lane group per unique row.  Rows with <= DIRECT_T lookups sum their
-// gradients straight from dE in sorted (= sample) order; hot rows sum their piece sums in order.
-// Then the sparse optimizer step for that row (Adam: rows were caught up to t-1 beforehand).
-template <int K>
-__host__ __device__ constexpr int rt_tile_floats() { return 8 * (32 / (K / 4)) * (K + 4); }   // 8 warps x rows per warp x row width
-
-template <int K, typename SRC>
-__global__ void __launch_bounds__(256) row_update_kernel(const uint32_t* __restrict__ urow, const uint32_t* __restrict__ uval,
-                                                         const uint32_t* __restrict__ svals,
-                                                         const uint32_t* __restrict__ row_start,
-                                                         const uint32_t* __restrict__ row_piece0,
-                                                         const uint32_t* __restrict__ piece_start,
-                                                         const SegCounts* __restrict__ cnt, SRC src,
-                                                         const float* __restrict__ piece_sum,
-                                                         Table tb, int emb_slots, OptDev od, OptDev ol,
-                                                         bool has_emb, bool has_lin, int step, RowReplay rr,
-                                                         float* __restrict__ gsum_out, int gsum_stride,
-                                                         const PeerRoute* __restrict__ rt, bool skip_single = false) {
-    // skip_single: rows with exactly one lookup were already written by fused_rows_kernel (row-buffer mode)
-    constexpr int LPR = K / 4;
-    const int sub = threadIdx.x % LPR;
-    const uint32_t gpb = blockDim.x / LPR;
-    const ReplayStep rs = replay_step_load(rr.rd.closed ? rr.rd : rr.rl, rr.upto);
-    const uint32_t U = cnt->n_rows;
-    // row mapping: within one trip the lane groups of a warp take rows n_warps apart
-    const uint32_t TG = gridDim.x * gpb, gid = blockIdx.x * gpb + threadIdx.x / LPR;
-    const uint32_t gpw = 32 / LPR, n_warps = TG / gpw;
-    // fused exchange (rt): consecutive rows go to consecutive addresses of one peer, so there the warp keeps
-    // consecutive rows and emits them as one contiguous store through shared memory
-    const uint32_t uoff = rt ? gid : (gid % gpw) * n_warps + gid / gpw;
-    __shared__ __align__(16) float gtile[rt_tile_floats<K>()];
-    for (uint32_t ubase = 0; ubase < U; ubase += TG) {   // block-uniform trip count
-        const uint32_t u = ubase + uoff;
-        bool coop = false;
-        bool act = u < U;
-        uint32_t beg = 0, end = 0, row = 0, v0 = 0xffffffffu;
-        if (act) { beg = row_start[u]; end = row_start[u + 1]; row = __ldg(urow + u); v0 = __ldg(uval + u); }
-        if (skip_single && end - beg == 1) { act = false; end = beg; }
-        // issue the table-record loads now: they only depend on the row id and overlap the gradient gather below
-        float4 w = make_float4(0.f, 0.f, 0.f, 0.f), s1 = w, s2 = w, lr = w;
-        if (act && !gsum_out) {
-            if (has_emb) {
-                w = tab_w(tb, row)[sub];
-                if (emb_slots >= 1) s1 = tab_s1(tb, row)[sub];
-                if (emb_slots >= 2) s2 = tab_s2(tb, row)[sub];
-            }
-            lr = *tab_lin(tb, row);        // every lane of the group (one broadcast load): last_step drives the replay
-        }
-        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-        float gl = 0.f;
-        if (!act) {
-        } else if (end - beg <= (uint32_t)DIRECT_T) {
-            src.fetch(v0, sub, sub == 0, g, gl);      // first lookup of the row: its payload came with the row id
-            for (uint32_t i = beg + 1; i < end; i += 4) {
-                uint32_t v[4];
-                float4 t[4];
-                float tl[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v[q] = (i + q < end) ? __ldg(svals + i + q) : 0xffffffffu;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    tl[q] = 0.f;
-                    if (v[q] != 0xffffffffu) src.fetch(v[q], sub, sub == 0, t[q], tl[q]);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-            }
-        } else {
-            uint32_t p0 = row_piece0[u], p1 = row_piece0[u + 1];
-            if (p1 - p0 > (uint32_t)COOP_PIECES) {
-                coop = true;      // summed below by the whole warp
-            } else {
-                for (uint32_t p = p0; p < p1; p += 4) {
-                    float4 t[4];
-                    float tl[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (p + q < p1) {
-                            const float* ps = piece_sum + (size_t)piece_slot(__ldg(piece_start + p + q)) * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-                }
-            }
-        }
-        // very hot rows (thousands of lookups -> many pieces): the lane groups of the warp take the pieces
-        // round-robin (4 loads in flight each) and a fixed butterfly combines them, instead of one group
-        // walking them all.  Rows are interleaved across warps (see the row mapping above) so that the
-        // adjacent hot rows of one small field land in different warps.
-        {
-            const int lane = threadIdx.x & 31, grp = lane / LPR;
-            constexpr int G = 32 / LPR;
-            uint32_t cmask = __ballot_sync(0xffffffffu, coop && sub == 0);
-            while (cmask) {
-                const int src_lane = __ffs(cmask) - 1;
-                cmask &= cmask - 1;
-                const uint32_t cu = __shfl_sync(0xffffffffu, u, src_lane);
-                const uint32_t p0 = __ldg(row_piece0 + cu), p1 = __ldg(row_piece0 + cu + 1);
-                float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-                float al = 0.f;
-                for (uint32_t p = p0 + grp; p < p1; p += 4 * G) {
-                    float4 t[4];
-                    float tl[4];
-                    uint32_t slot[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) slot[q] = (p + q * G < p1) ? piece_slot(__ldg(piece_start + p + q * G)) : 0xffffffffu;
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (slot[q] != 0xffffffffu) {
-                            const float* ps = piece_sum + (size_t)slot[q] * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(a, t[q]); al += tl[q]; }
-                }
-#pragma unroll
-                for (int o = LPR; o < 32; o <<= 1) {
-                    a.x += __shfl_xor_sync(0xffffffffu, a.x, o); a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
-                    a.z += __shfl_xor_sync(0xffffffffu, a.z, o); a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
-                    al += __shfl_xor_sync(0xffffffffu, al, o);
-                }
-                if (lane / LPR == src_lane / LPR) { g = a; gl = al; }
-            }
-        }
-        if (SRC::SUB_E) {
-            // the fused source delivers {sum(dz s + dh0), sum(dz)}; the piece paths keep sum(dz) on lane 0 of the group only
-            gl = __shfl_sync(0xffffffffu, gl, (int)(threadIdx.x & 31) - sub);
-            if (gsum_out && act && src.sub_e()) {     // sharded requester: E = the row as it was fetched from its owner
-                const float4 e = __ldg(reinterpret_cast<const float4*>(src.erow + (size_t)u * src.erow_stride) + sub);
-                g.x = fmaf(-gl, e.x, g.x); g.y = fmaf(-gl, e.y, g.y); g.z = fmaf(-gl, e.z, g.z); g.w = fmaf(-gl, e.w, g.w);
-            }
-        }
-        if (rt) {   // fused exchange: the gradient rows go straight into their owners' receive buffers over NVLink
-            constexpr int RW = K + 4, RW4 = RW / 4;
-            const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-            float* tl = gtile + wib * (gpw * RW);
-            const int r = lane / LPR;
-            reinterpret_cast<float4*>(tl + r * RW)[sub] = g;
-            if (sub == 0) *reinterpret_cast<float4*>(tl + r * RW + K) = make_float4(gl, 0.f, 0.f, 0.f);
-            __syncwarp();
-            const uint32_t u0 = ubase + (blockIdx.x * gpb + wib * gpw);       // first row of this warp
-            if (u0 < U) {
-                const uint32_t cnt = min(gpw, U - u0);
-                const int o0 = route_find(rt->send_off, rt->W, u0), o1 = route_find(rt->send_off, rt->W, u0 + cnt - 1);
-                if (o0 == o1) {
-                    float4* dst = reinterpret_cast<float4*>(rt->peer_grecv[o0] + (size_t)(rt->dst_off[o0] + (u0 - rt->send_off[o0])) * RW);
-                    for (uint32_t j = lane; j < cnt * RW4; j += 32) dst[j] = reinterpret_cast<const float4*>(tl)[j];
-                } else {
-                    for (uint32_t q = 0; q < cnt; ++q) {
-                        const uint32_t uu = u0 + q;
-                        const int o = route_find(rt->send_off, rt->W, uu);
-                        float4* dst = reinterpret_cast<float4*>(rt->peer_grecv[o] + (size_t)(rt->dst_off[o] + (uu - rt->send_off[o])) * RW);
-                        if (lane < RW4) dst[lane] = reinterpret_cast<const float4*>(tl + q * RW)[lane];
-                    }
-                }
-            }
-            __syncwarp();
-            continue;
-        }
-        if (!act) continue;
-        if (gsum_out) {   // sharded requester side: emit the per-row gradient sum, the owner applies it
-            float* gp = gsum_out + (size_t)u * gsum_stride;
-            reinterpret_cast<float4*>(gp)[sub] = g;
-            if (sub == 0) gp[K] = gl;
-            continue;
-        }
-        // non-lazy Adam: first the decay steps this row skipped since it was last written (replayed in registers) ...
-        replay_row(w, s1, s2, lr, sub == 0, rr, rs, od, ol);
-        if (SRC::SUB_E && src.sub_e()) {      // dE = sum(dz s + dh0) - sum(dz) * E,  E = the row as the forward pass saw it
-            g.x = fmaf(-gl, w.x, g.x); g.y = fmaf(-gl, w.y, g.y); g.z = fmaf(-gl, w.z, g.z); g.w = fmaf(-gl, w.w, g.w);
-        }
-        // ... then this step's gradient
-        if (has_emb) {
-            sparse_apply(w.x, s1.x, s2.x, g.x, od);
-            sparse_apply(w.y, s1.y, s2.y, g.y, od);
-            sparse_apply(w.z, s1.z, s2.z, g.z, od);
-            sparse_apply(w.w, s1.w, s2.w, g.w, od);
-            tab_w(tb, row)[sub] = w;
-            if (emb_slots >= 1) tab_s1(tb, row)[sub] = s1;
-            if (emb_slots >= 2) tab_s2(tb, row)[sub] = s2;
-        }
-        // (the lanes of a group read last_step in ONE warp-wide load instruction, before the full-mask ballot above:
-        //  lane 0's store below cannot overtake them)
-        if (sub == 0) {
-            if (has_lin) sparse_apply(lr.x, lr.y, lr.z, gl, ol);
-            lr.w = __int_as_float(step);
-            *tab_lin(tb, row) = lr;
-        }
+// The optimizer step of one unique row, by its lane group (lane `sub` holds elements 4 sub .. 4 sub + 3 of w / s1 / s2;
+// lr = {lin w, lin s1, lin s2, last_step} is on every lane): first the non-lazy Adam decay steps the row skipped since
+// it was last written (replayed in registers), then this step's gradient g / gl (gl on lane 0).  sub_e: g is still
+// sum(dz s + dh0) of the fused step, and dE = g - sum(dz) * E with E = the row as the forward pass saw it (the replayed w).
+// The record is stored with last_step = step.
+__device__ __forceinline__ void row_step(const Table& tb, size_t row, int sub, float4 w, float4 s1, float4 s2, float4 lr, float4 g,
+                                         float gl, bool sub_e, int emb_slots, const OptDev& od, const OptDev& ol, bool has_emb,
+                                         bool has_lin, int step, const RowReplay& rr, const ReplayStep& rs) {
+    replay_row(w, s1, s2, lr, sub == 0, rr, rs, od, ol);
+    if (sub_e) { g.x = fmaf(-gl, w.x, g.x); g.y = fmaf(-gl, w.y, g.y); g.z = fmaf(-gl, w.z, g.z); g.w = fmaf(-gl, w.w, g.w); }
+    if (has_emb) {
+        sparse_apply(w.x, s1.x, s2.x, g.x, od);
+        sparse_apply(w.y, s1.y, s2.y, g.y, od);
+        sparse_apply(w.z, s1.z, s2.z, g.z, od);
+        sparse_apply(w.w, s1.w, s2.w, g.w, od);
+        tab_w(tb, row)[sub] = w;
+        if (emb_slots >= 1) tab_s1(tb, row)[sub] = s1;
+        if (emb_slots >= 2) tab_s2(tb, row)[sub] = s2;
+    }
+    if (sub == 0) {
+        if (has_lin) sparse_apply(lr.x, lr.y, lr.z, gl, ol);
+        lr.w = __int_as_float(step);
+        *tab_lin(tb, row) = lr;
     }
 }
 
@@ -1432,21 +1257,7 @@ __global__ void __launch_bounds__(256) tiny_update_kernel(const float* __restric
         if (emb_slots >= 1) s1 = tab_s1(tb, row)[sub];
         if (emb_slots >= 2) s2 = tab_s2(tb, row)[sub];
     }
-    replay_row(w, s1, s2, lr, sub == 0, rr, rs, od, ol);       // decay steps skipped since the row was last written
-    if (has_emb) {
-        sparse_apply(w.x, s1.x, s2.x, g.x, od);
-        sparse_apply(w.y, s1.y, s2.y, g.y, od);
-        sparse_apply(w.z, s1.z, s2.z, g.z, od);
-        sparse_apply(w.w, s1.w, s2.w, g.w, od);
-        tab_w(tb, row)[sub] = w;
-        if (emb_slots >= 1) tab_s1(tb, row)[sub] = s1;
-        if (emb_slots >= 2) tab_s2(tb, row)[sub] = s2;
-    }
-    if (sub == 0) {
-        if (has_lin) sparse_apply(lr.x, lr.y, lr.z, gl, ol);
-        lr.w = __int_as_float(step);
-        *tab_lin(tb, row) = lr;
-    }
+    row_step(tb, row, sub, w, s1, s2, lr, g, gl, false, emb_slots, od, ol, has_emb, has_lin, step, rr, rs);
 }
 
 // owner side: reply[i] = {emb w[K], lin w, pad} of local row recv_rows[i]

@@ -129,7 +129,7 @@ __device__ __forceinline__ void mma3(float (&cm)[4], float (&cx)[4], const uint3
 // [unique row][w[K] | lin, pad] (ES = 0 records of K + 4 floats, nothing to replay), the table lives elsewhere: the
 // gradient row of a row looked up once in the local batch is stored straight into its owner's gradient segment (peer
 // memory over NVLink, or the local send buffer of the collective path); rows looked up several times are left to
-// row_gsum_kernel / row_update_kernel, which skip the single ones.
+// row_gsum_kernel, which skips the single ones.
 template <int K, int H1, int ES, bool RB, bool FAST>
 __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs A) {
     static_assert(!RB || ES == 0, "row-buffer records carry no optimizer slots");

@@ -1,7 +1,7 @@
 // K6, staged: segmented gradient reduction + sparse optimizer for the unique rows of a step, with the table records and
 // the first gradient operand of every row brought into shared memory by cp.async (LDGSTS) a few iterations ahead.
 //
-// Why: ncu on row_update_kernel at the Criteo shape (1.7 M unique rows of 256 bytes, profiles/r02b) showed 25 % occupancy,
+// Why: ncu on the unstaged kernel at the Criteo shape (1.7 M unique rows of 256 bytes, profiles/r02b) showed 25 % occupancy,
 // 32 % issue-active and 1.8 TB/s: every lane group held one row's loads in registers, so an SM had ~14 KB in flight —
 // a quarter of what HBM latency needs.  cp.async costs no registers: each warp keeps NST-1 iterations (8 rows each at
 // K = 16) in flight, ~90 KB per SM, and the arithmetic of iteration i overlaps the traffic of i+1, i+2.  The dense
@@ -26,11 +26,11 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // staging interface of the plain gradient sources (dE buffer of the unfused step / flat gradient rows of the sharded owner)
-template <int K>
+template <int K, bool BAGS = false>
 struct StageSrcPlain {
     static constexpr bool SUB_E = false;
-    static constexpr int STAGE_F = K + 4;           // [g[K] | g_lin, pad]
-    GradSrc<K, false> s;
+    static constexpr int STAGE_F = K + 4;           // [g[K] | g_lin, 1 / count (BAGS), pad]
+    GradSrc<K, BAGS> s;
     const float* erow = nullptr; int erow_stride = 0;       // (only sources with SUB_E carry the fetched rows)
     __device__ __forceinline__ bool sub_e() const { return false; }
     __device__ __forceinline__ void stage_async(uint32_t val, float* dst, int sub) const {
@@ -40,19 +40,120 @@ struct StageSrcPlain {
             cp_async16(dst + sub * 4, rp + sub * 4);
             if (sub == 0) cp_async16(dst + K, rp + K);
         } else {
-            const uint32_t b = payload_sample(val), f = payload_slot(val);
+            const uint32_t b = payload_sample(val);
+            uint32_t f = payload_slot(val);
+            if (BAGS) f = (uint32_t)__ldg(s.slot_field + f);
             if (s.dE) cp_async16(dst + sub * 4, s.dE + (size_t)b * s.dK + (size_t)f * K + sub * 4);
             if (sub == LPR - 1) cp_async4(dst + K, s.dz + b);
+            if (BAGS && sub == 0) cp_async4(dst + K + 1, s.inv_cnt + (size_t)b * s.dc + f);
         }
     }
     int aux_floats() const { return 0; }                              // no per-CTA shared-memory operand
     __device__ __forceinline__ void aux_load(float*, int) const {}
     __device__ __forceinline__ void consume(const float* st, const float*, uint32_t, int sub, float4& g, float& gl) const {
         g = (s.flat || s.dE) ? *reinterpret_cast<const float4*>(st + sub * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+        if (BAGS && !s.flat) {   // mean combiner, as in GradSrc::fetch: every present slot of the bag receives dE / count
+            const float ic = st[K + 1];
+            g.x *= ic; g.y *= ic; g.z *= ic; g.w *= ic;
+        }
         gl = st[K];
     }
     __device__ __forceinline__ void fetch(uint32_t val, int sub, bool want_lin, float4& g, float& gl) const { s.fetch(val, sub, want_lin, g, gl); }
 };
+
+// The gradient sum of unique row u (its lookups are beg .. end-1 of the sorted order; act: the row has work here), called
+// by every lane of the warp.  Rows with <= DIRECT_T lookups add them in sorted (= sample) order, the first one from the
+// staging slot `staged`; hotter rows add their piece sums in order; very hot rows (> COOP_PIECES pieces) are summed by
+// the whole warp: its lane groups take the pieces round-robin and a fixed butterfly combines them.  The summation order
+// is thus a function of the sorted order only.  gl is complete on lane 0 of the group (on every lane if SRC::SUB_E).
+template <int K, typename SRC>
+__device__ __forceinline__ void row_grad_sum(const SRC& src, const float* staged, const float* aux, bool act, uint32_t u, uint32_t v0,
+                                             uint32_t beg, uint32_t end, const uint32_t* __restrict__ svals,
+                                             const uint32_t* __restrict__ row_piece0, const uint32_t* __restrict__ piece_start,
+                                             const float* __restrict__ piece_sum, float4& g, float& gl) {
+    constexpr int LPR = K / 4, G = 32 / LPR;
+    const int lane = threadIdx.x & 31, sub = lane % LPR, grp = lane / LPR;
+    g = make_float4(0.f, 0.f, 0.f, 0.f);
+    gl = 0.f;
+    bool coop = false;
+    if (!act) {
+    } else if (end - beg <= (uint32_t)DIRECT_T) {
+        src.consume(staged, aux, v0, sub, g, gl);             // first lookup of the row: staged a few iterations ahead
+        for (uint32_t i = beg + 1; i < end; i += 4) {         // further lookups of the same row (rare with large tables)
+            uint32_t v[4];
+            float4 t[4];
+            float tl[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) v[q] = (i + q < end) ? __ldg(svals + i + q) : 0xffffffffu;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+                tl[q] = 0.f;
+                if (v[q] != 0xffffffffu) src.fetch(v[q], sub, sub == 0, t[q], tl[q]);
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
+        }
+    } else {
+        const uint32_t p0 = __ldg(row_piece0 + u), p1 = __ldg(row_piece0 + u + 1);
+        if (p1 - p0 > (uint32_t)COOP_PIECES) {
+            coop = true;      // summed below by the whole warp
+        } else {
+            for (uint32_t p = p0; p < p1; p += 4) {
+                float4 t[4];
+                float tl[4];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+                    tl[q] = 0.f;
+                    if (p + q < p1) {
+                        const float* ps = piece_sum + (size_t)piece_slot(__ldg(piece_start + p + q)) * (K + 4);
+                        t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
+                        if (sub == 0) tl[q] = __ldg(ps + K);
+                    }
+                }
+#pragma unroll
+                for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
+            }
+        }
+    }
+    uint32_t cmask = __ballot_sync(0xffffffffu, coop && sub == 0);
+    while (cmask) {
+        const int src_lane = __ffs(cmask) - 1;
+        cmask &= cmask - 1;
+        const uint32_t cu = __shfl_sync(0xffffffffu, u, src_lane);
+        const uint32_t p0 = __ldg(row_piece0 + cu), p1 = __ldg(row_piece0 + cu + 1);
+        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
+        float al = 0.f;
+        for (uint32_t p = p0 + grp; p < p1; p += 4 * G) {
+            float4 t[4];
+            float tl[4];
+            uint32_t ps_slot[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) ps_slot[q] = (p + q * G < p1) ? piece_slot(__ldg(piece_start + p + q * G)) : 0xffffffffu;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+                tl[q] = 0.f;
+                if (ps_slot[q] != 0xffffffffu) {
+                    const float* ps = piece_sum + (size_t)ps_slot[q] * (K + 4);
+                    t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
+                    if (sub == 0) tl[q] = __ldg(ps + K);
+                }
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) { add4(a, t[q]); al += tl[q]; }
+        }
+#pragma unroll
+        for (int o = LPR; o < 32; o <<= 1) {
+            a.x += __shfl_xor_sync(0xffffffffu, a.x, o); a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
+            a.z += __shfl_xor_sync(0xffffffffu, a.z, o); a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
+            al += __shfl_xor_sync(0xffffffffu, al, o);
+        }
+        if (lane / LPR == src_lane / LPR) { g = a; gl = al; }
+    }
+    if (SRC::SUB_E) gl = __shfl_sync(0xffffffffu, gl, lane - sub);   // the piece paths keep sum(dz) on lane 0 of the group only
+}
 
 template <int K, typename SRC>
 struct RowApplyCfg {
@@ -143,111 +244,10 @@ __global__ void __launch_bounds__(256, 2) row_apply_kernel(const uint32_t* __res
                 lr = *reinterpret_cast<const float4*>(slot);
             }
         }
-        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-        float gl = 0.f;
-        bool coop = false;
-        if (!act) {
-        } else if (end - beg <= (uint32_t)DIRECT_T) {
-            src.consume(slot + RSMAX, aux, v0, sub, g, gl);       // first lookup of the row: staged with the record
-            for (uint32_t i = beg + 1; i < end; i += 4) {         // further lookups of the same row (rare with large tables)
-                uint32_t v[4];
-                float4 t[4];
-                float tl[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v[q] = (i + q < end) ? __ldg(svals + i + q) : 0xffffffffu;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    tl[q] = 0.f;
-                    if (v[q] != 0xffffffffu) src.fetch(v[q], sub, sub == 0, t[q], tl[q]);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-            }
-        } else {
-            const uint32_t p0 = __ldg(row_piece0 + u), p1 = __ldg(row_piece0 + u + 1);
-            if (p1 - p0 > (uint32_t)COOP_PIECES) {
-                coop = true;      // summed below by the whole warp
-            } else {
-                for (uint32_t p = p0; p < p1; p += 4) {
-                    float4 t[4];
-                    float tl[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (p + q < p1) {
-                            const float* ps = piece_sum + (size_t)piece_slot(__ldg(piece_start + p + q)) * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-                }
-            }
-        }
-        // very hot rows (many pieces): the lane groups of the warp take the pieces round-robin, a fixed butterfly combines them
-        {
-            uint32_t cmask = __ballot_sync(0xffffffffu, coop && sub == 0);
-            while (cmask) {
-                const int src_lane = __ffs(cmask) - 1;
-                cmask &= cmask - 1;
-                const uint32_t cu = __shfl_sync(0xffffffffu, u, src_lane);
-                const uint32_t p0 = __ldg(row_piece0 + cu), p1 = __ldg(row_piece0 + cu + 1);
-                float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-                float al = 0.f;
-                for (uint32_t p = p0 + grp; p < p1; p += 4 * G) {
-                    float4 t[4];
-                    float tl[4];
-                    uint32_t ps_slot[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) ps_slot[q] = (p + q * G < p1) ? piece_slot(__ldg(piece_start + p + q * G)) : 0xffffffffu;
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (ps_slot[q] != 0xffffffffu) {
-                            const float* ps = piece_sum + (size_t)ps_slot[q] * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(a, t[q]); al += tl[q]; }
-                }
-#pragma unroll
-                for (int o = LPR; o < 32; o <<= 1) {
-                    a.x += __shfl_xor_sync(0xffffffffu, a.x, o); a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
-                    a.z += __shfl_xor_sync(0xffffffffu, a.z, o); a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
-                    al += __shfl_xor_sync(0xffffffffu, al, o);
-                }
-                if (lane / LPR == src_lane / LPR) { g = a; gl = al; }
-            }
-        }
-        if (SRC::SUB_E) gl = __shfl_sync(0xffffffffu, gl, lane - sub);   // the piece paths keep sum(dz) on lane 0 of the group only
-        if (act) {
-            // non-lazy Adam: first the decay steps this row skipped since it was last written (replayed in registers) ...
-            replay_row(w, s1, s2, lr, sub == 0, rr, rs, od, ol);
-            if (SRC::SUB_E && src.sub_e()) {      // dE = sum(dz s + dh0) - sum(dz) * E,  E = the row as the forward pass saw it
-                g.x = fmaf(-gl, w.x, g.x); g.y = fmaf(-gl, w.y, g.y); g.z = fmaf(-gl, w.z, g.z); g.w = fmaf(-gl, w.w, g.w);
-            }
-            // ... then this step's gradient
-            if (has_emb) {
-                sparse_apply(w.x, s1.x, s2.x, g.x, od);
-                sparse_apply(w.y, s1.y, s2.y, g.y, od);
-                sparse_apply(w.z, s1.z, s2.z, g.z, od);
-                sparse_apply(w.w, s1.w, s2.w, g.w, od);
-                tab_w(tb, row)[sub] = w;
-                if (emb_slots >= 1) tab_s1(tb, row)[sub] = s1;
-                if (emb_slots >= 2) tab_s2(tb, row)[sub] = s2;
-            }
-            if (sub == 0) {
-                if (has_lin) sparse_apply(lr.x, lr.y, lr.z, gl, ol);
-                lr.w = __int_as_float(step);
-                *tab_lin(tb, row) = lr;
-            }
-        }
+        float4 g;
+        float gl;
+        row_grad_sum<K>(src, slot + RSMAX, aux, act, u, v0, beg, end, svals, row_piece0, piece_start, piece_sum, g, gl);
+        if (act) row_step(tb, row, sub, w, s1, s2, lr, g, gl, SRC::SUB_E && src.sub_e(), emb_slots, od, ol, has_emb, has_lin, step, rr, rs);
         __syncwarp();      // the slot is overwritten by the copies issued in the next iteration
     }
     cp_async_wait<0>();
@@ -256,11 +256,12 @@ __global__ void __launch_bounds__(256, 2) row_apply_kernel(const uint32_t* __res
 }
 
 
-// Requester side of the row-sharded step: per-unique-row gradient sums of the local batch, stored straight into the
-// owners' gradient segments over NVLink (no table access here: the rows live on their owners).  Same warp-level
-// cp.async pipeline as row_apply_kernel; what is staged per row is the first lookup's gradient operand and, for the
-// fused source, the row E as it was fetched (dE = sum(dz s + dh0) - sum(dz) E).  A warp's G consecutive rows are
-// contiguous at the destination unless they straddle two owners, so they leave as one staged, fully coalesced store.
+// Requester side of the row-sharded step: per-unique-row gradient sums of the local batch (no table access here: the
+// rows live on their owners), stored either as local gradient rows gsum[u] = {g[K], g_lin, pad} that the collectives
+// send on (rt == nullptr), or straight into the owners' gradient segments over NVLink (rt).  Same warp-level cp.async
+// pipeline as row_apply_kernel; what is staged per row is the first lookup's gradient operand and, for the fused
+// source, the row E as it was fetched (dE = sum(dz s + dh0) - sum(dz) E).  A warp's G consecutive rows are contiguous
+// at the destination unless they straddle two owners, so they leave as one staged, fully coalesced store.
 template <int K, typename SRC>
 struct RowGsumCfg {
     static constexpr int LPR = K / 4, G = 32 / LPR;
@@ -275,7 +276,7 @@ __global__ void __launch_bounds__(256, 2) row_gsum_kernel(const uint32_t* __rest
                                                           const uint32_t* __restrict__ svals, const uint32_t* __restrict__ row_start,
                                                           const uint32_t* __restrict__ row_piece0, const uint32_t* __restrict__ piece_start,
                                                           const SegCounts* __restrict__ cnt, SRC src, const float* __restrict__ piece_sum,
-                                                          const PeerRoute* __restrict__ rt, bool skip_single = false) {
+                                                          const PeerRoute* __restrict__ rt, float* __restrict__ gsum, bool skip_single) {
     // skip_single: rows with exactly one lookup were already stored by fused_rows_kernel (row-buffer mode)
     using C = RowGsumCfg<K, SRC>;
     constexpr int LPR = C::LPR, G = C::G, SLOT = C::SLOT, NST = C::NST, RW = K + 4, RW4 = RW / 4;
@@ -328,96 +329,14 @@ __global__ void __launch_bounds__(256, 2) row_gsum_kernel(const uint32_t* __rest
         const uint4 meta = *reinterpret_cast<const uint4*>(slot + K + SRC::STAGE_F);
         const uint32_t v0 = meta.y, beg = meta.z, end = meta.w;
         const bool act = end > beg;
-        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-        float gl = 0.f;
-        bool coop = false;
-        if (!act) {
-        } else if (end - beg <= (uint32_t)DIRECT_T) {
-            src.consume(slot + K, aux, v0, sub, g, gl);
-            for (uint32_t i = beg + 1; i < end; i += 4) {
-                uint32_t v[4];
-                float4 t[4];
-                float tl[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v[q] = (i + q < end) ? __ldg(svals + i + q) : 0xffffffffu;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    tl[q] = 0.f;
-                    if (v[q] != 0xffffffffu) src.fetch(v[q], sub, sub == 0, t[q], tl[q]);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-            }
-        } else {
-            const uint32_t p0 = __ldg(row_piece0 + u), p1 = __ldg(row_piece0 + u + 1);
-            if (p1 - p0 > (uint32_t)COOP_PIECES) {
-                coop = true;
-            } else {
-                for (uint32_t p = p0; p < p1; p += 4) {
-                    float4 t[4];
-                    float tl[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (p + q < p1) {
-                            const float* ps = piece_sum + (size_t)piece_slot(__ldg(piece_start + p + q)) * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(g, t[q]); gl += tl[q]; }
-                }
-            }
+        float4 g;
+        float gl;
+        row_grad_sum<K>(src, slot + K, aux, act, u, v0, beg, end, svals, row_piece0, piece_start, piece_sum, g, gl);
+        if (act && sub_e) {
+            const float4 e = *reinterpret_cast<const float4*>(slot + sub * 4);
+            g.x = fmaf(-gl, e.x, g.x); g.y = fmaf(-gl, e.y, g.y); g.z = fmaf(-gl, e.z, g.z); g.w = fmaf(-gl, e.w, g.w);
         }
-        {
-            uint32_t cmask = __ballot_sync(0xffffffffu, coop && sub == 0);
-            while (cmask) {
-                const int src_lane = __ffs(cmask) - 1;
-                cmask &= cmask - 1;
-                const uint32_t cu = __shfl_sync(0xffffffffu, u, src_lane);
-                const uint32_t p0 = __ldg(row_piece0 + cu), p1 = __ldg(row_piece0 + cu + 1);
-                float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-                float al = 0.f;
-                for (uint32_t p = p0 + grp; p < p1; p += 4 * G) {
-                    float4 t[4];
-                    float tl[4];
-                    uint32_t ps_slot[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) ps_slot[q] = (p + q * G < p1) ? piece_slot(__ldg(piece_start + p + q * G)) : 0xffffffffu;
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        t[q] = make_float4(0.f, 0.f, 0.f, 0.f);
-                        tl[q] = 0.f;
-                        if (ps_slot[q] != 0xffffffffu) {
-                            const float* ps = piece_sum + (size_t)ps_slot[q] * (K + 4);
-                            t[q] = __ldg(reinterpret_cast<const float4*>(ps) + sub);
-                            if (sub == 0) tl[q] = __ldg(ps + K);
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) { add4(a, t[q]); al += tl[q]; }
-                }
-#pragma unroll
-                for (int o = LPR; o < 32; o <<= 1) {
-                    a.x += __shfl_xor_sync(0xffffffffu, a.x, o); a.y += __shfl_xor_sync(0xffffffffu, a.y, o);
-                    a.z += __shfl_xor_sync(0xffffffffu, a.z, o); a.w += __shfl_xor_sync(0xffffffffu, a.w, o);
-                    al += __shfl_xor_sync(0xffffffffu, al, o);
-                }
-                if (lane / LPR == src_lane / LPR) { g = a; gl = al; }
-            }
-        }
-        if (SRC::SUB_E) {
-            gl = __shfl_sync(0xffffffffu, gl, lane - sub);
-            if (act && sub_e) {
-                const float4 e = *reinterpret_cast<const float4*>(slot + sub * 4);
-                g.x = fmaf(-gl, e.x, g.x); g.y = fmaf(-gl, e.y, g.y); g.z = fmaf(-gl, e.z, g.z); g.w = fmaf(-gl, e.w, g.w);
-            }
-        }
-        // the warp's rows -> one contiguous store into their owner's gradient segment (rows left out by skip_single are
-        // not touched: fused_rows_kernel stored them)
+        // the warp's rows -> one contiguous store (rows left out by skip_single are not touched: fused_rows_kernel stored them)
         const unsigned rowmask = __ballot_sync(0xffffffffu, act && sub == 0);
         reinterpret_cast<float4*>(otile + grp * RW)[sub] = g;
         if (sub == 0) *reinterpret_cast<float4*>(otile + grp * RW + K) = make_float4(gl, 0.f, 0.f, 0.f);
@@ -425,9 +344,10 @@ __global__ void __launch_bounds__(256, 2) row_gsum_kernel(const uint32_t* __rest
         const uint32_t u0 = u - grp;                              // first row of this warp's chunk
         if (u0 < U && rowmask) {
             const uint32_t n_rows = min((uint32_t)G, U - u0);
-            const int o0 = route_find(rt->send_off, rt->W, u0), o1 = route_find(rt->send_off, rt->W, u0 + n_rows - 1);
+            const int o0 = rt ? route_find(rt->send_off, rt->W, u0) : 0, o1 = rt ? route_find(rt->send_off, rt->W, u0 + n_rows - 1) : 0;
             if (o0 == o1) {
-                float4* dst = reinterpret_cast<float4*>(rt->peer_grecv[o0] + (size_t)(rt->dst_off[o0] + (u0 - rt->send_off[o0])) * RW);
+                float4* dst = reinterpret_cast<float4*>(rt ? rt->peer_grecv[o0] + (size_t)(rt->dst_off[o0] + (u0 - rt->send_off[o0])) * RW
+                                                           : gsum + (size_t)u0 * RW);
                 for (uint32_t j = lane; j < n_rows * RW4; j += 32)
                     if ((rowmask >> ((j / RW4) * LPR)) & 1u) dst[j] = reinterpret_cast<const float4*>(otile)[j];
             } else {
