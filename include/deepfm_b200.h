@@ -333,18 +333,21 @@ int dfm_test_tc_gemm(int32_t mode, const float* A_dev, const float* B_dev, float
 /* ---- GPU CSV record decoder: replaces tf.data.TextLineDataset(csv) + tf.decode_csv(value, DEFAULTS) of the
  * reference's input_fn (trainers/ml_100k.py:44-58; schema COLUMNS / DEFAULTS, trainers/ml_100k.py:3-15) for the
  * fields the model consumes.  The host hands over whole records (lines); field splitting, RFC-4180 unquoting
- * ('""' inside a quoted field), int32 parsing, default substitution for empty fields and the label threshold
- * (rating >= cutoff, trainers/ml_100k.py:47-48) run on the device.  The decoded columns stay in the reader's
- * device buffers in the layout dfm_raw_batch takes: int32[n] columns, Arrow-style string columns
- * (int32 offsets[n+1] + bytes), float labels[n].  Errors follow tf.decode_csv: wrong field count, a field that
- * is not a valid int32, a quote inside an unquoted field or an unterminated quote -> DFM_ERR_PARSE, with the
- * first offending record in dfm_csv_last_error. */
+ * ('""' inside a quoted field), int32 and float32 parsing, default substitution for empty fields and the label
+ * threshold (rating >= cutoff, trainers/ml_100k.py:47-48) run on the device.  The decoded columns stay in the
+ * reader's device buffers in the layout dfm_raw_batch takes: int32[n] and float32[n] columns, Arrow-style string
+ * columns (int32 offsets[n+1] + bytes), float labels[n].  Float32 fields follow TF 1.12's strings::safe_strtof,
+ * correctly rounded (oracle/strtof.py states the grammar), except that hexadecimal is rejected.  Errors follow
+ * tf.decode_csv: wrong field count, a field that is not a valid int32 or float32, a quote inside an unquoted field
+ * or an unterminated quote -> DFM_ERR_PARSE, with the first offending record in dfm_csv_last_error. */
 #define DFM_CSV_SKIP    0          /* parsed for structure only (15 of the 42 ML-100K fields are never consumed) */
 #define DFM_CSV_INT32   1          /* record_defaults [0]      */
 #define DFM_CSV_STRING  2          /* record_defaults ["null"] */
+#define DFM_CSV_FLOAT32 3          /* record_defaults [0.0]    */
 #define DFM_CSV_ERR_FIELDS 1
 #define DFM_CSV_ERR_INT    2
 #define DFM_CSV_ERR_QUOTE  3
+#define DFM_CSV_ERR_FLOAT  4
 typedef struct {
     int32_t            n_fields;       /* fields per record (42) */
     const int32_t*     kind;           /* [n_fields] DFM_CSV_* */
@@ -355,6 +358,10 @@ typedef struct {
     int32_t            max_records;    /* per decode call */
     int64_t            max_bytes;      /* per decode call, < 4 GiB */
     int32_t            device;
+    const float*       float_default;  /* [n_fields] value of an empty float32 field (NULL: 0.0f) */
+    int32_t            field_delim;    /* field separator, one byte other than '"', '\n' and '\r' (0: ',') */
+    const int32_t*     as_float;       /* [n_fields] nonzero on an int32 field: also write it as float32, rounded to
+                                          nearest (tf.to_float of a numeric_column over an int field); NULL: none */
 } dfm_csv_config;
 typedef struct dfm_csv_reader dfm_csv_reader;
 int dfm_csv_create(const dfm_csv_config* cfg, dfm_csv_reader** out);
@@ -374,6 +381,8 @@ int32_t dfm_csv_num_records(const dfm_csv_reader* r);
 const int32_t* dfm_csv_int_column(const dfm_csv_reader* r, int32_t field);     /* device int32[n_records] */
 const char*    dfm_csv_str_bytes(const dfm_csv_reader* r, int32_t field);      /* device bytes */
 const int32_t* dfm_csv_str_offsets(const dfm_csv_reader* r, int32_t field);    /* device int32[n_records + 1] */
+/* device float32[n_records] of a float32 field or of an int32 field with as_float; NULL for any other field */
+const float*   dfm_csv_float_column(const dfm_csv_reader* r, int32_t field);
 const float*   dfm_csv_labels(const dfm_csv_reader* r);                        /* device float[n_records] */
 
 const char* dfm_version(void);

@@ -110,6 +110,7 @@ _SIGS = {
     "dfm_csv_int_column": (C.c_void_p, [C.c_void_p, C.c_int32]),
     "dfm_csv_str_bytes": (C.c_void_p, [C.c_void_p, C.c_int32]),
     "dfm_csv_str_offsets": (C.c_void_p, [C.c_void_p, C.c_int32]),
+    "dfm_csv_float_column": (C.c_void_p, [C.c_void_p, C.c_int32]),
     "dfm_csv_labels": (C.c_void_p, [C.c_void_p]),
     "dfm_test_sort_pairs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]),
     "dfm_test_sort_pairs_algo": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32]),

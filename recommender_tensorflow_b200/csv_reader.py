@@ -13,24 +13,32 @@ import numpy as np
 from . import _lib
 from .engine import DfmError, PackedBatch
 
-CSV_SKIP, CSV_INT32, CSV_STRING = 0, 1, 2
+CSV_SKIP, CSV_INT32, CSV_STRING, CSV_FLOAT32 = 0, 1, 2, 3
 
 
 class CsvConfig(C.Structure):
     _fields_ = [("n_fields", C.c_int32), ("kind", C.POINTER(C.c_int32)), ("int_default", C.POINTER(C.c_int32)),
                 ("str_default", C.POINTER(C.c_char_p)), ("label_field", C.c_int32), ("label_min", C.c_int32),
-                ("max_records", C.c_int32), ("max_bytes", C.c_int64), ("device", C.c_int32)]
+                ("max_records", C.c_int32), ("max_bytes", C.c_int64), ("device", C.c_int32),
+                ("float_default", C.POINTER(C.c_float)), ("field_delim", C.c_int32), ("as_float", C.POINTER(C.c_int32))]
+
+
+def _default_dtype(d):
+    """record_defaults entry -> the dtype tf.decode_csv gives the field"""
+    if isinstance(d, (int, np.integer)):
+        return "int32"
+    return "float32" if isinstance(d, (float, np.floating)) else "string"
 
 
 class GpuCsvReader:
-    def __init__(self, engine, columns, defaults, label_col=None, cutoff=5, max_records=65536, max_bytes=None):
-        """columns / defaults: the CSV schema (names and `record_defaults`, e.g. trainers.ml_100k.COLUMNS / DEFAULTS).
-        Only the fields `engine` consumes (plus the label) are materialised; the rest is parsed for structure only."""
+    def __init__(self, engine, columns, defaults, label_col=None, cutoff=5, max_records=65536, max_bytes=None, field_delim=","):
+        """columns / defaults: the CSV schema (names and `record_defaults`, e.g. trainers.ml_100k.COLUMNS / DEFAULTS;
+        [0] is int32, [0.0] float32, anything else a string).  Only the fields `engine` consumes (plus the label) are
+        materialised; the rest is parsed for structure only.  A numeric column reads a float32 field, or an int32 field
+        converted with tf.to_float.  field_delim: one character, as tf.decode_csv's."""
         self.lib = _lib.load()
         self.eng = engine
         self.columns = list(columns)
-        if engine.num_columns:
-            raise ValueError("GpuCsvReader: numeric (float) model columns are not supported, the CSV schema is int32 / string")
         wanted = {}
         for s in engine.raw_specs:          # model columns and the source columns of crossed ones
             if s["kind"] == "crossed":
@@ -38,31 +46,43 @@ class GpuCsvReader:
             if s["width"] != 1:
                 raise ValueError("GpuCsvReader: multivalent column %r has no CSV encoding in the reference" % s["source"])
             wanted[s["source"]] = s["dtype"]
+        numeric = {c.key for c in engine.num_columns}
+        delim = field_delim.encode() if isinstance(field_delim, str) else bytes(field_delim)
+        if len(delim) != 1:
+            raise ValueError("field_delim must be one byte, got %r" % (field_delim,))
         n = len(self.columns)
         kind = (C.c_int32 * n)()
         idef = (C.c_int32 * n)()
         sdef = (C.c_char_p * n)()
+        fdef = (C.c_float * n)()
+        as_float = (C.c_int32 * n)()
         for j, (name, d) in enumerate(zip(self.columns, defaults)):
-            is_int = isinstance(d[0], (int, np.integer))
-            if name in wanted and wanted[name] != ("int32" if is_int else "string"):
+            dt = _default_dtype(d[0])
+            if name in wanted and wanted[name] != dt:
                 raise ValueError("column %r: model expects %s, CSV default %r says otherwise" % (name, wanted[name], d))
-            if name in wanted or name == label_col:
-                kind[j] = CSV_INT32 if is_int else CSV_STRING
+            if name in numeric and dt == "string":
+                raise ValueError("column %r: numeric column expects float32 or int32, CSV default %r says otherwise" % (name, d))
+            if name in wanted or name in numeric or name == label_col:
+                kind[j] = {"int32": CSV_INT32, "float32": CSV_FLOAT32, "string": CSV_STRING}[dt]
             else:
                 kind[j] = CSV_SKIP
-            if is_int:
+            as_float[j] = int(name in numeric and dt == "int32")
+            if dt == "int32":
                 idef[j] = int(d[0])
+            elif dt == "float32":
+                fdef[j] = float(d[0])
             else:
                 sdef[j] = str(d[0]).encode()
-        missing = [k for k in wanted if k not in self.columns]
+        missing = [k for k in list(wanted) + sorted(numeric) if k not in self.columns]
         if missing:
             raise ValueError("model columns missing from the CSV schema: %r" % missing)
         self.label_field = self.columns.index(label_col) if label_col is not None else -1
         self.max_records = int(max_records)
         self.max_bytes = int(max_bytes or 512 * self.max_records)
         cfg = CsvConfig(n, C.cast(kind, C.POINTER(C.c_int32)), C.cast(idef, C.POINTER(C.c_int32)), C.cast(sdef, C.POINTER(C.c_char_p)),
-                        self.label_field, int(cutoff), self.max_records, self.max_bytes, engine.device)
-        self._keep = [kind, idef, sdef]
+                        self.label_field, int(cutoff), self.max_records, self.max_bytes, engine.device,
+                        C.cast(fdef, C.POINTER(C.c_float)), delim[0], C.cast(as_float, C.POINTER(C.c_int32)))
+        self._keep = [kind, idef, sdef, fdef, as_float]
         h = C.c_void_p()
         rc = self.lib.dfm_csv_create(C.byref(cfg), C.byref(h))
         if rc != _lib.DFM_OK:
@@ -124,7 +144,7 @@ class GpuCsvReader:
         nc = max(len(eng.raw_specs), 1)
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
-        num = (C.c_void_p * 1)()
+        num = (C.c_void_p * max(len(eng.num_columns), 1))()
         for i, s in enumerate(eng.raw_specs):
             if s["kind"] == "crossed":
                 continue
@@ -132,8 +152,12 @@ class GpuCsvReader:
             if s["dtype"] == "string":
                 cat[i] = self.lib.dfm_csv_str_bytes(self.h, f)
                 off[i] = self.lib.dfm_csv_str_offsets(self.h, f)
+            elif s["dtype"] == "float32":      # bucketized column over a float32 field
+                cat[i] = self.lib.dfm_csv_float_column(self.h, f)
             else:
                 cat[i] = self.lib.dfm_csv_int_column(self.h, f)
+        for j, c in enumerate(eng.num_columns):
+            num[j] = self.lib.dfm_csv_float_column(self.h, self._field[c.key])
         lab = self.lib.dfm_csv_labels(self.h) if self.label_field >= 0 else None
         raw = _lib.RawBatch(n, C.cast(cat, C.POINTER(C.c_void_p)), C.cast(off, C.POINTER(C.c_void_p)),
                             C.cast(num, C.POINTER(C.c_void_p)), lab)
@@ -152,15 +176,26 @@ class GpuCsvReader:
         return torch.as_tensor(_View(), device="cuda").cpu().numpy()
 
     def column(self, name):
-        """Decoded column as numpy: int32 [n] or an object array of bytes (strings)."""
+        """Decoded column as numpy: int32 [n], float32 [n] or an object array of bytes (strings).  An int32 field that
+        a numeric column reads as float32 comes back as int32; float_column() gives its float32 copy."""
         f = self._field[name]
         n = int(self.lib.dfm_csv_num_records(self.h))
         p = self.lib.dfm_csv_int_column(self.h, f)
         if p:
             return self._d2h(p, 4 * n).view(np.int32).copy()
+        if self.lib.dfm_csv_float_column(self.h, f):
+            return self.float_column(name)
         offs = self._d2h(self.lib.dfm_csv_str_offsets(self.h, f), 4 * (n + 1)).view(np.int32).copy()
         data = self._d2h(self.lib.dfm_csv_str_bytes(self.h, f), int(offs[-1])).tobytes()
         return np.array([data[offs[i]:offs[i + 1]] for i in range(n)], dtype=object)
+
+    def float_column(self, name):
+        """float32 [n] of a float32 field, or of an int32 field that a numeric column reads"""
+        p = self.lib.dfm_csv_float_column(self.h, self._field[name])
+        if not p:
+            raise ValueError("column %r has no float32 copy: it is neither a float32 field nor an int32 field a numeric column reads" % name)
+        n = int(self.lib.dfm_csv_num_records(self.h))
+        return self._d2h(p, 4 * n).view(np.float32).copy()
 
     def labels(self):
         n = int(self.lib.dfm_csv_num_records(self.h))

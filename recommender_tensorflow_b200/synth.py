@@ -84,6 +84,46 @@ def criteo_batch(batch_size, rng, n_cat=26, n_num=13, zipf_alpha=None, key_space
     return feats, y
 
 
+def _float_text(x, form):
+    """float32 x printed in one of several forms that all read back as x (form 0..4)"""
+    if form == 0:
+        return np.format_float_positional(x, unique=True, trim="-")       # shortest repr: 1.0986123, 0
+    if form == 1:
+        return "%.9g" % x
+    if form == 2:
+        return "%d" % x if float(x).is_integer() else "%.9g" % x
+    if form == 3:
+        return "%.8e" % x                                                   # 1.09861231e+00
+    return np.format_float_scientific(x, unique=True, exp_digits=1)         # 1.0986123e+0
+
+
+def criteo_tsv_schema(n_cat=26, n_num=13):
+    """(columns, record_defaults) of a Criteo TSV line: label, I1..I13 ([0.0]), C1..C26 ([""])"""
+    cols = ["label"] + ["I%d" % (j + 1) for j in range(n_num)] + ["C%d" % (f + 1) for f in range(n_cat)]
+    return cols, [[0]] + [[0.0]] * n_num + [[""]] * n_cat
+
+
+def write_criteo_tsv(path, n_rows, seed, empty_frac=0.05, n_cat=26, n_num=13):
+    """Criteo-style raw text: per line the 0/1 label, I1..I13, C1..C26, tab-separated, no header.  The numerics are the
+    float32 values criteo_batch draws, printed in a mix of forms (shortest repr, %.9g, integers, exponent forms); the
+    categoricals are its 8-hex-char keys.  A share empty_frac of the numeric and categorical fields is left empty."""
+    rng = np.random.default_rng(seed)
+    feats, y = criteo_batch(n_rows, rng, n_cat, n_num)
+    forms = rng.integers(0, 5, (n_rows, n_num))
+    empty = rng.random((n_rows, n_num + n_cat)) < empty_frac
+    cats = [feats["C%d" % (f + 1)][0].reshape(n_rows, 8).tobytes() for f in range(n_cat)]
+    lines = []
+    for i in range(n_rows):
+        row = ["%d" % y[i]]
+        for j in range(n_num):
+            row.append("" if empty[i, j] else _float_text(feats["I%d" % (j + 1)][i], forms[i, j]))
+        for f in range(n_cat):
+            row.append("" if empty[i, n_num + f] else cats[f][8 * i:8 * i + 8].decode())
+        lines.append("\t".join(row))
+    with open(path, "w", newline="") as fh:
+        fh.write("\n".join(lines) + "\n")
+
+
 def criteo_columns(buckets_per_field, n_cat=26, n_num=13):
     from . import feature_column as fc
     cats = [fc.categorical_column_with_hash_bucket("C%d" % (f + 1), buckets_per_field) for f in range(n_cat)]
