@@ -141,6 +141,11 @@ typedef struct {
      * dfm_raw_batch.cat_data[n_cat + s] / cat_offsets[n_cat + s].  n_cat + n_src <= DFM_MAX_CAT. */
     int32_t           n_src;
     const dfm_column* src;
+    /* weight_column of the canned estimators / binary head: nonzero makes every TRAIN batch carry per-example weights
+     * (dfm_raw_batch.weights).  The per-sample loss and its gradient are multiplied by the weight:
+     * SUM: loss = sum_b w_b l_b, dz_b = w_b (sigmoid(z_b) - y_b); MEAN: both divided by the (global) batch size, not by
+     * sum w.  Zero, negative and fractional weights are accepted, as in TF.  0 = unweighted: weights is never read. */
+    int32_t           weighted;
 } dfm_config;
 
 /* One batch of raw (un-hashed) feature columns = what input_fn's parse_csv yields
@@ -152,6 +157,10 @@ typedef struct {
     const int32_t* const* cat_offsets;  /* [n_cat + n_src]: int32[B+1] byte offsets for string columns, else NULL */
     const float* const*   num_data;     /* [n_num]: float32[B] */
     const float*          labels;       /* [B] 0/1 (rating >= cutoff, trainers/ml_100k.py:48); NULL for forward */
+    /* [B] float32 per-example weights, on the same side (host / device) as labels.  Read only by a handle created with
+     * dfm_config.weighted != 0, and only by train steps (required there: NULL -> DFM_ERR_INVALID_ARG); forward,
+     * PREDICT and layer_summary ignore it.  An unweighted handle never reads this field. */
+    const float*          weights;
 } dfm_raw_batch;
 
 #define DFM_ACT_RELU 0

@@ -111,6 +111,9 @@ tf::Status Collect(tf::OpKernelContext* ctx, const std::vector<int>& cat_order, 
     b->raw.cat_offsets = b->off.data();
     b->raw.num_data = b->num.data();
     b->raw.labels = nullptr;
+    // per-example weights (dfm_raw_batch.weights) are read only by handles created with dfm_config.weighted != 0; this
+    // op creates unweighted handles and has no weights input yet
+    b->raw.weights = nullptr;
     if (with_labels) {
         const tf::Tensor* y;
         TF_RETURN_IF_ERROR(ctx->input("labels", &y));

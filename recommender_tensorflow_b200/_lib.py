@@ -40,14 +40,14 @@ class Config(C.Structure):
                 ("loss_reduction", C.c_int32), ("opt_deep", Optimizer), ("opt_linear", Optimizer),
                 ("max_batch", C.c_int32), ("device", C.c_int32), ("rank", C.c_int32), ("world", C.c_int32),
                 ("nccl_comm", C.c_void_p), ("dropout", C.c_float), ("dropout_seed", C.c_uint64), ("activation", C.c_int32),
-                ("n_src", C.c_int32), ("src", C.POINTER(Column))]
+                ("n_src", C.c_int32), ("src", C.POINTER(Column)), ("weighted", C.c_int32)]
 ACTIVATIONS = {"relu": 0, "tanh": 1, "sigmoid": 2, "identity": 3, "linear": 3, None: 3}
 
 
 class RawBatch(C.Structure):
     _fields_ = [("batch_size", C.c_int32), ("cat_data", C.POINTER(C.c_void_p)),
                 ("cat_offsets", C.POINTER(C.c_void_p)), ("num_data", C.POINTER(C.c_void_p)),
-                ("labels", C.c_void_p)]
+                ("labels", C.c_void_p), ("weights", C.c_void_p)]
 
 
 _SIGS = {

@@ -104,6 +104,7 @@ struct dfm_handle {
     int max_batch = 0, device = 0, rank = 0, world = 1;
     float dropout = 0.f; uint64_t dropout_seed = 0;
     int activation = 0;          // DFM_ACT_*; != ReLU: general CUDA-core tower only
+    bool weighted = false;       // dfm_config.weighted: train batches carry per-example weights
     std::vector<ColDev> cols;
     std::vector<std::string> col_names;
     std::vector<uint32_t> row_off;   // [dc+1]
@@ -502,6 +503,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     h->dropout = cfg->dropout; h->dropout_seed = cfg->dropout_seed;
     if (cfg->activation < DFM_ACT_RELU || cfg->activation > DFM_ACT_IDENTITY) FAIL(DFM_ERR_INVALID_ARG, "activation must be one of DFM_ACT_*");
     h->activation = cfg->activation;
+    h->weighted = cfg->weighted != 0;
     CK(cudaSetDevice(h->device));
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, h->device));
@@ -861,19 +863,19 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                 const int rs = K + 4 + h->emb_slots * K;
                 if (fused_rows_supported(K, m.H[0], h->dc, h->dn) && h->world > 1 && !h->has_bags && h->dropout == 0.f && h->need_emb &&
                     getenv("DFM_NO_FUSED_ROWS") == nullptr) {
-                    h->fr_smem_rb = fused_rows_smem_bytes(m, K, h->dc, h->dn, K + 4);
+                    h->fr_smem_rb = fused_rows_smem_bytes(m, K, h->dc, h->dn, K + 4, h->weighted);
                     if (h->fr_smem_rb <= 227 * 1024) {
                         h->fused_rows_rb = true;
-                        CK(fused_rows_set_attr((int)h->fr_smem_rb));
+                        CK(fused_rows_set_attr((int)h->fr_smem_rb, h->weighted));
                         if (dalloc(h, &h->once_lk, (size_t)h->max_batch * h->dcs)) return DFM_ERR_CUDA;
                     }
                 }
                 if (fused_rows_supported(K, m.H[0], h->dc, h->dn) && h->world == 1 && !h->has_bags && h->dropout == 0.f && h->need_emb &&
                     getenv("DFM_NO_FUSED_ROWS") == nullptr) {
-                    h->fr_smem = fused_rows_smem_bytes(m, K, h->dc, h->dn, rs);
+                    h->fr_smem = fused_rows_smem_bytes(m, K, h->dc, h->dn, rs, h->weighted);
                     if (h->fr_smem <= 227 * 1024) {
                         h->fused_rows = true;
-                        CK(fused_rows_set_attr((int)h->fr_smem));
+                        CK(fused_rows_set_attr((int)h->fr_smem, h->weighted));
                         uint64_t slots = 1024;
                         while (slots < (uint64_t)h->R && slots < (1ull << 26)) slots <<= 1;      // 16 MB at most: L2 resident
                         h->claim_mask = (uint32_t)(slots - 1);
@@ -891,9 +893,14 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                     CK(cudaFree(h->head_part)); h->head_part = nullptr;
                     if (dalloc(h, &h->head_part, (size_t)h->small_grid * 2)) return DFM_ERR_CUDA;
                 }
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                if (h->weighted) {
+                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
+                }
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<8>(K)));
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<16>(K)));
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<32>(K)));
@@ -1093,6 +1100,7 @@ static BatchPtrs make_ptrs(const dfm_handle* h, const dfm_raw_batch* b) {
     }
     for (int j = 0; j < h->dn; ++j) bp.num[j] = b->num_data ? b->num_data[j] : nullptr;
     bp.labels = b->labels;
+    if (h->weighted && b->labels) bp.weights = b->weights;     // an unweighted handle never reads the field
     return bp;
 }
 
@@ -1117,6 +1125,7 @@ static int check_batch(dfm_handle* h, const dfm_raw_batch* b, bool need_labels) 
     for (int j = 0; j < h->dn; ++j)
         if (!b->num_data[j]) FAIL(DFM_ERR_INVALID_ARG, "missing numeric column");
     if (need_labels && !b->labels) FAIL(DFM_ERR_INVALID_ARG, "labels are required for a train step");
+    if (need_labels && h->weighted && !b->weights) FAIL(DFM_ERR_INVALID_ARG, "weights are required for a train step of a weighted model");
     return DFM_OK;
 }
 
@@ -1305,6 +1314,7 @@ template <int K>
 static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t st, const float* labels, float scale,
                         float* logits_out, Phase* ph, const float* rowbuf = nullptr, int64_t upto = -1) {
     const int d = h->dc + h->dn, dK = d * K;
+    const float* wts = labels ? bp.weights : nullptr;     // per-example weights of a weighted train step
     launch_gather<K>(h, bp, B, st, rowbuf, upto);
     if (ph) ph->next();
     const float* hL = nullptr; int H = 0;
@@ -1318,8 +1328,9 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
             smd.drop_keep = 1.f - h->dropout; smd.drop_inv = 1.f / (1.f - h->dropout);
             smd.drop_seed = h->dropout_seed; smd.drop_step = (uint64_t)(h->step + 1); smd.drop_row0 = (int64_t)h->rank * h->max_batch;
         }
-#define SMALL_FWD(HH) small_mlp_fwd_bwd_top_kernel<HH><<<grid, 256, h->small_smem, st>>>(smd, h->dw, h->h0, za, labels, B, scale, train, \
-            h->logits, logits_out, h->dz, h->dact[1], h->up_partial, h->head_part)
+#define SMALL_FWD(HH)                                                                                                               \
+    (wts ? small_mlp_fwd_bwd_top_kernel<HH, true> : small_mlp_fwd_bwd_top_kernel<HH, false>)<<<grid, 256, h->small_smem, st>>>( \
+        smd, h->dw, h->h0, za, labels, wts, B, scale, train, h->logits, logits_out, h->dz, h->dact[1], h->up_partial, h->head_part)
         if (h->sm.H[0] == 8) SMALL_FWD(8); else if (h->sm.H[0] == 16) SMALL_FWD(16); else SMALL_FWD(32);
 #undef SMALL_FWD
         h->launches++;
@@ -1366,8 +1377,10 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
     const float* za = (h->use_linear || h->use_mf) ? h->zacc : nullptr;
     if (h->fused_head && labels) {
         const int grid = std::min(h->fused_head_blocks, (B + 7) / 8);
-#define HEAD_BWD(NHH) head_bwd_kernel<NHH><<<grid, 256, 0, st>>>(za, hL, h->dw + Wo->off, h->dw + bo->off, labels, B, scale, h->logits, logits_out, \
-                                                             h->dz, h->dact[h->L], h->head_part, h->head_gpart, h->dropout > 0.f ? 1.f / (1.f - h->dropout) : 1.f)
+#define HEAD_BWD(NHH)                                                                                                                         \
+    (wts ? head_bwd_kernel<NHH, true> : head_bwd_kernel<NHH, false>)<<<grid, 256, 0, st>>>(                                                   \
+        za, hL, h->dw + Wo->off, h->dw + bo->off, labels, wts, B, scale, h->logits, logits_out, h->dz, h->dact[h->L], h->head_part, h->head_gpart, \
+        h->dropout > 0.f ? 1.f / (1.f - h->dropout) : 1.f)
         switch (H / 32) {
             case 1: HEAD_BWD(1); break; case 2: HEAD_BWD(2); break; case 3: HEAD_BWD(3); break; case 4: HEAD_BWD(4); break;
             case 5: HEAD_BWD(5); break; case 6: HEAD_BWD(6); break; case 7: HEAD_BWD(7); break; default: HEAD_BWD(8); break;
@@ -1376,8 +1389,8 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
         h->launches++;
         return DFM_OK;
     }
-    head_kernel<<<std::min(h->head_blocks, (B + 7) / 8), 256, 0, st>>>(za, hL, H, Wo ? h->dw + Wo->off : nullptr,
-                                                bo ? h->dw + bo->off : nullptr, labels, B, scale, h->logits, logits_out, h->dz, h->head_part);
+    (wts ? head_kernel<true> : head_kernel<false>)<<<std::min(h->head_blocks, (B + 7) / 8), 256, 0, st>>>(
+        za, hL, H, Wo ? h->dw + Wo->off : nullptr, bo ? h->dw + bo->off : nullptr, labels, wts, B, scale, h->logits, logits_out, h->dz, h->head_part);
     h->launches++;
     return DFM_OK;
 }
@@ -1645,6 +1658,7 @@ static FusedArgs make_fused_args(dfm_handle* h, const BatchPtrs& bp, int B, cons
         a.m.drop_seed = h->dropout_seed; a.m.drop_step = (uint64_t)(h->step + 1); a.m.drop_row0 = (int64_t)h->rank * h->max_batch;
     }
     a.labels = labels; a.scale = scale; a.train = train;
+    if (!train) a.bp.weights = nullptr;            // the kernels' W instantiations run exactly when this is set
     a.rr = make_rr(h, rowbuf ? -1 : upto);
     a.od = make_opt(h->od, 0.f); a.ol = make_opt(h->ol, 0.f);
     a.uidx = rowbuf ? h->uidx : nullptr; a.rowbuf = rowbuf; a.rowbuf_stride = K + 4;
@@ -1692,8 +1706,13 @@ static int launch_fused(dfm_handle* h, const BatchPtrs& bp, int B, const float* 
     // (Criteo k=16 [16,..]: 10, ML-100K k=16: 7, ML-100K k=4: 2), the generic bound otherwise
 #define FUSED_GO(HH, NCC)                                                                                              \
     do {                                                                                                               \
-        if (rowbuf) fused_small_kernel<K, HH, true, NCC><<<grid, 256, h->fused_smem, st>>>(a);                         \
-        else fused_small_kernel<K, HH, false, NCC><<<grid, 256, h->fused_smem, st>>>(a);                               \
+        if (a.bp.weights) {                                                                                            \
+            if (rowbuf) fused_small_kernel<K, HH, true, NCC, true><<<grid, 256, h->fused_smem, st>>>(a);               \
+            else fused_small_kernel<K, HH, false, NCC, true><<<grid, 256, h->fused_smem, st>>>(a);                     \
+        } else {                                                                                                       \
+            if (rowbuf) fused_small_kernel<K, HH, true, NCC, false><<<grid, 256, h->fused_smem, st>>>(a);              \
+            else fused_small_kernel<K, HH, false, NCC, false><<<grid, 256, h->fused_smem, st>>>(a);                    \
+        }                                                                                                              \
     } while (0)
     bool done = false;
     if constexpr (K == 16) {
@@ -1714,8 +1733,12 @@ template <int K>
 static int fused_set_attr(dfm_handle* h) {
     const int smem = (int)h->fused_smem;
 #define FUSED_ATTR(HH, NCC)                                                                                                            \
-    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));                \
-    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));         \
+    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));          \
+    if (h->weighted) {                                                                                                                 \
+        CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));      \
+        CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));       \
+    }
     FUSED_ATTR(8, FS_NC) FUSED_ATTR(16, FS_NC) FUSED_ATTR(32, FS_NC)
     if constexpr (K == 16) { FUSED_ATTR(16, 7) FUSED_ATTR(16, 10) }
     if constexpr (K == 4) { FUSED_ATTR(16, 2) }
@@ -2802,6 +2825,8 @@ static int stage_batch(dfm_handle* h, const dfm_raw_batch* b, HostStage& sg, boo
     for (int j = 0; j < h->dn; ++j)
         segs.push_back({reinterpret_cast<const uint8_t*>(b->num_data[j]), (size_t)B * 4, reinterpret_cast<const void**>(&out.num[j])});
     if (need_labels) segs.push_back({reinterpret_cast<const uint8_t*>(b->labels), (size_t)B * 4, reinterpret_cast<const void**>(&out.labels)});
+    if (need_labels && h->weighted)
+        segs.push_back({reinterpret_cast<const uint8_t*>(b->weights), (size_t)B * 4, reinterpret_cast<const void**>(&out.weights)});
     const uint8_t* lo = nullptr; const uint8_t* hi = nullptr; size_t sum = 0;
     for (const Seg& s : segs) {
         if (!lo || s.p < lo) lo = s.p;

@@ -35,6 +35,7 @@ struct BatchPtrs {
     const int32_t* off[DFM_MAX_CAT];
     const float*   num[DFM_MAX_NUM];
     const float*   labels;
+    const float*   weights;      // per-example weights of a weighted handle's train step, else nullptr
 };
 
 // optimizer constants as seen by one step (SURVEY.md A.3)

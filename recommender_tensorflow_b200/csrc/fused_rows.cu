@@ -130,7 +130,9 @@ __device__ __forceinline__ void mma3(float (&cm)[4], float (&cx)[4], const uint3
 // gradient row of a row looked up once in the local batch is stored straight into its owner's gradient segment (peer
 // memory over NVLink, or the local send buffer of the collective path); rows looked up several times are left to
 // row_gsum_kernel, which skips the single ones.
-template <int K, int H1, int ES, bool RB, bool FAST>
+// WGT: weighted model - the producers stage each sample's weight beside its label, and the head multiplies the loss term and
+// dz by it once (after the scale, so w = 1 reproduces the unweighted bits); everything downstream consumes dz as it is.
+template <int K, int H1, int ES, bool RB, bool FAST, bool WGT>
 __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs A) {
     static_assert(!RB || ES == 0, "row-buffer records carry no optimizer slots");
     static_assert(K == 16 && H1 == 16, "instantiated for embedding_size 16 / first hidden layer 16");
@@ -154,6 +156,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
     uint32_t* once = reinterpret_cast<uint32_t*>(smem + L.once);                 // [NSLOT][TS*dc] 1: this kernel applies the row's gradient
     float* xsb = smem + L.xsb;                                   // [NSLOT][TS][dn]
     float* ysb = smem + L.ysb;                                   // [NSLOT][TS] labels (a global load would sit on P3's critical path)
+                                                                 // WGT: followed by [NSLOT][TS] weights
     float* part = smem + L.part;                                 // [CW][TS][H1] layer-0 partials; later the warps' dE staging
     float* p1 = smem + L.p1;                                     // [CW][2K + 4] FM / linear partials of P1
     float* dh1s = smem + L.dh1s;                                 // [TS][H1]
@@ -251,6 +254,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
             if (pw == FR_PW - 1 && lane < FR_TS) {
                 const int b = tile * FR_TS + lane;
                 ysb[s * FR_TS + lane] = (train && b < a.B) ? __ldg(a.labels + b) : 0.f;
+                if constexpr (WGT) ysb[(FR_NSLOT + s) * FR_TS + lane] = (train && b < a.B) ? __ldg(a.bp.weights + b) : 0.f;
             }
 #pragma unroll
             for (int o = 16; o >= 1; o >>= 1) nvalid += __shfl_xor_sync(0xffffffffu, nvalid, o);
@@ -300,6 +304,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
         const uint32_t* onc = once + s * nrows;
         const float* xs = xsb + (size_t)s * FR_TS * dn;
         const float* ys = ysb + s * FR_TS;
+        const float* wsl = ysb + (FR_NSLOT + s) * FR_TS;              // WGT only
         tc::mbar_wait(&full[s], (it / FR_NSLOT) & 1);
         // ------------------------------------------------------------------ P1: two warps per sample: replay in place, FM / linear partial sums
         if (!(A.ablate & 64)) {
@@ -430,6 +435,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
                     const float y = ys[sl];
                     lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
                     gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                    if constexpr (WGT) { gz *= wsl[sl]; lterm *= wsl[sl]; }
                 }
                 if (o == 0) {
                     if (b < a.B) {
@@ -547,6 +553,7 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
                         const float y = ys[sl];
                         lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
                         gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                        if constexpr (WGT) { gz *= wsl[sl]; lterm *= wsl[sl]; }
                         a.dz_out[b] = gz;
                     }
                 }
@@ -967,7 +974,7 @@ void fr_layout(FusedRowsArgs& A, const SmallMlpDesc& m, int K, int dc, int dn) {
     L.rowix = o; o += FR_NSLOT * nrows;
     L.once = o; o += FR_NSLOT * nrows;
     L.xsb = o; o += FR_NSLOT * FR_TS * (dn > 0 ? dn : 1);
-    L.ysb = o; o += FR_NSLOT * FR_TS;
+    L.ysb = o; o += FR_NSLOT * FR_TS * (A.f.bp.weights ? 2 : 1);
     o += (4 - (o & 3)) & 3;
     L.part = o; o += FR_CW * FR_TS * H1;
     L.p1 = o; o += FR_CW * (2 * K + 4);
@@ -983,8 +990,8 @@ void fr_layout(FusedRowsArgs& A, const SmallMlpDesc& m, int K, int dc, int dn) {
     o += o & 1;
     L.bars = o;
 }
-size_t fused_rows_smem_bytes(const SmallMlpDesc& m, int K, int dc, int dn, int rs) {
-    size_t f = (size_t)m.D * FR_W0S + 2 * (size_t)m.up_count + 8;
+size_t fused_rows_smem_bytes(const SmallMlpDesc& m, int K, int dc, int dn, int rs, bool weighted) {
+    size_t f = (size_t)m.D * FR_W0S + 2 * (size_t)m.up_count + 8 + (weighted ? FR_NSLOT * FR_TS : 0);
     f += (size_t)FR_NSLOT * FR_TS * fr_sst(dc, dn, K, rs);
     f += (size_t)FR_NSLOT * (2 * FR_TS * dc + FR_TS * (dn > 0 ? dn : 1) + FR_TS + 8);
     f += (size_t)FR_CW * FR_TS * m.H[0] + (size_t)FR_CW * (2 * K + 4) + (size_t)FR_TS * m.H[0] + 2 * (size_t)FR_TS * m.act_stride + 3 * FR_TS +
@@ -1014,37 +1021,45 @@ int fused_rows_grid(int B, int sm_count, bool side_stream_busy) {
     return std::max(1, std::min(tiles, sm_count - reserve));
 }
 
-template <int ES, bool RB>
+template <int ES, bool RB, bool WGT>
 static cudaError_t fr_attr(int smem_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    return e ? e : cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    cudaError_t e = cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, false, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    return e ? e : cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, true, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
 }
-cudaError_t fused_rows_set_attr(int smem_bytes) {
-    cudaError_t e = fr_attr<0, false>(smem_bytes);
-    if (!e) e = fr_attr<1, false>(smem_bytes);
-    if (!e) e = fr_attr<2, false>(smem_bytes);
-    if (!e) e = fr_attr<0, true>(smem_bytes);
+template <bool WGT>
+static cudaError_t fr_attr_all(int smem_bytes) {
+    cudaError_t e = fr_attr<0, false, WGT>(smem_bytes);
+    if (!e) e = fr_attr<1, false, WGT>(smem_bytes);
+    if (!e) e = fr_attr<2, false, WGT>(smem_bytes);
+    if (!e) e = fr_attr<0, true, WGT>(smem_bytes);
     return e;
 }
-template <int ES, bool RB>
+cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted) {
+    cudaError_t e = fr_attr_all<false>(smem_bytes);
+    return (e || !weighted) ? e : fr_attr_all<true>(smem_bytes);
+}
+template <int ES, bool RB, bool WGT>
 static void fr_go(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
     // FAST: every optimizer step the kernel takes is Adam and every replay is the closed form (row-buffer mode does neither)
     const RowReplay& rr = A.f.rr;
     const bool replay_fast = rr.upto < 0 || (rr.emb_adam && rr.rd.closed && (rr.same || !rr.lin_adam));
     const bool apply_fast = RB || !A.f.train || A.claim == nullptr || (A.od_t.kind == DFM_OPT_ADAM && (!A.f.use_linear || A.ol_t.kind == DFM_OPT_ADAM));
     static const bool allow = getenv("DFM_FR_NO_FAST") == nullptr;
-    if (allow && replay_fast && apply_fast) fused_rows_kernel<16, 16, ES, RB, true><<<grid, FR_THREADS, smem_bytes, st>>>(A);
-    else fused_rows_kernel<16, 16, ES, RB, false><<<grid, FR_THREADS, smem_bytes, st>>>(A);
+    if (allow && replay_fast && apply_fast) fused_rows_kernel<16, 16, ES, RB, true, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
+    else fused_rows_kernel<16, 16, ES, RB, false, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
+}
+template <bool WGT>
+static void fr_go_slots(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
+    if (A.rowbuf_mode) { fr_go<0, true, WGT>(A, grid, smem_bytes, st); return; }
+    switch (A.emb_slots) {
+        case 0: fr_go<0, false, WGT>(A, grid, smem_bytes, st); break;
+        case 1: fr_go<1, false, WGT>(A, grid, smem_bytes, st); break;
+        default: fr_go<2, false, WGT>(A, grid, smem_bytes, st); break;
+    }
 }
 cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
-    if (A.rowbuf_mode) {
-        fr_go<0, true>(A, grid, smem_bytes, st);
-        return cudaGetLastError();
-    }
-    switch (A.emb_slots) {
-        case 0: fr_go<0, false>(A, grid, smem_bytes, st); break;
-        case 1: fr_go<1, false>(A, grid, smem_bytes, st); break;
-        default: fr_go<2, false>(A, grid, smem_bytes, st); break;
-    }
+    // weighted train step (make_fused_args sets the weights pointer only then): the WGT instantiations
+    if (A.f.bp.weights) fr_go_slots<true>(A, grid, smem_bytes, st);
+    else fr_go_slots<false>(A, grid, smem_bytes, st);
     return cudaGetLastError();
 }

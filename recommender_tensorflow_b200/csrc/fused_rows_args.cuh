@@ -42,7 +42,7 @@ __host__ __device__ inline int fr_sst(int dc, int dn, int K, int rs) {
 }
 // host interface (fused_rows.cu)
 bool fused_rows_supported(int K, int H1, int dc, int dn);                     // shape limits of the instantiated kernel
-size_t fused_rows_smem_bytes(const SmallMlpDesc& m, int K, int dc, int dn, int rs);
+size_t fused_rows_smem_bytes(const SmallMlpDesc& m, int K, int dc, int dn, int rs, bool weighted);   // weighted: room for staged weights
 int fused_rows_grid(int B, int sm_count, bool side_stream_busy);                                     // CTAs (= per-CTA partial sets) of a launch
 // Deterministic stream compaction of the step's (row, lookup) pairs: only the lookups whose claim state is "more than
 // once" go through the sort / ordered reduction.  n_out[0] = pairs kept, n_out[1] = once-only lookups.  scratch: n / 2048 + 2 words.
@@ -50,5 +50,5 @@ cudaError_t fused_rows_compact(const uint32_t* keys_in, const uint32_t* vals_in,
                                uint32_t* keys_out, uint32_t* vals_out, uint32_t* scratch, uint32_t* n_out, cudaStream_t st, int64_t* launches);
 void fr_layout(FusedRowsArgs& A, const SmallMlpDesc& m, int K, int dc, int dn);      // needs A.sst
 void fr_balance(FusedRowsArgs& A, int dc, int dn, bool cat_tasks);   // cat_tasks: the kernel applies / forwards the once-only rows' gradients
-cudaError_t fused_rows_set_attr(int smem_bytes);
+cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted);      // weighted: also the W instantiations
 cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st);

@@ -308,9 +308,11 @@ static __global__ void __launch_bounds__(256) numeric_grad_partial_kernel(BatchP
 
 // head: z = zacc + h_L . Wo + bo ; loss_b = max(z,0) - z*y + log1p(exp(-|z|)) ; dz = (sigmoid(z)-y)*scale
 // one warp per sample; per-block partial sums of loss and dz (fixed order inside the block).
-static __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ zacc, const float* __restrict__ hL, int H,
+// WGT: weighted model, loss_b *= w_b and dz = ((sigmoid(z)-y)*scale)*w_b (w = 1 gives the unweighted bits)
+template <bool WGT>
+__global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ zacc, const float* __restrict__ hL, int H,
                                                    const float* __restrict__ Wo, const float* __restrict__ bo,
-                                                   const float* __restrict__ labels, int B, float scale,
+                                                   const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale,
                                                    float* __restrict__ logits, float* __restrict__ logits_out,
                                                    float* __restrict__ dz, float* __restrict__ part /*[grid][2]*/) {
     __shared__ float sl[8], sd[8];
@@ -334,6 +336,7 @@ static __global__ void __launch_bounds__(256) head_kernel(const float* __restric
                 float l = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
                 float sg = 1.f / (1.f + expf(-z));
                 float g = (sg - y) * scale;
+                if constexpr (WGT) { const float w = weights[b]; g *= w; l *= w; }
                 dz[b] = g;
                 lsum += l;
                 dsum += g;
@@ -356,10 +359,10 @@ static __global__ void __launch_bounds__(256) head_kernel(const float* __restric
 // while h_L is still in registers; per-block partial sums (fixed order) of the loss, dz,
 // gWo = h_L^T dz and gb_L = column sums of dh_L'.  Replaces head_kernel + dh_last_kernel + two column-sum
 // launches (and one re-read of h_L).   gpart layout: [grid][2*H] = {gWo | gb_L}
-template <int NH>
+template <int NH, bool WGT>
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ zacc, const float* __restrict__ hL,
                                                        const float* __restrict__ Wo, const float* __restrict__ bo,
-                                                       const float* __restrict__ labels, int B, float scale,
+                                                       const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale,
                                                        float* __restrict__ logits, float* __restrict__ logits_out,
                                                        float* __restrict__ dz, float* __restrict__ dh,
                                                        float* __restrict__ part /*[grid][2]*/, float* __restrict__ gpart,
@@ -388,6 +391,8 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
         }
         const float za0 = zacc ? zacc[b] : 0.f, za1 = (zacc && two) ? zacc[b2] : 0.f;
         const float y0 = labels[b], y1 = two ? labels[b2] : 0.f;
+        float w0 = 1.f, w1 = 1.f;
+        if constexpr (WGT) { w0 = weights[b]; w1 = two ? weights[b2] : 0.f; }
 #pragma unroll
         for (int i = 0; i < NH; ++i) { z[0] = fmaf(h[0][i], wo[i], z[0]); z[1] = fmaf(h[1][i], wo[i], z[1]); }
 #pragma unroll
@@ -398,12 +403,15 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
             const int bb = s2 ? b2 : b;
             const float zz = z[s2] + b0 + (s2 ? za1 : za0);
             const float y = s2 ? y1 : y0;
-            const float g = (1.f / (1.f + expf(-zz)) - y) * scale;
+            float g = (1.f / (1.f + expf(-zz)) - y) * scale;
+            if constexpr (WGT) g *= s2 ? w1 : w0;
             if (lane == 0) {
                 logits[bb] = zz;
                 if (logits_out) logits_out[bb] = zz;
                 dz[bb] = g;
-                lsum += fmaxf(zz, 0.f) - zz * y + log1pf(expf(-fabsf(zz)));
+                float l = fmaxf(zz, 0.f) - zz * y + log1pf(expf(-fabsf(zz)));
+                if constexpr (WGT) l *= s2 ? w1 : w0;
+                lsum += l;
                 dsum += g;
             }
 #pragma unroll

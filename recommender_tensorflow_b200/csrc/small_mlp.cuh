@@ -39,10 +39,11 @@ static inline size_t small_mlp_fwd_smem(const SmallMlpDesc& m) {
 }
 
 // per-sample scratch row layout: [h_1 | h_2 | ... | h_L]; gradients use a second array of the same shape
-template <int H1>
+// WGT: weighted model, the loss term and dz of sample b are multiplied by weights[b] (after the scale: w = 1 is exact)
+template <int H1, bool WGT>
 __global__ void __launch_bounds__(256, 2) small_mlp_fwd_bwd_top_kernel(
     SmallMlpDesc m, const float* __restrict__ dw, const float* __restrict__ h0, const float* __restrict__ zacc,
-    const float* __restrict__ labels, int B, float scale, int train, float* __restrict__ logits,
+    const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale, int train, float* __restrict__ logits,
     float* __restrict__ logits_out, float* __restrict__ dz_out, float* __restrict__ dh1_out,
     float* __restrict__ up_partial /*[grid][up_count]*/, float* __restrict__ head_part /*[grid][2]*/) {
     extern __shared__ __align__(16) float smem[];
@@ -157,6 +158,7 @@ __global__ void __launch_bounds__(256, 2) small_mlp_fwd_bwd_top_kernel(
                     float y = labels[b];
                     lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
                     g = (1.f / (1.f + expf(-z)) - y) * scale;
+                    if constexpr (WGT) { const float w = weights[b]; g *= w; lterm *= w; }
                     dz_out[b] = g;
                 }
             }

@@ -31,11 +31,14 @@ def _default_dtype(d):
 
 
 class GpuCsvReader:
-    def __init__(self, engine, columns, defaults, label_col=None, cutoff=5, max_records=65536, max_bytes=None, field_delim=","):
+    def __init__(self, engine, columns, defaults, label_col=None, cutoff=5, max_records=65536, max_bytes=None, field_delim=",",
+                 weight_col=None):
         """columns / defaults: the CSV schema (names and `record_defaults`, e.g. trainers.ml_100k.COLUMNS / DEFAULTS;
         [0] is int32, [0.0] float32, anything else a string).  Only the fields `engine` consumes (plus the label) are
         materialised; the rest is parsed for structure only.  A numeric column reads a float32 field, or an int32 field
-        converted with tf.to_float.  field_delim: one character, as tf.decode_csv's."""
+        converted with tf.to_float.  field_delim: one character, as tf.decode_csv's.  weight_col: the field holding the
+        per-example weight of a weighted engine (float32, or int32 read as float like a numeric column); the batches
+        point RawBatch.weights at its float32 column."""
         self.lib = _lib.load()
         self.eng = engine
         self.columns = list(columns)
@@ -47,6 +50,9 @@ class GpuCsvReader:
                 raise ValueError("GpuCsvReader: multivalent column %r has no CSV encoding in the reference" % s["source"])
             wanted[s["source"]] = s["dtype"]
         numeric = {c.key for c in engine.num_columns}
+        if weight_col is not None and weight_col not in self.columns:
+            raise KeyError(weight_col)
+        as_float_fields = numeric | ({weight_col} if weight_col is not None else set())
         delim = field_delim.encode() if isinstance(field_delim, str) else bytes(field_delim)
         if len(delim) != 1:
             raise ValueError("field_delim must be one byte, got %r" % (field_delim,))
@@ -60,13 +66,13 @@ class GpuCsvReader:
             dt = _default_dtype(d[0])
             if name in wanted and wanted[name] != dt:
                 raise ValueError("column %r: model expects %s, CSV default %r says otherwise" % (name, wanted[name], d))
-            if name in numeric and dt == "string":
+            if name in as_float_fields and dt == "string":
                 raise ValueError("column %r: numeric column expects float32 or int32, CSV default %r says otherwise" % (name, d))
-            if name in wanted or name in numeric or name == label_col:
+            if name in wanted or name in as_float_fields or name == label_col:
                 kind[j] = {"int32": CSV_INT32, "float32": CSV_FLOAT32, "string": CSV_STRING}[dt]
             else:
                 kind[j] = CSV_SKIP
-            as_float[j] = int(name in numeric and dt == "int32")
+            as_float[j] = int(name in as_float_fields and dt == "int32")
             if dt == "int32":
                 idef[j] = int(d[0])
             elif dt == "float32":
@@ -77,6 +83,7 @@ class GpuCsvReader:
         if missing:
             raise ValueError("model columns missing from the CSV schema: %r" % missing)
         self.label_field = self.columns.index(label_col) if label_col is not None else -1
+        self.weight_field = self.columns.index(weight_col) if weight_col is not None else -1
         self.max_records = int(max_records)
         self.max_bytes = int(max_bytes or 512 * self.max_records)
         cfg = CsvConfig(n, C.cast(kind, C.POINTER(C.c_int32)), C.cast(idef, C.POINTER(C.c_int32)), C.cast(sdef, C.POINTER(C.c_char_p)),
@@ -159,8 +166,9 @@ class GpuCsvReader:
         for j, c in enumerate(eng.num_columns):
             num[j] = self.lib.dfm_csv_float_column(self.h, self._field[c.key])
         lab = self.lib.dfm_csv_labels(self.h) if self.label_field >= 0 else None
+        wgt = self.lib.dfm_csv_float_column(self.h, self.weight_field) if self.weight_field >= 0 else None
         raw = _lib.RawBatch(n, C.cast(cat, C.POINTER(C.c_void_p)), C.cast(off, C.POINTER(C.c_void_p)),
-                            C.cast(num, C.POINTER(C.c_void_p)), lab)
+                            C.cast(num, C.POINTER(C.c_void_p)), lab, wgt)
         return PackedBatch(None, 0, raw, [cat, off, num, self], 0, n, True)
 
     # ---- read-back helpers (tests, debugging) ----
@@ -200,3 +208,9 @@ class GpuCsvReader:
     def labels(self):
         n = int(self.lib.dfm_csv_num_records(self.h))
         return self._d2h(self.lib.dfm_csv_labels(self.h), 4 * n).view(np.float32).copy()
+
+    def weights(self):
+        """float32 [n] per-example weights of the last decode (the weight_col field)"""
+        if self.weight_field < 0:
+            raise ValueError("this reader was created without weight_col")
+        return self.float_column(self.columns[self.weight_field])

@@ -94,7 +94,9 @@ class DeepFMEngine:
     def __init__(self, categorical_columns, numeric_columns=(), embedding_size=4, hidden_units=(16, 16),
                  use_linear=True, use_mf=True, use_dnn=True, loss_reduction="mean", opt_deep=None,
                  opt_linear=None, max_batch=65536, device=0, feature_dtypes=None, sort_columns=True, rank=0, world=1, dropout=0.0, dropout_seed=0,
-                 multivalent=None, activation="relu"):
+                 multivalent=None, activation="relu", weighted=False):
+        """weighted: train batches carry per-example weights (the estimators' weight_column): the per-sample loss and
+        its gradient are multiplied by the weight on the device.  train_step / pack then require `weights`."""
         self.lib = _lib.load()
         # params["activation"] (trainers/deep_fm.py:22): a name, None (identity) or a callable named like a tf.nn activation
         act = activation if (activation is None or isinstance(activation, str)) else getattr(activation, "__name__", str(activation))
@@ -116,6 +118,7 @@ class DeepFMEngine:
         self.max_batch, self.device = int(max_batch), int(device)
         self.rank, self.world = int(rank), int(world)
         self.dropout, self.dropout_seed = float(dropout or 0.0), int(dropout_seed)
+        self.weighted = bool(weighted)
         fd = dict(feature_dtypes or {})
         mv = dict(multivalent or {})      # raw feature key -> value slots per sample (multi-hot / multivalent column)
         self.specs = []
@@ -176,7 +179,8 @@ class DeepFMEngine:
                           C.cast(hid, C.POINTER(C.c_int32)), int(self.use_linear), int(self.use_mf), int(self.use_dnn),
                           _lib.LOSS_RED[loss_reduction], _opt_struct(self.opt_deep), _opt_struct(self.opt_linear),
                           self.max_batch, self.device, self.rank, self.world, None, self.dropout, self.dropout_seed,
-                          _lib.ACTIVATIONS[self.activation], len(self.src_specs), C.cast(srcs, C.POINTER(_lib.Column)))
+                          _lib.ACTIVATIONS[self.activation], len(self.src_specs), C.cast(srcs, C.POINTER(_lib.Column)),
+                          int(self.weighted))
         self._keep += [cols, srcs, hid]
         handle = C.c_void_p()
         rc = self.lib.dfm_create(C.byref(cfg), C.byref(handle))
@@ -425,8 +429,8 @@ class DeepFMEngine:
         self._check(self.lib.dfm_init_random(self.h, seed))
 
     # ------------------------------------------------------------------ batches
-    def _segments(self, features, labels):
-        """-> list of (kind, index, ndarray) in arena order; kind in cat|off|num|lab."""
+    def _segments(self, features, labels, weights=None):
+        """-> list of (kind, index, ndarray) in arena order; kind in cat|off|num|lab|wgt."""
         segs = []
         B = None
         for f, s in enumerate(self.raw_specs):
@@ -464,11 +468,19 @@ class DeepFMEngine:
             segs.append(("num", j, arr))
         if labels is not None:
             segs.append(("lab", 0, np.ascontiguousarray(np.asarray(labels).reshape(-1), dtype=np.float32)))
+            if self.weighted:
+                if weights is None:
+                    raise ValueError("this engine was created with weighted=True: a batch with labels needs weights")
+                w = np.ascontiguousarray(np.asarray(weights).reshape(-1), dtype=np.float32)
+                if w.shape[0] != B:
+                    raise ValueError("weights have %d rows, expected %d" % (w.shape[0], B))
+                segs.append(("wgt", 0, w))
         return segs, B
 
-    def pack(self, features, labels=None, device=False, pinned=True):
-        """Lay the raw columns out in ONE arena so that the H2D transfer is a single copy."""
-        segs, B = self._segments(features, labels)
+    def pack(self, features, labels=None, device=False, pinned=True, weights=None):
+        """Lay the raw columns out in ONE arena so that the H2D transfer is a single copy.  weights: [B] per-example
+        weights, required with labels on a weighted engine and ignored otherwise."""
+        segs, B = self._segments(features, labels, weights)
         offs, total = [], 0
         for _, _, a in segs:
             offs.append(total)
@@ -500,7 +512,7 @@ class DeepFMEngine:
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
         num = (C.c_void_p * nn)()
-        lab = None
+        lab = wgt = None
         for (kind, idx, a), o in zip(segs, offs):
             if kind == "cat":
                 cat[idx] = base + o
@@ -508,10 +520,12 @@ class DeepFMEngine:
                 off[idx] = base + o
             elif kind == "num":
                 num[idx] = base + o
+            elif kind == "wgt":
+                wgt = base + o
             else:
                 lab = base + o
         raw = _lib.RawBatch(B, C.cast(cat, C.POINTER(C.c_void_p)), C.cast(off, C.POINTER(C.c_void_p)),
-                            C.cast(num, C.POINTER(C.c_void_p)), lab)
+                            C.cast(num, C.POINTER(C.c_void_p)), lab, wgt)
         keep += [cat, off, num]
         layout = [(kind, idx, o, a.nbytes) for (kind, idx, a), o in zip(segs, offs)]
         return PackedBatch(arena, base, raw, keep, total, B, device, layout)
@@ -523,7 +537,7 @@ class DeepFMEngine:
         cat = (C.c_void_p * nc)()
         off = (C.c_void_p * nc)()
         num = (C.c_void_p * nn)()
-        lab = None
+        lab = wgt = None
         for kind, idx, o, _ in pb.layout:
             if kind == "cat":
                 cat[idx] = base + o
@@ -531,16 +545,18 @@ class DeepFMEngine:
                 off[idx] = base + o
             elif kind == "num":
                 num[idx] = base + o
+            elif kind == "wgt":
+                wgt = base + o
             else:
                 lab = base + o
         raw = _lib.RawBatch(pb.batch_size, C.cast(cat, C.POINTER(C.c_void_p)), C.cast(off, C.POINTER(C.c_void_p)),
-                            C.cast(num, C.POINTER(C.c_void_p)), lab)
+                            C.cast(num, C.POINTER(C.c_void_p)), lab, wgt)
         return PackedBatch(arena, base, raw, [cat, off, num], pb.nbytes, pb.batch_size, arena.is_cuda, pb.layout)
 
-    def _as_batch(self, features, labels, device=False):
+    def _as_batch(self, features, labels, device=False, weights=None):
         if isinstance(features, PackedBatch):
             return features
-        return self.pack(features, labels, device=device)
+        return self.pack(features, labels, device=device, weights=weights)
 
     # ------------------------------------------------------------------ the hot path
     def transform(self, features):
@@ -552,9 +568,10 @@ class DeepFMEngine:
         self.sync()
         return out.cpu().numpy()
 
-    def train_step(self, features, labels=None, return_logits=False):
-        """One train step from HOST buffers (H2D + step + D2H of the loss)."""
-        pb = self._as_batch(features, labels)
+    def train_step(self, features, labels=None, return_logits=False, weights=None):
+        """One train step from HOST buffers (H2D + step + D2H of the loss).  weights: per-example weights (weighted
+        engines only)."""
+        pb = self._as_batch(features, labels, weights=weights)
         if pb.on_device:
             return self.train_step_device(pb, return_logits)
         loss = C.c_float()

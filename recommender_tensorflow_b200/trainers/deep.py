@@ -4,13 +4,16 @@
 from ..engine import DeepFMEngine, default_optimizer
 from .linear_deep import _CannedBase, canned_parser, canned_train_and_evaluate
 from .ml_100k import FEATURE_DTYPES
+from .model_utils import weight_column_key
 
 _LEARNING_RATE = 0.05
 
 
 class DNNClassifier(_CannedBase):
     def __init__(self, hidden_units, feature_columns, model_dir=None, dropout=None, config=None, max_batch=4096, device=0,
-                 feature_dtypes=FEATURE_DTYPES, tf_random_seed=None):
+                 feature_dtypes=FEATURE_DTYPES, tf_random_seed=None, weight_column=None):
+        weight_column_key(weight_column)        # type check, as TF's constructor does
+        self.weight_column = weight_column
         cols = list(feature_columns)
         if not cols:
             raise ValueError("feature_columns must be defined.")
@@ -21,7 +24,7 @@ class DNNClassifier(_CannedBase):
                                    hidden_units=list(hidden_units), use_linear=False, use_mf=False, use_dnn=True,
                                    loss_reduction="sum", opt_deep=default_optimizer("Adagrad", _LEARNING_RATE),
                                    opt_linear=default_optimizer("Adagrad", _LEARNING_RATE), max_batch=max_batch, device=device,
-                                   feature_dtypes=feature_dtypes, dropout=float(dropout or 0.0))
+                                   feature_dtypes=feature_dtypes, dropout=float(dropout or 0.0), weighted=weight_column is not None)
         self._finish_init(model_dir, tf_random_seed)
 
 

@@ -13,9 +13,9 @@ from collections import namedtuple
 
 import numpy as np
 
-from ..engine import DeepFMEngine
+from ..engine import DeepFMEngine, PackedBatch
 from .ml_100k import FEATURE_DTYPES, ModeKeys, get_feature_columns, get_input_fn
-from .model_utils import get_binary_metrics, get_binary_predictions, get_optimizer
+from .model_utils import get_binary_metrics, get_binary_predictions, get_optimizer, get_weights, weight_column_key
 
 EstimatorSpec = namedtuple("EstimatorSpec", ["mode", "loss", "train_op", "predictions", "eval_metric_ops", "global_step"])
 _ENGINE_KEY = "_b200_engine"
@@ -33,6 +33,9 @@ def _build_engine(params, batch_size):
     dropout = params.get("dropout", 0)
     optimizer = params.get("optimizer", "Adam")
     learning_rate = params.get("learning_rate", 0.001)
+    # weight_column of the binary head (contrib binary_classification_head(weight_column=...)): absent in the
+    # reference's model_fn, so None keeps the unweighted model
+    weighted = weight_column_key(params.get("weight_column")) is not None
     # check params (trainers/deep_fm.py:28-34)
     if (len(categorical_columns) + len(numeric_columns)) == 0:
         raise ValueError("At least 1 feature column of categorical_columns or numeric_columns must be specified.")
@@ -45,7 +48,8 @@ def _build_engine(params, batch_size):
                        use_linear=bool(use_linear), use_mf=bool(use_mf), use_dnn=bool(use_dnn), loss_reduction="mean",
                        opt_deep=opt, opt_linear=dict(opt), max_batch=params.get("max_batch", max(batch_size, 1)),
                        device=params.get("device", 0), feature_dtypes=params.get("feature_dtypes", FEATURE_DTYPES),
-                       dropout=float(dropout or 0.0), dropout_seed=int(params.get("dropout_seed", 0)), activation=activation_fn)
+                       dropout=float(dropout or 0.0), dropout_seed=int(params.get("dropout_seed", 0)), activation=activation_fn,
+                       weighted=weighted)
     # the variable initialisers TF runs when the graph is first executed (truncated normal 1/sqrt(k) for the embedding
     # tables, glorot uniform for the dense kernels, zeros for linear weights and biases); RunConfig.tf_random_seed
     seed = params.get("tf_random_seed")
@@ -65,14 +69,17 @@ def model_fn(features, labels, mode, params):
     engine = params.get(_ENGINE_KEY)
     if engine is None:
         engine = params[_ENGINE_KEY] = _build_engine(params, _batch_size(features))
+    weight_column = params.get("weight_column")
     if mode == ModeKeys.TRAIN:
-        loss, logits = engine.train_step(features, labels, return_logits=True)
+        # a device batch (get_gpu_input_fn) carries its weights inside; a host batch has them among its features
+        weights = None if isinstance(features, PackedBatch) else get_weights(features, weight_column, _batch_size(features))
+        loss, logits = engine.train_step(features, labels, return_logits=True, weights=weights)
         return EstimatorSpec(mode, loss, None, get_binary_predictions(logits), None, engine.global_step)
     logits = engine.predict_logits(features)
     preds = get_binary_predictions(logits)
     if mode == ModeKeys.PREDICT:
         return EstimatorSpec(mode, None, None, preds, None, engine.global_step)
-    metrics = get_binary_metrics(labels, logits)
+    metrics = get_binary_metrics(labels, logits, get_weights(features, weight_column, logits.shape[0]))
     return EstimatorSpec(mode, metrics["average_loss"], None, preds, metrics, engine.global_step)
 
 
@@ -165,7 +172,8 @@ class Estimator:
         return loss
 
     def evaluate(self, input_fn):
-        ys, zs = [], []
+        ys, zs, ws = [], [], []
+        weight_column = self.params.get("weight_column")
         for feats, labels in input_fn():
             if self.engine is None:
                 self.params[_ENGINE_KEY] = _build_engine(self.params, _batch_size(feats))
@@ -173,9 +181,11 @@ class Estimator:
             spec = self.model_fn(feats, labels, ModeKeys.EVAL, self.params)
             ys.append(np.asarray(labels, dtype=np.float32).reshape(-1))
             zs.append(spec.predictions["logits"].reshape(-1))
+            if weight_column is not None:
+                ws.append(get_weights(feats, weight_column, zs[-1].shape[0]))
         if not ys:
             raise ValueError("evaluate(): input_fn yielded no batches")
-        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs))
+        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
         m["global_step"] = self.engine.global_step
         return m
 

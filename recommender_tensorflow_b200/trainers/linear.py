@@ -6,20 +6,23 @@ import math
 from ..engine import DeepFMEngine, default_optimizer
 from .linear_deep import _CannedBase, canned_parser, canned_train_and_evaluate
 from .ml_100k import FEATURE_DTYPES
+from .model_utils import weight_column_key
 
 _LEARNING_RATE = 0.2
 
 
 class LinearClassifier(_CannedBase):
     def __init__(self, feature_columns, model_dir=None, config=None, max_batch=4096, device=0, feature_dtypes=FEATURE_DTYPES,
-                 tf_random_seed=None):
+                 tf_random_seed=None, weight_column=None):
+        weight_column_key(weight_column)        # type check, as TF's constructor does
+        self.weight_column = weight_column
         cols = list(feature_columns)
         if not cols:
             raise ValueError("feature_columns must be defined.")
         lr = min(_LEARNING_RATE, 1.0 / math.sqrt(len(cols)))
         self.engine = DeepFMEngine(cols, (), use_linear=True, use_mf=False, use_dnn=False, loss_reduction="sum",
                                    opt_deep=default_optimizer("Ftrl", lr), opt_linear=default_optimizer("Ftrl", lr),
-                                   max_batch=max_batch, device=device, feature_dtypes=feature_dtypes)
+                                   max_batch=max_batch, device=device, feature_dtypes=feature_dtypes, weighted=weight_column is not None)
         self._finish_init(model_dir, tf_random_seed)      # (linear weights start at zero like TF's; the seed is unused here)
 
 

@@ -7,9 +7,9 @@ import os
 
 import numpy as np
 
-from ..engine import DeepFMEngine, default_optimizer
+from ..engine import DeepFMEngine, PackedBatch, default_optimizer
 from .ml_100k import FEATURE_DTYPES, ModeKeys
-from .model_utils import get_binary_metrics, get_binary_predictions
+from .model_utils import get_binary_metrics, get_binary_predictions, get_weights, weight_column_key
 
 _DNN_LEARNING_RATE = 0.001
 _LINEAR_LEARNING_RATE = 0.005
@@ -20,8 +20,16 @@ class _CannedBase:
     behaviour (resume from model_dir, save at the end of train(), keep_checkpoint_max = 5)."""
     engine = None
     model_dir = None
+    weight_column = None       # weight_column: a feature key or numeric_column whose value weights each example
     KEEP_CHECKPOINT_MAX = 5
     _restored = False
+
+    def _weights(self, feats, n=None):
+        """per-example weights of a host batch (None when unweighted; a device batch carries its own)"""
+        if self.weight_column is None or (n is None and isinstance(feats, PackedBatch)):
+            return None
+        from .deep_fm import _batch_size
+        return get_weights(feats, self.weight_column, _batch_size(feats) if n is None else n)
 
     def _finish_init(self, model_dir, tf_random_seed):
         """Variable initialisers (TF runs them on the first session.run; RunConfig.tf_random_seed): embeddings truncated
@@ -59,7 +67,7 @@ class _CannedBase:
         for feats, labels in input_fn():
             if max_steps is not None and self.engine.global_step >= max_steps:
                 break
-            loss = self.engine.train_step(feats, labels)
+            loss = self.engine.train_step(feats, labels, weights=self._weights(feats))
             if steps is not None:
                 steps -= 1
                 if steps <= 0:
@@ -68,12 +76,14 @@ class _CannedBase:
         return loss
 
     def evaluate(self, input_fn):
-        ys, zs = [], []
+        ys, zs, ws = [], [], []
         self._maybe_restore()
         for feats, labels in input_fn():
             ys.append(np.asarray(labels, dtype=np.float32).reshape(-1))
             zs.append(self.engine.predict_logits(feats))
-        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs))
+            if self.weight_column is not None:
+                ws.append(self._weights(feats, zs[-1].shape[0]))
+        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
         m["global_step"] = self.engine.global_step
         return m
 
@@ -88,7 +98,10 @@ class _CannedBase:
 
 class DNNLinearCombinedClassifier(_CannedBase):
     def __init__(self, model_dir=None, linear_feature_columns=None, dnn_feature_columns=None, dnn_hidden_units=None,
-                 dnn_dropout=None, config=None, max_batch=4096, device=0, feature_dtypes=FEATURE_DTYPES, tf_random_seed=None):
+                 dnn_dropout=None, config=None, max_batch=4096, device=0, feature_dtypes=FEATURE_DTYPES, tf_random_seed=None,
+                 weight_column=None):
+        weight_column_key(weight_column)        # type check, as TF's constructor does
+        self.weight_column = weight_column
         linear_feature_columns = list(linear_feature_columns or [])
         dnn_feature_columns = list(dnn_feature_columns or [])
         if not linear_feature_columns and not dnn_feature_columns:
@@ -107,7 +120,7 @@ class DNNLinearCombinedClassifier(_CannedBase):
                                    opt_deep=default_optimizer("Adagrad", _DNN_LEARNING_RATE),
                                    opt_linear=default_optimizer("Ftrl", lin_lr), max_batch=max_batch, device=device,
                                    dropout=float(dnn_dropout or 0.0),
-                                   feature_dtypes=feature_dtypes)
+                                   feature_dtypes=feature_dtypes, weighted=weight_column is not None)
         self._finish_init(model_dir, tf_random_seed)
 
 

@@ -154,15 +154,19 @@ def _train_index_stream(n_rows, cap, rng):
         yield from buf
 
 
-def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutoff=5, seed=None):
+def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutoff=5, seed=None, weight_column=None):
     """get_input_fn with tf.decode_csv moved to the GPU (SURVEY.md §8f rank 2): the host only selects whole records
     (same shuffle algorithm and RNG stream as get_input_fn, so the same seed gives the same batches); the file itself
     is uploaded once and stays in HBM, a batch travels as 4 bytes per record (its line number); `GpuCsvReader` splits,
     unquotes, parses and thresholds on the device.  Yields
     (PackedBatch on the device, labels): in TRAIN mode labels is None (they are inside the batch), otherwise the
     float32 labels are read back for the metrics.  A record is one text line, as with tf.data.TextLineDataset (a
-    quoted field cannot contain a line break)."""
+    quoted field cannot contain a line break).  weight_column (a field key or numeric_column of a weighted engine): the
+    batches carry that field as their per-example weights; outside TRAIN its host copy is the batch's `weights`
+    attribute, for the weighted metrics."""
     from ..csv_reader import GpuCsvReader
+    from .model_utils import weight_column_key
+    wkey = weight_column_key(weight_column)
 
     def input_fn():
         data = np.fromfile(csv_path, dtype=np.uint8)
@@ -172,13 +176,17 @@ def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutof
         ends = np.concatenate([nl + 1, [data.size]])[:n_lines]
         lens = np.diff(np.concatenate([[0], ends]))[1:]
         max_bytes = int(np.sort(lens)[-batch_size:].sum()) + 16 if n_rows else 16    # bound on one batch's string bytes
-        reader = GpuCsvReader(engine, COLUMNS, DEFAULTS, LABEL_COL, cutoff, max_records=batch_size, max_bytes=max_bytes)
+        reader = GpuCsvReader(engine, COLUMNS, DEFAULTS, LABEL_COL, cutoff, max_records=batch_size, max_bytes=max_bytes, weight_col=wkey)
         if n_rows:
             assert reader.load_file(csv_path) == n_lines                  # the file now lives in HBM, split into lines
 
         def emit(idx):
             pb = reader.decode_lines(np.asarray(idx, dtype=np.int32) + 1)    # +1: line 0 is the header
-            return pb, (None if mode == ModeKeys.TRAIN else reader.labels())
+            if mode == ModeKeys.TRAIN:
+                return pb, None
+            if wkey is not None:
+                pb.weights = reader.weights()
+            return pb, reader.labels()
 
         if mode == ModeKeys.TRAIN:
             rng = np.random.default_rng(seed)

@@ -2,6 +2,7 @@
 import numpy as np
 
 from ..engine import default_optimizer
+from ..feature_column import NumericColumn
 
 
 def layer_summary(value):
@@ -25,16 +26,56 @@ def get_binary_predictions(logits):
             "class_ids": (logistic > 0.5).astype(np.int64), "class_id": (logistic > 0.5).astype(np.int32)}
 
 
-def _auc(labels, probs, curve="ROC", num_thresholds=200):
-    """tf.metrics.auc: trapezoidal over num_thresholds evenly spaced thresholds (+/- epsilon ends)."""
+def weight_column_key(weight_column):
+    """weight_column of the estimators / binary head: None, a feature key or a numeric_column -> the feature key or None"""
+    if weight_column is None:
+        return None
+    if isinstance(weight_column, str):
+        return weight_column
+    if isinstance(weight_column, NumericColumn):
+        return weight_column.key
+    raise TypeError("Weight column must be either a string or _NumericColumn. Given type: {}.".format(type(weight_column)))
+
+
+def get_weights(features, weight_column, n):
+    """head.py _get_weights_and_check_match_logits (TF 1.12): the weight feature as float32 [n] (tf.to_float).  A missing
+    feature raises KeyError, weights whose shape does not match the n logits ([n] or [n, 1]) raise ValueError.  Zero,
+    negative and fractional weights are accepted, as in TF.  A device batch (PackedBatch) carries its weights inside
+    the batch; its host copy, when one was read back for the metrics, is its `weights` attribute."""
+    key = weight_column_key(weight_column)
+    if key is None:
+        return None
+    if isinstance(features, dict):
+        if key not in features:
+            raise KeyError(key)
+        w = features[key]
+    else:
+        w = getattr(features, "weights", None)
+        if w is None:
+            raise KeyError(key)
+    w = np.asarray(w).astype(np.float32)
+    if w.shape not in ((n,), (n, 1)):
+        raise ValueError("weights shape must be [D0, 1] or [D0] matching logits [%d, 1]; got %s" % (n, list(w.shape)))
+    return w.reshape(-1)
+
+
+def _auc(labels, probs, curve="ROC", num_thresholds=200, weights=None):
+    """tf.metrics.auc: trapezoidal over num_thresholds evenly spaced thresholds (+/- epsilon ends).  weights: the
+    confusion counts are sums of the per-example weights."""
     eps = 1e-7
     th = np.concatenate([[0.0 - eps], (np.arange(1, num_thresholds - 1)) / (num_thresholds - 1.0), [1.0 + eps]])
     pos = labels > 0.5
     pred = probs[None, :] > th[:, None]
-    tp = (pred & pos[None, :]).sum(1).astype(np.float64)
-    fp = (pred & ~pos[None, :]).sum(1).astype(np.float64)
-    fn = pos.sum() - tp
-    tn = (~pos).sum() - fp
+    if weights is None:
+        tp = (pred & pos[None, :]).sum(1).astype(np.float64)
+        fp = (pred & ~pos[None, :]).sum(1).astype(np.float64)
+        fn = pos.sum() - tp
+        tn = (~pos).sum() - fp
+    else:
+        tp = (pred & pos[None, :]).astype(np.float64) @ weights
+        fp = (pred & ~pos[None, :]).astype(np.float64) @ weights
+        fn = weights[pos].sum() - tp
+        tn = weights[~pos].sum() - fp
     if curve == "ROC":
         x = fp / (fp + tn + eps)
         y = (tp + eps) / (tp + fn + eps)
@@ -44,13 +85,23 @@ def _auc(labels, probs, curve="ROC", num_thresholds=200):
     return float(np.sum((x[:-1] - x[1:]) * (y[:-1] + y[1:]) / 2.0))
 
 
-def get_binary_metrics(labels, logits):
+def get_binary_metrics(labels, logits, weights=None):
     """Metrics the binary head reports in EVAL mode (accuracy, auc, auc_precision_recall,
-    average_loss, label/mean, prediction/mean; cf. trainers/model_utils.py:39-54)."""
+    average_loss, label/mean, prediction/mean; cf. trainers/model_utils.py:39-54).  weights (weight_column, head.py
+    _eval_metric_ops): every metric is weighted - means are sum(w x) / sum(w), the AUC confusion counts are sums of
+    weights, and loss is sum(w l)."""
     y = np.asarray(labels, dtype=np.float64).reshape(-1)
     z = np.asarray(logits, dtype=np.float64).reshape(-1)
     p = 1.0 / (1.0 + np.exp(-z))
     loss = np.maximum(z, 0) - z * y + np.log1p(np.exp(-np.abs(z)))
+    if weights is not None:
+        w = np.asarray(weights, dtype=np.float32).astype(np.float64).reshape(-1)
+        if w.shape != y.shape:
+            raise ValueError("weights shape %s does not match labels %s" % (list(w.shape), list(y.shape)))
+        sw = w.sum()
+        return {"accuracy": float((w * ((p > 0.5) == (y > 0.5))).sum() / sw), "auc": _auc(y, p, weights=w),
+                "auc_precision_recall": _auc(y, p, "PR", weights=w), "average_loss": float((w * loss).sum() / sw),
+                "loss": float((w * loss).sum()), "label/mean": float((w * y).sum() / sw), "prediction/mean": float((w * p).sum() / sw)}
     return {"accuracy": float(((p > 0.5) == (y > 0.5)).mean()), "auc": _auc(y, p), "auc_precision_recall": _auc(y, p, "PR"),
             "average_loss": float(loss.mean()), "loss": float(loss.sum()), "label/mean": float(y.mean()),
             "prediction/mean": float(p.mean())}
