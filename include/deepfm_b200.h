@@ -131,6 +131,13 @@ typedef struct {
      * (trainers/deep_fm.py:102-103).  Own counter-based generator keyed on (seed, step, layer, element);
      * TF's RNG stream is not reproducible, the oracle restates this one. */
     float             dropout;
+    /* the head (TF 1.12 contrib binary_classification_head / regression_head, canned *Classifier / *Regressor):
+     * DFM_HEAD_LOGISTIC (0, a zeroed config): l_b = sigmoid cross-entropy, dz_b = sigmoid(z_b) - y_b, y in {0, 1}.
+     * DFM_HEAD_SQUARED: l_b = (y_b - z_b)^2, dz_b = 2 (z_b - y_b), y any float32 (label_dimension 1, identity inverse
+     * link: the prediction is the logit).  Then the loss_reduction scale, then the weight, as for the logistic head.
+     * Any other value -> DFM_ERR_INVALID_ARG.  It fills the alignment gap before dropout_seed, so the size of the
+     * struct and the offset of every other field are what they were without it. */
+    int32_t           head;
     uint64_t          dropout_seed;
     /* params["activation"] (trainers/deep_fm.py:22,100; default tf.nn.relu): DFM_ACT_*.  Anything but ReLU runs the
      * general CUDA-core tower (the fused and tensor-core towers are built around the ReLU mask). */
@@ -148,6 +155,9 @@ typedef struct {
     int32_t           weighted;
 } dfm_config;
 
+#define DFM_HEAD_LOGISTIC 0
+#define DFM_HEAD_SQUARED  1
+
 /* One batch of raw (un-hashed) feature columns = what input_fn's parse_csv yields
  * (trainers/ml_100k.py:44-49) for the columns the model consumes. */
 typedef struct {
@@ -156,7 +166,8 @@ typedef struct {
                                            of a crossed column is ignored (may be NULL), source columns follow cat */
     const int32_t* const* cat_offsets;  /* [n_cat + n_src]: int32[B+1] byte offsets for string columns, else NULL */
     const float* const*   num_data;     /* [n_num]: float32[B] */
-    const float*          labels;       /* [B] 0/1 (rating >= cutoff, trainers/ml_100k.py:48); NULL for forward */
+    const float*          labels;       /* [B] float32 labels; NULL for forward.  The logistic head takes 0/1 (rating >=
+                                           cutoff, trainers/ml_100k.py:48), the squared head any value (the rating) */
     /* [B] float32 per-example weights, on the same side (host / device) as labels.  Read only by a handle created with
      * dfm_config.weighted != 0, and only by train steps (required there: NULL -> DFM_ERR_INVALID_ARG); forward,
      * PREDICT and layer_summary ignore it.  An unweighted handle never reads this field. */
@@ -343,7 +354,7 @@ int dfm_test_tc_gemm(int32_t mode, const float* A_dev, const float* B_dev, float
  * reference's input_fn (trainers/ml_100k.py:44-58; schema COLUMNS / DEFAULTS, trainers/ml_100k.py:3-15) for the
  * fields the model consumes.  The host hands over whole records (lines); field splitting, RFC-4180 unquoting
  * ('""' inside a quoted field), int32 and float32 parsing, default substitution for empty fields and the label
- * threshold (rating >= cutoff, trainers/ml_100k.py:47-48) run on the device.  The decoded columns stay in the
+ * threshold (rating >= cutoff, trainers/ml_100k.py:47-48; or the raw rating with label_raw) run on the device.  The decoded columns stay in the
  * reader's device buffers in the layout dfm_raw_batch takes: int32[n] and float32[n] columns, Arrow-style string
  * columns (int32 offsets[n+1] + bytes), float labels[n].  Float32 fields follow TF 1.12's strings::safe_strtof,
  * correctly rounded (oracle/strtof.py states the grammar), except that hexadecimal is rejected.  Errors follow
@@ -362,7 +373,7 @@ typedef struct {
     const int32_t*     kind;           /* [n_fields] DFM_CSV_* */
     const int32_t*     int_default;    /* [n_fields] value of an empty int32 field (NULL: 0) */
     const char* const* str_default;    /* [n_fields] value of an empty string field (NULL entries: "") */
-    int32_t            label_field;    /* int32 field the label is derived from, -1: none */
+    int32_t            label_field;    /* int32 field the label is derived from (float32 too with label_raw), -1: none */
     int32_t            label_min;      /* label = value >= label_min */
     int32_t            max_records;    /* per decode call */
     int64_t            max_bytes;      /* per decode call, < 4 GiB */
@@ -371,6 +382,9 @@ typedef struct {
     int32_t            field_delim;    /* field separator, one byte other than '"', '\n' and '\r' (0: ',') */
     const int32_t*     as_float;       /* [n_fields] nonzero on an int32 field: also write it as float32, rounded to
                                           nearest (tf.to_float of a numeric_column over an int field); NULL: none */
+    int32_t            label_raw;      /* nonzero: the label is the label field's value as float32 (tf.to_float: an
+                                          int32 field rounded to nearest, or a float32 field) and label_min is not
+                                          used - the regression head's label.  0: label = value >= label_min */
 } dfm_csv_config;
 typedef struct dfm_csv_reader dfm_csv_reader;
 int dfm_csv_create(const dfm_csv_config* cfg, dfm_csv_reader** out);

@@ -115,6 +115,8 @@ tf::Status Collect(tf::OpKernelContext* ctx, const std::vector<int>& cat_order, 
     // op creates unweighted handles and has no weights input yet
     b->raw.weights = nullptr;
     if (with_labels) {
+        // float32 labels as they are: 0/1 for a handle with the logistic head, any value (the rating) for one created
+        // with dfm_config.head = DFM_HEAD_SQUARED; the head belongs to the handle, the op needs no attr for it
         const tf::Tensor* y;
         TF_RETURN_IF_ERROR(ctx->input("labels", &y));
         b->raw.labels = y->flat<float>().data();

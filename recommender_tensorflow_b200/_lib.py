@@ -39,9 +39,10 @@ class Config(C.Structure):
                 ("use_linear", C.c_int32), ("use_mf", C.c_int32), ("use_dnn", C.c_int32),
                 ("loss_reduction", C.c_int32), ("opt_deep", Optimizer), ("opt_linear", Optimizer),
                 ("max_batch", C.c_int32), ("device", C.c_int32), ("rank", C.c_int32), ("world", C.c_int32),
-                ("nccl_comm", C.c_void_p), ("dropout", C.c_float), ("dropout_seed", C.c_uint64), ("activation", C.c_int32),
-                ("n_src", C.c_int32), ("src", C.POINTER(Column)), ("weighted", C.c_int32)]
+                ("nccl_comm", C.c_void_p), ("dropout", C.c_float), ("head", C.c_int32), ("dropout_seed", C.c_uint64),
+                ("activation", C.c_int32), ("n_src", C.c_int32), ("src", C.POINTER(Column)), ("weighted", C.c_int32)]
 ACTIVATIONS = {"relu": 0, "tanh": 1, "sigmoid": 2, "identity": 3, "linear": 3, None: 3}
+HEADS = {"logistic": 0, "squared": 1}       # DFM_HEAD_*
 
 
 class RawBatch(C.Structure):

@@ -35,6 +35,12 @@ static int build_replay(dfm_handle* h, int64_t cap);
 static RowReplay make_rr(const dfm_handle* h, int64_t upto);
 template <int K> static int fused_set_attr(dfm_handle* h);
 static bool tc_presplit();
+template <bool SQ, bool WGT>
+static cudaError_t small_mlp_set_attr(int smem) {
+    cudaError_t e = cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (!e) e = cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    return e ? e : cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+}
 // Split count of the weight-gradient GEMM (reduction over the batch).  tcgen05 aligns and TRUNCATES the products it
 // folds into the fp32 TMEM accumulator: measured bias ~3e-8 x (products in the chain) relative to the accumulated
 // magnitude (1.9e-5 after an 8 192-row chain of random operands, tests/test_gpu_tc_gemm.py; an fp32 reference: 3.5e-7).
@@ -105,6 +111,7 @@ struct dfm_handle {
     float dropout = 0.f; uint64_t dropout_seed = 0;
     int activation = 0;          // DFM_ACT_*; != ReLU: general CUDA-core tower only
     bool weighted = false;       // dfm_config.weighted: train batches carry per-example weights
+    bool squared = false;        // dfm_config.head == DFM_HEAD_SQUARED: train steps run the SQ head instantiations
     std::vector<ColDev> cols;
     std::vector<std::string> col_names;
     std::vector<uint32_t> row_off;   // [dc+1]
@@ -504,6 +511,8 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
     if (cfg->activation < DFM_ACT_RELU || cfg->activation > DFM_ACT_IDENTITY) FAIL(DFM_ERR_INVALID_ARG, "activation must be one of DFM_ACT_*");
     h->activation = cfg->activation;
     h->weighted = cfg->weighted != 0;
+    if (cfg->head != DFM_HEAD_LOGISTIC && cfg->head != DFM_HEAD_SQUARED) FAIL(DFM_ERR_INVALID_ARG, "head must be one of DFM_HEAD_*");
+    h->squared = cfg->head == DFM_HEAD_SQUARED;
     CK(cudaSetDevice(h->device));
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, h->device));
@@ -866,7 +875,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                     h->fr_smem_rb = fused_rows_smem_bytes(m, K, h->dc, h->dn, K + 4, h->weighted);
                     if (h->fr_smem_rb <= 227 * 1024) {
                         h->fused_rows_rb = true;
-                        CK(fused_rows_set_attr((int)h->fr_smem_rb, h->weighted));
+                        CK(fused_rows_set_attr((int)h->fr_smem_rb, h->weighted, h->squared));
                         if (dalloc(h, &h->once_lk, (size_t)h->max_batch * h->dcs)) return DFM_ERR_CUDA;
                     }
                 }
@@ -875,7 +884,7 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                     h->fr_smem = fused_rows_smem_bytes(m, K, h->dc, h->dn, rs, h->weighted);
                     if (h->fr_smem <= 227 * 1024) {
                         h->fused_rows = true;
-                        CK(fused_rows_set_attr((int)h->fr_smem, h->weighted));
+                        CK(fused_rows_set_attr((int)h->fr_smem, h->weighted, h->squared));
                         uint64_t slots = 1024;
                         while (slots < (uint64_t)h->R && slots < (1ull << 26)) slots <<= 1;      // 16 MB at most: L2 resident
                         h->claim_mask = (uint32_t)(slots - 1);
@@ -893,14 +902,10 @@ static int create_impl(const dfm_config* cfg, dfm_handle* h) {
                     CK(cudaFree(h->head_part)); h->head_part = nullptr;
                     if (dalloc(h, &h->head_part, (size_t)h->small_grid * 2)) return DFM_ERR_CUDA;
                 }
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                if (h->weighted) {
-                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                    CK(cudaFuncSetAttribute(small_mlp_fwd_bwd_top_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->small_smem));
-                }
+                CK((small_mlp_set_attr<false, false>((int)h->small_smem)));
+                if (h->weighted) CK((small_mlp_set_attr<false, true>((int)h->small_smem)));
+                if (h->squared) CK((small_mlp_set_attr<true, false>((int)h->small_smem)));
+                if (h->weighted && h->squared) CK((small_mlp_set_attr<true, true>((int)h->small_smem)));
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<8>(K)));
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<16>(K)));
                 CK(cudaFuncSetAttribute(small_mlp_bwd_input_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_mlp_bwd_smem<32>(K)));
@@ -1315,6 +1320,7 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
                         float* logits_out, Phase* ph, const float* rowbuf = nullptr, int64_t upto = -1) {
     const int d = h->dc + h->dn, dK = d * K;
     const float* wts = labels ? bp.weights : nullptr;     // per-example weights of a weighted train step
+    const bool sq = labels && h->squared;                 // squared head of a train step (a forward forms no loss)
     launch_gather<K>(h, bp, B, st, rowbuf, upto);
     if (ph) ph->next();
     const float* hL = nullptr; int H = 0;
@@ -1329,7 +1335,8 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
             smd.drop_seed = h->dropout_seed; smd.drop_step = (uint64_t)(h->step + 1); smd.drop_row0 = (int64_t)h->rank * h->max_batch;
         }
 #define SMALL_FWD(HH)                                                                                                               \
-    (wts ? small_mlp_fwd_bwd_top_kernel<HH, true> : small_mlp_fwd_bwd_top_kernel<HH, false>)<<<grid, 256, h->small_smem, st>>>( \
+    (wts ? (sq ? small_mlp_fwd_bwd_top_kernel<HH, true, true> : small_mlp_fwd_bwd_top_kernel<HH, false, true>)                      \
+         : (sq ? small_mlp_fwd_bwd_top_kernel<HH, true, false> : small_mlp_fwd_bwd_top_kernel<HH, false, false>))<<<grid, 256, h->small_smem, st>>>( \
         smd, h->dw, h->h0, za, labels, wts, B, scale, train, h->logits, logits_out, h->dz, h->dact[1], h->up_partial, h->head_part)
         if (h->sm.H[0] == 8) SMALL_FWD(8); else if (h->sm.H[0] == 16) SMALL_FWD(16); else SMALL_FWD(32);
 #undef SMALL_FWD
@@ -1378,7 +1385,8 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
     if (h->fused_head && labels) {
         const int grid = std::min(h->fused_head_blocks, (B + 7) / 8);
 #define HEAD_BWD(NHH)                                                                                                                         \
-    (wts ? head_bwd_kernel<NHH, true> : head_bwd_kernel<NHH, false>)<<<grid, 256, 0, st>>>(                                                   \
+    (wts ? (sq ? head_bwd_kernel<NHH, true, true> : head_bwd_kernel<NHH, false, true>)                                                       \
+         : (sq ? head_bwd_kernel<NHH, true, false> : head_bwd_kernel<NHH, false, false>))<<<grid, 256, 0, st>>>(                                \
         za, hL, h->dw + Wo->off, h->dw + bo->off, labels, wts, B, scale, h->logits, logits_out, h->dz, h->dact[h->L], h->head_part, h->head_gpart, \
         h->dropout > 0.f ? 1.f / (1.f - h->dropout) : 1.f)
         switch (H / 32) {
@@ -1389,7 +1397,8 @@ static int forward_impl(dfm_handle* h, const BatchPtrs& bp, int B, cudaStream_t 
         h->launches++;
         return DFM_OK;
     }
-    (wts ? head_kernel<true> : head_kernel<false>)<<<std::min(h->head_blocks, (B + 7) / 8), 256, 0, st>>>(
+    (wts ? (sq ? head_kernel<true, true> : head_kernel<false, true>) : (sq ? head_kernel<true, false> : head_kernel<false, false>))
+        <<<std::min(h->head_blocks, (B + 7) / 8), 256, 0, st>>>(
         za, hL, H, Wo ? h->dw + Wo->off : nullptr, bo ? h->dw + bo->off : nullptr, labels, wts, B, scale, h->logits, logits_out, h->dz, h->head_part);
     h->launches++;
     return DFM_OK;
@@ -1688,11 +1697,17 @@ static int launch_fused_rows(dfm_handle* h, const BatchPtrs& bp, int B, const fl
         fr_layout(A, h->sm, K, h->dc, h->dn);
         fr_balance(A, h->dc, h->dn, A.f.train && (A.rowbuf_mode || A.claim != nullptr));
         const int grid = fused_rows_grid(B, h->sm_count, rowbuf ? false : h->fr_side);
-        CK(fused_rows_launch(A, grid, rowbuf ? h->fr_smem_rb : h->fr_smem, st));
+        CK(fused_rows_launch(A, grid, rowbuf ? h->fr_smem_rb : h->fr_smem, st, h->squared));
         h->launches++;
         return DFM_OK;
     }
     return DFM_ERR_UNSUPPORTED;
+}
+
+template <int K, int HH, int NCC, bool SQ, bool WGT>
+static void fused_go(const FusedArgs& a, bool rowbuf, int grid, size_t smem, cudaStream_t st) {
+    if (rowbuf) fused_small_kernel<K, HH, true, NCC, SQ, WGT><<<grid, 256, smem, st>>>(a);
+    else fused_small_kernel<K, HH, false, NCC, SQ, WGT><<<grid, 256, smem, st>>>(a);
 }
 
 template <int K>
@@ -1704,14 +1719,15 @@ static int launch_fused(dfm_handle* h, const BatchPtrs& bp, int B, const float* 
     const int need_nc = ((h->dc + h->dn) + (256 / (H1 / 4)) / K - 1) / ((256 / (H1 / 4)) / K);     // ceil(d / fields per column group)
     // NC (dW0 columns per thread) is a compile-time bound: exact instantiations for the shapes BASELINE.json names
     // (Criteo k=16 [16,..]: 10, ML-100K k=16: 7, ML-100K k=4: 2), the generic bound otherwise
+    const bool sq = h->squared && a.train;      // squared head of a train step (a forward forms no loss)
 #define FUSED_GO(HH, NCC)                                                                                              \
     do {                                                                                                               \
         if (a.bp.weights) {                                                                                            \
-            if (rowbuf) fused_small_kernel<K, HH, true, NCC, true><<<grid, 256, h->fused_smem, st>>>(a);               \
-            else fused_small_kernel<K, HH, false, NCC, true><<<grid, 256, h->fused_smem, st>>>(a);                     \
+            if (sq) fused_go<K, HH, NCC, true, true>(a, rowbuf != nullptr, grid, h->fused_smem, st);                   \
+            else fused_go<K, HH, NCC, false, true>(a, rowbuf != nullptr, grid, h->fused_smem, st);                     \
         } else {                                                                                                       \
-            if (rowbuf) fused_small_kernel<K, HH, true, NCC, false><<<grid, 256, h->fused_smem, st>>>(a);              \
-            else fused_small_kernel<K, HH, false, NCC, false><<<grid, 256, h->fused_smem, st>>>(a);                    \
+            if (sq) fused_go<K, HH, NCC, true, false>(a, rowbuf != nullptr, grid, h->fused_smem, st);                  \
+            else fused_go<K, HH, NCC, false, false>(a, rowbuf != nullptr, grid, h->fused_smem, st);                    \
         }                                                                                                              \
     } while (0)
     bool done = false;
@@ -1729,16 +1745,21 @@ static int launch_fused(dfm_handle* h, const BatchPtrs& bp, int B, const float* 
     return DFM_OK;
 }
 
+template <int K, int HH, int NCC, bool SQ, bool WGT>
+static cudaError_t fused_attr(int smem) {
+    cudaError_t e = cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    return e ? e : cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+}
+
 template <int K>
 static int fused_set_attr(dfm_handle* h) {
     const int smem = (int)h->fused_smem;
+    // the WGT / SQ instantiations only on handles that can launch them, as for the small tower
 #define FUSED_ATTR(HH, NCC)                                                                                                            \
-    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));         \
-    CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));          \
-    if (h->weighted) {                                                                                                                 \
-        CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, false, NCC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));      \
-        CK(cudaFuncSetAttribute(fused_small_kernel<K, HH, true, NCC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));       \
-    }
+    CK((fused_attr<K, HH, NCC, false, false>(smem)));                                                                                  \
+    if (h->weighted) CK((fused_attr<K, HH, NCC, false, true>(smem)));                                                                  \
+    if (h->squared) CK((fused_attr<K, HH, NCC, true, false>(smem)));                                                                   \
+    if (h->weighted && h->squared) CK((fused_attr<K, HH, NCC, true, true>(smem)));
     FUSED_ATTR(8, FS_NC) FUSED_ATTR(16, FS_NC) FUSED_ATTR(32, FS_NC)
     if constexpr (K == 16) { FUSED_ATTR(16, 7) FUSED_ATTR(16, 10) }
     if constexpr (K == 4) { FUSED_ATTR(16, 2) }

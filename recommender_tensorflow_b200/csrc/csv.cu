@@ -409,6 +409,7 @@ __global__ void __launch_bounds__(256) csv_copy_strings_kernel(const char* __res
 
 struct dfm_csv_reader {
     int device = 0, n_fields = 0, n_int = 0, n_str = 0, n_float = 0, label_field = -1, label_min = 0;
+    bool label_raw = false;      // dfm_csv_config.label_raw: labels are the label field's float32 column
     char delim = ',';
     int32_t max_records = 0;
     int64_t max_bytes = 0;
@@ -497,13 +498,16 @@ extern "C" int dfm_csv_create(const dfm_csv_config* cfg, dfm_csv_reader** out) {
     r->device = cfg->device; r->n_fields = cfg->n_fields; r->max_records = cfg->max_records;
     r->max_bytes = (cfg->max_bytes + 15) / 16 * 16;
     r->label_field = cfg->label_field; r->label_min = cfg->label_min;
+    r->label_raw = cfg->label_raw != 0 && cfg->label_field >= 0;
     std::vector<int32_t> int_default(cfg->n_fields, 0), def_off(cfg->n_fields + 1, 0);
     std::vector<uint32_t> float_default(cfg->n_fields, 0);
     std::string def_bytes;
     for (int f = 0; f < cfg->n_fields; ++f) {
         const int k = cfg->kind[f];
         r->kind.push_back(k);
-        r->fslot.push_back(k == DFM_CSV_FLOAT32 || (k == DFM_CSV_INT32 && cfg->as_float && cfg->as_float[f]) ? r->n_float++ : -1);
+        // a raw int32 label is written as float32 like an as_float field: that column is the labels
+        const bool int_as_float = (cfg->as_float && cfg->as_float[f]) || (r->label_raw && f == r->label_field);
+        r->fslot.push_back(k == DFM_CSV_FLOAT32 || (k == DFM_CSV_INT32 && int_as_float) ? r->n_float++ : -1);
         if (k == DFM_CSV_INT32) {
             r->slot.push_back(r->n_int++);
             if (cfg->int_default) int_default[f] = cfg->int_default[f];
@@ -522,9 +526,11 @@ extern "C" int dfm_csv_create(const dfm_csv_config* cfg, dfm_csv_reader** out) {
         }
         def_off[f + 1] = (int32_t)def_bytes.size();
     }
-    if (r->label_field >= 0 && (r->label_field >= cfg->n_fields || r->kind[r->label_field] != DFM_CSV_INT32)) {
+    if (r->label_field >= 0 && (r->label_field >= cfg->n_fields ||
+                                (r->kind[r->label_field] != DFM_CSV_INT32 && !(r->label_raw && r->kind[r->label_field] == DFM_CSV_FLOAT32)))) {
         delete r;
-        CSV_FAIL((dfm_csv_reader*)nullptr, DFM_ERR_INVALID_ARG, "dfm_csv_create: label_field must be an int32 field");
+        CSV_FAIL((dfm_csv_reader*)nullptr, DFM_ERR_INVALID_ARG,
+                 "dfm_csv_create: label_field must be an int32 field (or a float32 field with label_raw)");
     }
     *out = r;     // from here on dfm_csv_destroy cleans up
 #define CR(call)                                                                                                  \
@@ -606,7 +612,8 @@ static int csv_split_lines(dfm_csv_reader* r, const char* text_dev, int64_t n_by
 static int csv_parse_records(dfm_csv_reader* r, const char* text_dev, const uint32_t* line_start, const int32_t* line_idx, int64_t n_rec,
                              int32_t* n_records_out, cudaStream_t st) {
     CSV_CK(r, cudaMemsetAsync(r->d_err, 0xff, 8, st));
-    CsvDev cfg{r->n_fields, r->d_kind, r->d_slot, r->d_int_default, r->d_def_off, r->d_def_bytes, r->label_field, r->label_min, (int)r->delim,
+    // label_raw: the labels are a float column the kernel writes anyway, so it forms no thresholded label
+    CsvDev cfg{r->n_fields, r->d_kind, r->d_slot, r->d_int_default, r->d_def_off, r->d_def_bytes, r->label_raw ? -1 : r->label_field, r->label_min, (int)r->delim,
                r->d_fslot, r->d_float_default};
     auto parse = r->n_float ? csv_parse_kernel<true> : csv_parse_kernel<false>;
     parse<<<(unsigned)((n_rec + 127) / 128), 128, 0, st>>>(text_dev, line_start, line_idx, (uint32_t)n_rec, cfg, r->d_int_out, r->d_str_pos, r->d_str_off,
@@ -734,4 +741,7 @@ extern "C" const float* dfm_csv_float_column(const dfm_csv_reader* r, int32_t fi
     if (!r || field < 0 || field >= r->n_fields || r->fslot[field] < 0) return nullptr;
     return r->float_out[r->fslot[field]];
 }
-extern "C" const float* dfm_csv_labels(const dfm_csv_reader* r) { return r ? r->labels : nullptr; }
+extern "C" const float* dfm_csv_labels(const dfm_csv_reader* r) {
+    if (!r) return nullptr;
+    return r->label_raw ? r->float_out[r->fslot[r->label_field]] : r->labels;
+}

@@ -29,6 +29,15 @@ __host__ __device__ __forceinline__ uint64_t vocab_mix(uint64_t k) {
     return k ^ (k >> 31);
 }
 
+// squared head (DFM_HEAD_SQUARED; TF 1.12 regression_head: mean_squared_error unreduced, label_dimension 1):
+// l = (y - z)^2 and dz = 2 (z - y) * scale.  Each head kernel picks this or the sigmoid cross-entropy with its
+// compile-time SQ parameter; the weight multiplies both afterwards, as for the logistic head.
+__device__ __forceinline__ void sq_head(float z, float y, float scale, float& l, float& g) {
+    const float d = z - y;
+    l = d * d;
+    g = (2.f * d) * scale;
+}
+
 // raw batch as kernel parameter (pointer tables by value: no H2D copy of pointer arrays)
 struct BatchPtrs {
     const void*    cat[DFM_MAX_CAT];

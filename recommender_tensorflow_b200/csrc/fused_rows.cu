@@ -132,7 +132,8 @@ __device__ __forceinline__ void mma3(float (&cm)[4], float (&cx)[4], const uint3
 // row_gsum_kernel, which skips the single ones.
 // WGT: weighted model - the producers stage each sample's weight beside its label, and the head multiplies the loss term and
 // dz by it once (after the scale, so w = 1 reproduces the unweighted bits); everything downstream consumes dz as it is.
-template <int K, int H1, int ES, bool RB, bool FAST, bool WGT>
+// SQ: squared head (sq_head) instead of the sigmoid cross-entropy at both head sites; nothing else changes.
+template <int K, int H1, int ES, bool RB, bool FAST, bool SQ, bool WGT>
 __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs A) {
     static_assert(!RB || ES == 0, "row-buffer records carry no optimizer slots");
     static_assert(K == 16 && H1 == 16, "instantiated for embedding_size 16 / first hidden layer 16");
@@ -433,8 +434,12 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
                 float gz = 0.f, lterm = 0.f;
                 if (b < a.B && train) {
                     const float y = ys[sl];
-                    lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
-                    gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                    if constexpr (SQ) {
+                        sq_head(z, y, a.scale, lterm, gz);
+                    } else {
+                        lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+                        gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                    }
                     if constexpr (WGT) { gz *= wsl[sl]; lterm *= wsl[sl]; }
                 }
                 if (o == 0) {
@@ -551,8 +556,12 @@ __global__ void __launch_bounds__(FR_THREADS, 1) fused_rows_kernel(FusedRowsArgs
                     if (a.logits_out) a.logits_out[b] = z;
                     if (train) {
                         const float y = ys[sl];
-                        lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
-                        gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                        if constexpr (SQ) {
+                            sq_head(z, y, a.scale, lterm, gz);
+                        } else {
+                            lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+                            gz = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                        }
                         if constexpr (WGT) { gz *= wsl[sl]; lterm *= wsl[sl]; }
                         a.dz_out[b] = gz;
                     }
@@ -1021,45 +1030,56 @@ int fused_rows_grid(int B, int sm_count, bool side_stream_busy) {
     return std::max(1, std::min(tiles, sm_count - reserve));
 }
 
-template <int ES, bool RB, bool WGT>
+template <int ES, bool RB, bool SQ, bool WGT>
 static cudaError_t fr_attr(int smem_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, false, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    return e ? e : cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, true, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    cudaError_t e = cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, false, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+    return e ? e : cudaFuncSetAttribute(fused_rows_kernel<16, 16, ES, RB, true, SQ, WGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
 }
-template <bool WGT>
+template <bool SQ, bool WGT>
 static cudaError_t fr_attr_all(int smem_bytes) {
-    cudaError_t e = fr_attr<0, false, WGT>(smem_bytes);
-    if (!e) e = fr_attr<1, false, WGT>(smem_bytes);
-    if (!e) e = fr_attr<2, false, WGT>(smem_bytes);
-    if (!e) e = fr_attr<0, true, WGT>(smem_bytes);
+    cudaError_t e = fr_attr<0, false, SQ, WGT>(smem_bytes);
+    if (!e) e = fr_attr<1, false, SQ, WGT>(smem_bytes);
+    if (!e) e = fr_attr<2, false, SQ, WGT>(smem_bytes);
+    if (!e) e = fr_attr<0, true, SQ, WGT>(smem_bytes);
     return e;
 }
-cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted) {
-    cudaError_t e = fr_attr_all<false>(smem_bytes);
-    return (e || !weighted) ? e : fr_attr_all<true>(smem_bytes);
+cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted, bool squared) {
+    // the logistic instantiations always (a squared handle's forward-only launches use them too), the others as needed
+    cudaError_t e = fr_attr_all<false, false>(smem_bytes);
+    if (!e && weighted) e = fr_attr_all<false, true>(smem_bytes);
+    if (!e && squared) e = fr_attr_all<true, false>(smem_bytes);
+    if (!e && squared && weighted) e = fr_attr_all<true, true>(smem_bytes);
+    return e;
 }
-template <int ES, bool RB, bool WGT>
+template <int ES, bool RB, bool SQ, bool WGT>
 static void fr_go(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
     // FAST: every optimizer step the kernel takes is Adam and every replay is the closed form (row-buffer mode does neither)
     const RowReplay& rr = A.f.rr;
     const bool replay_fast = rr.upto < 0 || (rr.emb_adam && rr.rd.closed && (rr.same || !rr.lin_adam));
     const bool apply_fast = RB || !A.f.train || A.claim == nullptr || (A.od_t.kind == DFM_OPT_ADAM && (!A.f.use_linear || A.ol_t.kind == DFM_OPT_ADAM));
     static const bool allow = getenv("DFM_FR_NO_FAST") == nullptr;
-    if (allow && replay_fast && apply_fast) fused_rows_kernel<16, 16, ES, RB, true, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
-    else fused_rows_kernel<16, 16, ES, RB, false, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
+    if (allow && replay_fast && apply_fast) fused_rows_kernel<16, 16, ES, RB, true, SQ, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
+    else fused_rows_kernel<16, 16, ES, RB, false, SQ, WGT><<<grid, FR_THREADS, smem_bytes, st>>>(A);
 }
-template <bool WGT>
+template <bool SQ, bool WGT>
 static void fr_go_slots(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
-    if (A.rowbuf_mode) { fr_go<0, true, WGT>(A, grid, smem_bytes, st); return; }
+    if (A.rowbuf_mode) { fr_go<0, true, SQ, WGT>(A, grid, smem_bytes, st); return; }
     switch (A.emb_slots) {
-        case 0: fr_go<0, false, WGT>(A, grid, smem_bytes, st); break;
-        case 1: fr_go<1, false, WGT>(A, grid, smem_bytes, st); break;
-        default: fr_go<2, false, WGT>(A, grid, smem_bytes, st); break;
+        case 0: fr_go<0, false, SQ, WGT>(A, grid, smem_bytes, st); break;
+        case 1: fr_go<1, false, SQ, WGT>(A, grid, smem_bytes, st); break;
+        default: fr_go<2, false, SQ, WGT>(A, grid, smem_bytes, st); break;
     }
 }
-cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st) {
-    // weighted train step (make_fused_args sets the weights pointer only then): the WGT instantiations
-    if (A.f.bp.weights) fr_go_slots<true>(A, grid, smem_bytes, st);
-    else fr_go_slots<false>(A, grid, smem_bytes, st);
+cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st, bool squared) {
+    // weighted train step (make_fused_args sets the weights pointer only then): the WGT instantiations; squared: the
+    // SQ ones, for train steps only (a forward forms no loss, so it runs the logistic code)
+    const bool sq = squared && A.f.train;
+    if (A.f.bp.weights) {
+        if (sq) fr_go_slots<true, true>(A, grid, smem_bytes, st);
+        else fr_go_slots<false, true>(A, grid, smem_bytes, st);
+    } else {
+        if (sq) fr_go_slots<true, false>(A, grid, smem_bytes, st);
+        else fr_go_slots<false, false>(A, grid, smem_bytes, st);
+    }
     return cudaGetLastError();
 }

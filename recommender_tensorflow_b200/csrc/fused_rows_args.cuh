@@ -50,5 +50,5 @@ cudaError_t fused_rows_compact(const uint32_t* keys_in, const uint32_t* vals_in,
                                uint32_t* keys_out, uint32_t* vals_out, uint32_t* scratch, uint32_t* n_out, cudaStream_t st, int64_t* launches);
 void fr_layout(FusedRowsArgs& A, const SmallMlpDesc& m, int K, int dc, int dn);      // needs A.sst
 void fr_balance(FusedRowsArgs& A, int dc, int dn, bool cat_tasks);   // cat_tasks: the kernel applies / forwards the once-only rows' gradients
-cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted);      // weighted: also the W instantiations
-cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st);
+cudaError_t fused_rows_set_attr(int smem_bytes, bool weighted, bool squared);   // also the WGT / SQ instantiations
+cudaError_t fused_rows_launch(const FusedRowsArgs& A, int grid, size_t smem_bytes, cudaStream_t st, bool squared);   // squared: SQ for a train step

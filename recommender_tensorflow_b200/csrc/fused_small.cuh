@@ -72,7 +72,8 @@ static inline size_t fused_smem_floats(const SmallMlpDesc& m, int K, int dc, int
 // NC: input columns per thread in the dW0 accumulation = ceil(d / (CG / K)), CG = 256 / (H1/4)  (compile time so that
 // the accumulators stay in registers without per-column predicates)
 // WGT: weighted model, the head multiplies the loss term and dz of sample b by a.bp.weights[b] (after the scale: w = 1 is exact)
-template <int K, int H1, bool ROWBUF, int NC, bool WGT>
+// SQ: squared head (sq_head) instead of the sigmoid cross-entropy
+template <int K, int H1, bool ROWBUF, int NC, bool SQ, bool WGT>
 __global__ void __launch_bounds__(256, 2) fused_small_kernel(FusedArgs a) {
     constexpr int LPR = K / 4, FPR = 32 / LPR;
     constexpr int OQ = H1 / 4;                     // output quads
@@ -357,8 +358,12 @@ __global__ void __launch_bounds__(256, 2) fused_small_kernel(FusedArgs a) {
                 if (a.logits_out) a.logits_out[b] = z;
                 if (train) {
                     const float y = a.labels[b];
-                    lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
-                    g = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                    if constexpr (SQ) {
+                        sq_head(z, y, a.scale, lterm, g);
+                    } else {
+                        lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+                        g = (1.f / (1.f + expf(-z)) - y) * a.scale;
+                    }
                     if constexpr (WGT) { const float w = a.bp.weights[b]; g *= w; lterm *= w; }
                     a.dz_out[b] = g;
                 }

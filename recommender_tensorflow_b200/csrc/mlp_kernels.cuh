@@ -309,7 +309,8 @@ static __global__ void __launch_bounds__(256) numeric_grad_partial_kernel(BatchP
 // head: z = zacc + h_L . Wo + bo ; loss_b = max(z,0) - z*y + log1p(exp(-|z|)) ; dz = (sigmoid(z)-y)*scale
 // one warp per sample; per-block partial sums of loss and dz (fixed order inside the block).
 // WGT: weighted model, loss_b *= w_b and dz = ((sigmoid(z)-y)*scale)*w_b (w = 1 gives the unweighted bits)
-template <bool WGT>
+// SQ: squared head, loss_b = (y - z)^2 and dz = 2 (z - y) * scale (sq_head), then the weight
+template <bool SQ, bool WGT>
 __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ zacc, const float* __restrict__ hL, int H,
                                                    const float* __restrict__ Wo, const float* __restrict__ bo,
                                                    const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale,
@@ -333,9 +334,14 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ zac
             if (logits_out) logits_out[b] = z;
             if (labels) {
                 float y = labels[b];
-                float l = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
-                float sg = 1.f / (1.f + expf(-z));
-                float g = (sg - y) * scale;
+                float l, g;
+                if constexpr (SQ) {
+                    sq_head(z, y, scale, l, g);
+                } else {
+                    l = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+                    float sg = 1.f / (1.f + expf(-z));
+                    g = (sg - y) * scale;
+                }
                 if constexpr (WGT) { const float w = weights[b]; g *= w; l *= w; }
                 dz[b] = g;
                 lsum += l;
@@ -359,7 +365,8 @@ __global__ void __launch_bounds__(256) head_kernel(const float* __restrict__ zac
 // while h_L is still in registers; per-block partial sums (fixed order) of the loss, dz,
 // gWo = h_L^T dz and gb_L = column sums of dh_L'.  Replaces head_kernel + dh_last_kernel + two column-sum
 // launches (and one re-read of h_L).   gpart layout: [grid][2*H] = {gWo | gb_L}
-template <int NH, bool WGT>
+// WGT / SQ: as head_kernel
+template <int NH, bool SQ, bool WGT>
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ zacc, const float* __restrict__ hL,
                                                        const float* __restrict__ Wo, const float* __restrict__ bo,
                                                        const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale,
@@ -403,13 +410,15 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
             const int bb = s2 ? b2 : b;
             const float zz = z[s2] + b0 + (s2 ? za1 : za0);
             const float y = s2 ? y1 : y0;
-            float g = (1.f / (1.f + expf(-zz)) - y) * scale;
+            float g, lsq = 0.f;
+            if constexpr (SQ) sq_head(zz, y, scale, lsq, g);
+            else g = (1.f / (1.f + expf(-zz)) - y) * scale;
             if constexpr (WGT) g *= s2 ? w1 : w0;
             if (lane == 0) {
                 logits[bb] = zz;
                 if (logits_out) logits_out[bb] = zz;
                 dz[bb] = g;
-                float l = fmaxf(zz, 0.f) - zz * y + log1pf(expf(-fabsf(zz)));
+                float l = SQ ? lsq : fmaxf(zz, 0.f) - zz * y + log1pf(expf(-fabsf(zz)));
                 if constexpr (WGT) l *= s2 ? w1 : w0;
                 lsum += l;
                 dsum += g;

@@ -40,7 +40,8 @@ static inline size_t small_mlp_fwd_smem(const SmallMlpDesc& m) {
 
 // per-sample scratch row layout: [h_1 | h_2 | ... | h_L]; gradients use a second array of the same shape
 // WGT: weighted model, the loss term and dz of sample b are multiplied by weights[b] (after the scale: w = 1 is exact)
-template <int H1, bool WGT>
+// SQ: squared head (sq_head) instead of the sigmoid cross-entropy
+template <int H1, bool SQ, bool WGT>
 __global__ void __launch_bounds__(256, 2) small_mlp_fwd_bwd_top_kernel(
     SmallMlpDesc m, const float* __restrict__ dw, const float* __restrict__ h0, const float* __restrict__ zacc,
     const float* __restrict__ labels, const float* __restrict__ weights, int B, float scale, int train, float* __restrict__ logits,
@@ -156,8 +157,12 @@ __global__ void __launch_bounds__(256, 2) small_mlp_fwd_bwd_top_kernel(
                 if (logits_out) logits_out[b] = z;
                 if (train) {
                     float y = labels[b];
-                    lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
-                    g = (1.f / (1.f + expf(-z)) - y) * scale;
+                    if constexpr (SQ) {
+                        sq_head(z, y, scale, lterm, g);
+                    } else {
+                        lterm = fmaxf(z, 0.f) - z * y + log1pf(expf(-fabsf(z)));
+                        g = (1.f / (1.f + expf(-z)) - y) * scale;
+                    }
                     if constexpr (WGT) { const float w = weights[b]; g *= w; lterm *= w; }
                     dz_out[b] = g;
                 }

@@ -20,7 +20,8 @@ class CsvConfig(C.Structure):
     _fields_ = [("n_fields", C.c_int32), ("kind", C.POINTER(C.c_int32)), ("int_default", C.POINTER(C.c_int32)),
                 ("str_default", C.POINTER(C.c_char_p)), ("label_field", C.c_int32), ("label_min", C.c_int32),
                 ("max_records", C.c_int32), ("max_bytes", C.c_int64), ("device", C.c_int32),
-                ("float_default", C.POINTER(C.c_float)), ("field_delim", C.c_int32), ("as_float", C.POINTER(C.c_int32))]
+                ("float_default", C.POINTER(C.c_float)), ("field_delim", C.c_int32), ("as_float", C.POINTER(C.c_int32)),
+                ("label_raw", C.c_int32)]
 
 
 def _default_dtype(d):
@@ -36,7 +37,9 @@ class GpuCsvReader:
         """columns / defaults: the CSV schema (names and `record_defaults`, e.g. trainers.ml_100k.COLUMNS / DEFAULTS;
         [0] is int32, [0.0] float32, anything else a string).  Only the fields `engine` consumes (plus the label) are
         materialised; the rest is parsed for structure only.  A numeric column reads a float32 field, or an int32 field
-        converted with tf.to_float.  field_delim: one character, as tf.decode_csv's.  weight_col: the field holding the
+        converted with tf.to_float.  cutoff: the label is `value >= cutoff` (the binary head's 0/1); None makes it the
+        label field's value as float32 (tf.to_float of the rating: the regression head's label), and the label field may
+        then also be a float32 field.  field_delim: one character, as tf.decode_csv's.  weight_col: the field holding the
         per-example weight of a weighted engine (float32, or int32 read as float like a numeric column); the batches
         point RawBatch.weights at its float32 column."""
         self.lib = _lib.load()
@@ -87,8 +90,8 @@ class GpuCsvReader:
         self.max_records = int(max_records)
         self.max_bytes = int(max_bytes or 512 * self.max_records)
         cfg = CsvConfig(n, C.cast(kind, C.POINTER(C.c_int32)), C.cast(idef, C.POINTER(C.c_int32)), C.cast(sdef, C.POINTER(C.c_char_p)),
-                        self.label_field, int(cutoff), self.max_records, self.max_bytes, engine.device,
-                        C.cast(fdef, C.POINTER(C.c_float)), delim[0], C.cast(as_float, C.POINTER(C.c_int32)))
+                        self.label_field, 0 if cutoff is None else int(cutoff), self.max_records, self.max_bytes, engine.device,
+                        C.cast(fdef, C.POINTER(C.c_float)), delim[0], C.cast(as_float, C.POINTER(C.c_int32)), int(cutoff is None))
         self._keep = [kind, idef, sdef, fdef, as_float]
         h = C.c_void_p()
         rc = self.lib.dfm_csv_create(C.byref(cfg), C.byref(h))

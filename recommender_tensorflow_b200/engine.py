@@ -94,9 +94,11 @@ class DeepFMEngine:
     def __init__(self, categorical_columns, numeric_columns=(), embedding_size=4, hidden_units=(16, 16),
                  use_linear=True, use_mf=True, use_dnn=True, loss_reduction="mean", opt_deep=None,
                  opt_linear=None, max_batch=65536, device=0, feature_dtypes=None, sort_columns=True, rank=0, world=1, dropout=0.0, dropout_seed=0,
-                 multivalent=None, activation="relu", weighted=False):
+                 multivalent=None, activation="relu", weighted=False, head="logistic"):
         """weighted: train batches carry per-example weights (the estimators' weight_column): the per-sample loss and
-        its gradient are multiplied by the weight on the device.  train_step / pack then require `weights`."""
+        its gradient are multiplied by the weight on the device.  train_step / pack then require `weights`.
+        head: "logistic" (sigmoid cross-entropy on 0/1 labels, the binary classifiers) or "squared" ((y - z)^2 on
+        float labels, the regressors); the logits are the same either way, only the train step's loss and dz differ."""
         self.lib = _lib.load()
         # params["activation"] (trainers/deep_fm.py:22): a name, None (identity) or a callable named like a tf.nn activation
         act = activation if (activation is None or isinstance(activation, str)) else getattr(activation, "__name__", str(activation))
@@ -119,6 +121,9 @@ class DeepFMEngine:
         self.rank, self.world = int(rank), int(world)
         self.dropout, self.dropout_seed = float(dropout or 0.0), int(dropout_seed)
         self.weighted = bool(weighted)
+        if head not in _lib.HEADS:
+            raise ValueError("head %r is not one of %s" % (head, sorted(_lib.HEADS)))
+        self.head = head
         fd = dict(feature_dtypes or {})
         mv = dict(multivalent or {})      # raw feature key -> value slots per sample (multi-hot / multivalent column)
         self.specs = []
@@ -178,9 +183,9 @@ class DeepFMEngine:
         cfg = _lib.Config(len(cats), C.cast(cols, C.POINTER(_lib.Column)), len(nums), self.k, len(self.hidden),
                           C.cast(hid, C.POINTER(C.c_int32)), int(self.use_linear), int(self.use_mf), int(self.use_dnn),
                           _lib.LOSS_RED[loss_reduction], _opt_struct(self.opt_deep), _opt_struct(self.opt_linear),
-                          self.max_batch, self.device, self.rank, self.world, None, self.dropout, self.dropout_seed,
-                          _lib.ACTIVATIONS[self.activation], len(self.src_specs), C.cast(srcs, C.POINTER(_lib.Column)),
-                          int(self.weighted))
+                          self.max_batch, self.device, self.rank, self.world, None, self.dropout, _lib.HEADS[self.head],
+                          self.dropout_seed, _lib.ACTIVATIONS[self.activation], len(self.src_specs),
+                          C.cast(srcs, C.POINTER(_lib.Column)), int(self.weighted))
         self._keep += [cols, srcs, hid]
         handle = C.c_void_p()
         rc = self.lib.dfm_create(C.byref(cfg), C.byref(handle))

@@ -15,10 +15,24 @@ import numpy as np
 
 from ..engine import DeepFMEngine, PackedBatch
 from .ml_100k import FEATURE_DTYPES, ModeKeys, get_feature_columns, get_input_fn
-from .model_utils import get_binary_metrics, get_binary_predictions, get_optimizer, get_weights, weight_column_key
+from .model_utils import (check_regression_head, get_binary_metrics, get_binary_predictions, get_optimizer,
+                          get_regression_metrics, get_regression_predictions, get_weights, weight_column_key)
 
 EstimatorSpec = namedtuple("EstimatorSpec", ["mode", "loss", "train_op", "predictions", "eval_metric_ops", "global_step"])
 _ENGINE_KEY = "_b200_engine"
+# params["head"] -> (engine head, predictions, EVAL metrics): the reference's contrib binary_classification_head, or
+# regression_head (label_dimension 1, mean squared error, identity inverse link) to predict the rating itself
+_HEADS = {"binary": ("logistic", get_binary_predictions, get_binary_metrics),
+          "regression": ("squared", get_regression_predictions, get_regression_metrics)}
+
+
+def _head(params):
+    head = params.get("head", "binary")
+    if head not in _HEADS:
+        raise ValueError("params['head'] must be one of %s, got %r" % (sorted(_HEADS), head))
+    if head == "regression":
+        check_regression_head(params.get("label_dimension", 1), params.get("inverse_link_fn"), params.get("loss_fn"))
+    return _HEADS[head]
 
 
 def _build_engine(params, batch_size):
@@ -36,6 +50,7 @@ def _build_engine(params, batch_size):
     # weight_column of the binary head (contrib binary_classification_head(weight_column=...)): absent in the
     # reference's model_fn, so None keeps the unweighted model
     weighted = weight_column_key(params.get("weight_column")) is not None
+    head = _head(params)[0]
     # check params (trainers/deep_fm.py:28-34)
     if (len(categorical_columns) + len(numeric_columns)) == 0:
         raise ValueError("At least 1 feature column of categorical_columns or numeric_columns must be specified.")
@@ -49,7 +64,7 @@ def _build_engine(params, batch_size):
                        opt_deep=opt, opt_linear=dict(opt), max_batch=params.get("max_batch", max(batch_size, 1)),
                        device=params.get("device", 0), feature_dtypes=params.get("feature_dtypes", FEATURE_DTYPES),
                        dropout=float(dropout or 0.0), dropout_seed=int(params.get("dropout_seed", 0)), activation=activation_fn,
-                       weighted=weighted)
+                       weighted=weighted, head=head)
     # the variable initialisers TF runs when the graph is first executed (truncated normal 1/sqrt(k) for the embedding
     # tables, glorot uniform for the dense kernels, zeros for linear weights and biases); RunConfig.tf_random_seed
     seed = params.get("tf_random_seed")
@@ -70,16 +85,17 @@ def model_fn(features, labels, mode, params):
     if engine is None:
         engine = params[_ENGINE_KEY] = _build_engine(params, _batch_size(features))
     weight_column = params.get("weight_column")
+    _, predictions, eval_metrics = _head(params)
     if mode == ModeKeys.TRAIN:
         # a device batch (get_gpu_input_fn) carries its weights inside; a host batch has them among its features
         weights = None if isinstance(features, PackedBatch) else get_weights(features, weight_column, _batch_size(features))
         loss, logits = engine.train_step(features, labels, return_logits=True, weights=weights)
-        return EstimatorSpec(mode, loss, None, get_binary_predictions(logits), None, engine.global_step)
+        return EstimatorSpec(mode, loss, None, predictions(logits), None, engine.global_step)
     logits = engine.predict_logits(features)
-    preds = get_binary_predictions(logits)
+    preds = predictions(logits)
     if mode == ModeKeys.PREDICT:
         return EstimatorSpec(mode, None, None, preds, None, engine.global_step)
-    metrics = get_binary_metrics(labels, logits, get_weights(features, weight_column, logits.shape[0]))
+    metrics = eval_metrics(labels, logits, get_weights(features, weight_column, logits.shape[0]))
     return EstimatorSpec(mode, metrics["average_loss"], None, preds, metrics, engine.global_step)
 
 
@@ -174,18 +190,20 @@ class Estimator:
     def evaluate(self, input_fn):
         ys, zs, ws = [], [], []
         weight_column = self.params.get("weight_column")
+        _, _, eval_metrics = _head(self.params)
+        zkey = "predictions" if eval_metrics is get_regression_metrics else "logits"    # the head's logits, [B, 1]
         for feats, labels in input_fn():
             if self.engine is None:
                 self.params[_ENGINE_KEY] = _build_engine(self.params, _batch_size(feats))
             self._maybe_restore()
             spec = self.model_fn(feats, labels, ModeKeys.EVAL, self.params)
             ys.append(np.asarray(labels, dtype=np.float32).reshape(-1))
-            zs.append(spec.predictions["logits"].reshape(-1))
+            zs.append(spec.predictions[zkey].reshape(-1))
             if weight_column is not None:
                 ws.append(get_weights(feats, weight_column, zs[-1].shape[0]))
         if not ys:
             raise ValueError("evaluate(): input_fn yielded no batches")
-        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
+        m = eval_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
         m["global_step"] = self.engine.global_step
         return m
 
@@ -200,7 +218,7 @@ class Estimator:
                     raise ValueError("Could not find trained model in model_dir: %s." % self.model_dir)
                 self._maybe_restore()
             spec = self.model_fn(feats, None, ModeKeys.PREDICT, self.params)
-            n = spec.predictions["logits"].shape[0]
+            n = next(iter(spec.predictions.values())).shape[0]
             for i in range(n):
                 yield {k: v[i] for k, v in spec.predictions.items()}
 

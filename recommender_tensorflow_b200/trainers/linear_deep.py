@@ -1,7 +1,8 @@
 """Mirror of trainers/linear_deep.py: the canned tf.estimator.DNNLinearCombinedClassifier
 (trainers/linear_deep.py:32-39) = wide&deep: linear_model(linear columns) + DNN(input_layer(deep
 columns)), no FM term, SUM loss, Adagrad(0.001) on the dnn side and FTRL(min(0.005, 1/sqrt(n_linear)))
-on the linear side (TF-1.12 canned defaults, SURVEY.md §8a row 8)."""
+on the linear side (TF-1.12 canned defaults, SURVEY.md §8a row 8).  DNNLinearCombinedRegressor is the same model
+with the regression head (squared error on the float label, the logits as predictions)."""
 import math
 import os
 
@@ -9,7 +10,8 @@ import numpy as np
 
 from ..engine import DeepFMEngine, PackedBatch, default_optimizer
 from .ml_100k import FEATURE_DTYPES, ModeKeys
-from .model_utils import get_binary_metrics, get_binary_predictions, get_weights, weight_column_key
+from .model_utils import (check_regression_head, get_binary_metrics, get_binary_predictions, get_regression_metrics,
+                          get_regression_predictions, get_weights, weight_column_key)
 
 _DNN_LEARNING_RATE = 0.001
 _LINEAR_LEARNING_RATE = 0.005
@@ -23,6 +25,15 @@ class _CannedBase:
     weight_column = None       # weight_column: a feature key or numeric_column whose value weights each example
     KEEP_CHECKPOINT_MAX = 5
     _restored = False
+    # the head: *Classifier binary (sigmoid cross-entropy), *Regressor regression (squared error, label_dimension 1)
+    HEAD = "binary"
+    _ENGINE_HEAD = {"binary": "logistic", "regression": "squared"}
+
+    def _head_fns(self):
+        """(predictions, EVAL metrics) of the head"""
+        if self.HEAD == "regression":
+            return get_regression_predictions, get_regression_metrics
+        return get_binary_predictions, get_binary_metrics
 
     def _weights(self, feats, n=None):
         """per-example weights of a host batch (None when unweighted; a device batch carries its own)"""
@@ -83,7 +94,7 @@ class _CannedBase:
             zs.append(self.engine.predict_logits(feats))
             if self.weight_column is not None:
                 ws.append(self._weights(feats, zs[-1].shape[0]))
-        m = get_binary_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
+        m = self._head_fns()[1](np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
         m["global_step"] = self.engine.global_step
         return m
 
@@ -91,8 +102,8 @@ class _CannedBase:
         self._maybe_restore()
         for item in input_fn():
             feats = item[0] if isinstance(item, tuple) else item
-            preds = get_binary_predictions(self.engine.predict_logits(feats))
-            for i in range(preds["logits"].shape[0]):
+            preds = self._head_fns()[0](self.engine.predict_logits(feats))
+            for i in range(next(iter(preds.values())).shape[0]):
                 yield {k: v[i] for k, v in preds.items()}
 
 
@@ -120,8 +131,23 @@ class DNNLinearCombinedClassifier(_CannedBase):
                                    opt_deep=default_optimizer("Adagrad", _DNN_LEARNING_RATE),
                                    opt_linear=default_optimizer("Ftrl", lin_lr), max_batch=max_batch, device=device,
                                    dropout=float(dnn_dropout or 0.0),
-                                   feature_dtypes=feature_dtypes, weighted=weight_column is not None)
+                                   feature_dtypes=feature_dtypes, weighted=weight_column is not None,
+                                   head=self._ENGINE_HEAD[self.HEAD])
         self._finish_init(model_dir, tf_random_seed)
+
+
+class DNNLinearCombinedRegressor(DNNLinearCombinedClassifier):
+    """canned tf.estimator.DNNLinearCombinedRegressor (TF 1.12): DNNLinearCombinedClassifier's model, optimizers,
+    checkpoint names and SUM reduction with the regression head"""
+    HEAD = "regression"
+
+    def __init__(self, model_dir=None, linear_feature_columns=None, dnn_feature_columns=None, dnn_hidden_units=None,
+                 dnn_dropout=None, label_dimension=1, weight_column=None, config=None, max_batch=4096, device=0,
+                 feature_dtypes=FEATURE_DTYPES, tf_random_seed=None):
+        check_regression_head(label_dimension)
+        super().__init__(model_dir=model_dir, linear_feature_columns=linear_feature_columns, dnn_feature_columns=dnn_feature_columns,
+                         dnn_hidden_units=dnn_hidden_units, dnn_dropout=dnn_dropout, config=config, max_batch=max_batch,
+                         device=device, feature_dtypes=feature_dtypes, tf_random_seed=tf_random_seed, weight_column=weight_column)
 
 
 def canned_train_and_evaluate(args, build):

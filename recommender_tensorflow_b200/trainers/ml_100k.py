@@ -66,12 +66,15 @@ def _to_batch(rows, cutoff):
         else:
             feats[name] = np.array([(v if v != "" else default[0]).encode() for v in col], dtype=object)
     label = feats.pop(LABEL_COL)
+    if cutoff is None:                                    # the rating itself: the regression head's tf.to_float(label)
+        return feats, label.astype(np.float32)
     return feats, (label >= cutoff).astype(np.float32)   # tf.math.greater_equal(label, cutoff)
 
 
 def get_input_fn(csv_path, mode=ModeKeys.TRAIN, batch_size=32, cutoff=5, seed=None):
     """trainers/ml_100k.py:42-61: skip header; TRAIN: shuffle(16*batch_size).repeat(); batch(batch_size).
-    Returns a callable producing an iterator of (features dict, label float32 [B])."""
+    Returns a callable producing an iterator of (features dict, label float32 [B]).  The label is rating >= cutoff;
+    cutoff=None makes it the rating itself (the regressors' label)."""
     def input_fn():
         rng = np.random.default_rng(seed)
         if mode == ModeKeys.TRAIN:
@@ -158,7 +161,7 @@ def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutof
     """get_input_fn with tf.decode_csv moved to the GPU (SURVEY.md §8f rank 2): the host only selects whole records
     (same shuffle algorithm and RNG stream as get_input_fn, so the same seed gives the same batches); the file itself
     is uploaded once and stays in HBM, a batch travels as 4 bytes per record (its line number); `GpuCsvReader` splits,
-    unquotes, parses and thresholds on the device.  Yields
+    unquotes, parses and thresholds on the device (cutoff=None: the label is the rating itself, as in get_input_fn).  Yields
     (PackedBatch on the device, labels): in TRAIN mode labels is None (they are inside the batch), otherwise the
     float32 labels are read back for the metrics.  A record is one text line, as with tf.data.TextLineDataset (a
     quoted field cannot contain a line break).  weight_column (a field key or numeric_column of a weighted engine): the

@@ -1,4 +1,4 @@
-"""Mirror of trainers/model_utils.py: optimizer lookup and the binary head's outputs."""
+"""Mirror of trainers/model_utils.py: optimizer lookup and the binary and regression heads' outputs."""
 import numpy as np
 
 from ..engine import default_optimizer
@@ -24,6 +24,25 @@ def get_binary_predictions(logits):
     logistic = 1.0 / (1.0 + np.exp(-logits))
     return {"logits": logits, "logistic": logistic, "probabilities": np.concatenate([1 - logistic, logistic], 1),
             "class_ids": (logistic > 0.5).astype(np.int64), "class_id": (logistic > 0.5).astype(np.int32)}
+
+
+def get_regression_predictions(logits):
+    """regression_head predictions (TF 1.12 head.py _RegressionHeadWithMeanSquaredErrorLoss, identity inverse link):
+    the logits [B, 1] under the key "predictions"; there are no probabilities or classes."""
+    return {"predictions": np.asarray(logits, dtype=np.float32).reshape(-1, 1)}
+
+
+def check_regression_head(label_dimension=1, inverse_link_fn=None, loss_fn=None, n_classes=None):
+    """The regression head is built for label_dimension = 1 with the identity inverse link and the mean squared error;
+    anything else is rejected rather than silently trained as that model."""
+    if label_dimension != 1:
+        raise ValueError("label_dimension must be 1 (got %r): only single-output regression is implemented" % (label_dimension,))
+    if inverse_link_fn is not None:
+        raise ValueError("inverse_link_fn is not supported: the regression head predicts the logits (identity link)")
+    if loss_fn is not None:
+        raise ValueError("a custom loss_fn is not supported: the regression head's loss is the squared error")
+    if n_classes not in (None, 2):
+        raise ValueError("n_classes=%r: multi-class heads are not supported" % (n_classes,))
 
 
 def weight_column_key(weight_column):
@@ -105,3 +124,23 @@ def get_binary_metrics(labels, logits, weights=None):
     return {"accuracy": float(((p > 0.5) == (y > 0.5)).mean()), "auc": _auc(y, p), "auc_precision_recall": _auc(y, p, "PR"),
             "average_loss": float(loss.mean()), "loss": float(loss.sum()), "label/mean": float(y.mean()),
             "prediction/mean": float(p.mean())}
+
+
+def get_regression_metrics(labels, logits, weights=None):
+    """Metrics the regression head reports in EVAL mode (TF 1.12 head.py _RegressionHeadWithMeanSquaredErrorLoss.
+    _eval_metric_ops: average_loss, label/mean, prediction/mean) plus `loss`, the summed loss, as for the binary head.
+    The per-example loss is (y - z)^2; weights (weight_column) make every metric weighted: means are
+    sum(w x) / sum(w) and loss is sum(w l)."""
+    y = np.asarray(labels, dtype=np.float64).reshape(-1)
+    z = np.asarray(logits, dtype=np.float64).reshape(-1)
+    if y.shape != z.shape:
+        raise ValueError("labels shape %s does not match logits %s (label_dimension is 1)" % (list(y.shape), list(z.shape)))
+    loss = (y - z) ** 2
+    w = np.ones_like(y)
+    if weights is not None:
+        w = np.asarray(weights, dtype=np.float32).astype(np.float64).reshape(-1)
+        if w.shape != y.shape:
+            raise ValueError("weights shape %s does not match labels %s" % (list(w.shape), list(y.shape)))
+    sw = w.sum()
+    return {"average_loss": float((w * loss).sum() / sw), "loss": float((w * loss).sum()),
+            "label/mean": float((w * y).sum() / sw), "prediction/mean": float((w * z).sum() / sw)}
