@@ -169,8 +169,8 @@ typedef struct {
     const float*          labels;       /* [B] float32 labels; NULL for forward.  The logistic head takes 0/1 (rating >=
                                            cutoff, trainers/ml_100k.py:48), the squared head any value (the rating) */
     /* [B] float32 per-example weights, on the same side (host / device) as labels.  Read only by a handle created with
-     * dfm_config.weighted != 0, and only by train steps (required there: NULL -> DFM_ERR_INVALID_ARG); forward,
-     * PREDICT and layer_summary ignore it.  An unweighted handle never reads this field. */
+     * dfm_config.weighted != 0, and only by train steps and dfm_evaluate / dfm_evaluate_host (required there: NULL ->
+     * DFM_ERR_INVALID_ARG); forward, PREDICT and layer_summary ignore it.  An unweighted handle never reads this field. */
     const float*          weights;
 } dfm_raw_batch;
 
@@ -225,6 +225,38 @@ int dfm_train_step_host_drain(dfm_handle* h, float* last_loss_host);
 /* mode == EVAL / PREDICT: logits only, no state change (device pointers). */
 int dfm_forward(dfm_handle* h, const dfm_raw_batch* dev_batch, float* logits_out_dev, void* stream);
 int dfm_forward_host(dfm_handle* h, const dfm_raw_batch* host_batch, float* logits_out_host);
+
+/* ---- EVAL metrics streamed on the device (csrc/metrics.cuh, DESIGN.md §8.6).  Every handle keeps one metric state in
+ * device memory; each batch adds to it, and the host finishes the metrics of the handle's head from the raw state (the
+ * states of several ranks are combined by summing the fields, in rank order).  Logistic head, as TF 1.12
+ * metrics_impl / head.py: p = 1.f / (1.f + expf(-z)) in float32; bin = number of TF's 200 float32 AUC thresholds t with
+ * p > t; positive = label > 0.5; predicted class = z > 0.  Squared head: only n and the four sums.  An unweighted
+ * batch counts with w = 1, so the weighted fields hold unit-weight totals.  Counts are exact; the float64 fields are
+ * summed in a fixed order, so a rerun gives the same bits. */
+#define DFM_METRIC_BINS 201
+typedef struct {
+    int64_t n;                                  /* samples accumulated */
+    int64_t bin_count[2][DFM_METRIC_BINS];      /* [0] negatives, [1] positives per bin (logistic head) */
+    int64_t tp, fp, fn, correct;                /* class z > 0 against label > 0.5 (logistic head) */
+    double  bin_weight[2][DFM_METRIC_BINS];     /* the same, sums of the weights */
+    double  w_tp, w_fp, w_fn, w_correct;
+    double  sum_w, sum_wy;                      /* sum w, sum w y */
+    double  sum_wpred;                          /* logistic: sum w p (p in float64); squared: sum w z */
+    double  sum_wloss;                          /* logistic: sum w (max(z,0) - z y + log1p(exp(-|z|))) in float64; squared: sum w (y - z)^2 */
+} dfm_metric_state;
+/* zero the handle's metric state */
+int dfm_metrics_reset(dfm_handle* h, void* stream);
+/* add n samples whose logits the caller already has (device pointers; the row-sharded ranks use this on their
+ * dfm_shard_forward / dfm_xchg_forward output).  weights_dev: read on a weighted handle only, and required there. */
+int dfm_metrics_accumulate(dfm_handle* h, const float* logits_dev, const float* labels_dev, const float* weights_dev, int64_t n,
+                           void* stream);
+/* the forward pass of dfm_forward into a handle workspace, then the accumulation of dev_batch->labels (required) and, on
+ * a weighted handle, dev_batch->weights (required there).  Does not synchronise.  Unsharded handles only. */
+int dfm_evaluate(dfm_handle* h, const dfm_raw_batch* dev_batch, void* stream);
+/* the same from host buffers (the copy path of dfm_forward_host); returns after the batch was accumulated */
+int dfm_evaluate_host(dfm_handle* h, const dfm_raw_batch* host_batch);
+/* copy the state to the host (enqueued on stream, NULL = the handle's own) and synchronise that stream */
+int dfm_metrics_read(dfm_handle* h, dfm_metric_state* out_host, void* stream);
 
 /* ---- layer_summary side outputs (reference: trainers/model_utils.py:4-6 `layer_summary`, called at trainers/deep_fm.py:43
  * (linear logit), :89 (MF logit), :105 (every hidden layer, after dropout in TRAIN mode), :110 (DNN logit), :115 (logits)).

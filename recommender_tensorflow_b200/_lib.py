@@ -45,6 +45,17 @@ ACTIVATIONS = {"relu": 0, "tanh": 1, "sigmoid": 2, "identity": 3, "linear": 3, N
 HEADS = {"logistic": 0, "squared": 1}       # DFM_HEAD_*
 
 
+METRIC_BINS = 201        # DFM_METRIC_BINS
+
+
+class MetricState(C.Structure):
+    """dfm_metric_state: the raw EVAL metric state of a handle (include/deepfm_b200.h)"""
+    _fields_ = [("n", C.c_int64), ("bin_count", (C.c_int64 * METRIC_BINS) * 2), ("tp", C.c_int64), ("fp", C.c_int64),
+                ("fn", C.c_int64), ("correct", C.c_int64), ("bin_weight", (C.c_double * METRIC_BINS) * 2),
+                ("w_tp", C.c_double), ("w_fp", C.c_double), ("w_fn", C.c_double), ("w_correct", C.c_double),
+                ("sum_w", C.c_double), ("sum_wy", C.c_double), ("sum_wpred", C.c_double), ("sum_wloss", C.c_double)]
+
+
 class RawBatch(C.Structure):
     _fields_ = [("batch_size", C.c_int32), ("cat_data", C.POINTER(C.c_void_p)),
                 ("cat_offsets", C.POINTER(C.c_void_p)), ("num_data", C.POINTER(C.c_void_p)),
@@ -67,6 +78,11 @@ _SIGS = {
     "dfm_prefetch_batch": (C.c_int, [C.c_void_p, C.POINTER(RawBatch), C.c_void_p]),
     "dfm_forward": (C.c_int, [C.c_void_p, C.POINTER(RawBatch), C.c_void_p, C.c_void_p]),
     "dfm_forward_host": (C.c_int, [C.c_void_p, C.POINTER(RawBatch), C.c_void_p]),
+    "dfm_metrics_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "dfm_metrics_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "dfm_evaluate": (C.c_int, [C.c_void_p, C.POINTER(RawBatch), C.c_void_p]),
+    "dfm_evaluate_host": (C.c_int, [C.c_void_p, C.POINTER(RawBatch)]),
+    "dfm_metrics_read": (C.c_int, [C.c_void_p, C.POINTER(MetricState), C.c_void_p]),
     "dfm_summary_bucket_limits": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "dfm_layer_summary": (C.c_int, [C.c_void_p, C.POINTER(RawBatch), C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.POINTER(C.c_int32)]),
     "dfm_layer_summary_tensor": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p]),

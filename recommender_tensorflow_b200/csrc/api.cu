@@ -20,6 +20,7 @@
 #include "fused_small.cuh"
 #include "fused_rows_args.cuh"
 #include "summary.cuh"
+#include "metrics.cuh"
 #include "tc_gemm.cuh"
 #include "xchg.cuh"
 
@@ -177,6 +178,8 @@ struct dfm_handle {
     // layer_summary workspace (summary.cuh), allocated on first use
     float *sum_h0 = nullptr, *sum_s = nullptr, *sum_lin = nullptr, *sum_mf = nullptr, *sum_hidden = nullptr, *sum_dnn = nullptr, *sum_logits = nullptr;
     double* sum_limits = nullptr; SummaryStats* sum_stats = nullptr; unsigned long long* sum_buckets = nullptr;
+    // EVAL metric state (metrics.cuh) and the per-CTA partials of one batch, allocated on first use
+    dfm_metric_state* d_metrics = nullptr; metrics::Part* metric_parts = nullptr;
     bool claim_live = false;          // this step's claim table is filled: once-only rows are applied by fused_rows_kernel
     bool last_step_rows = false;
     bool fr_side = false;             // this step's sort runs on the side stream beside fused_rows_kernel
@@ -290,7 +293,7 @@ static void free_all(dfm_handle* h) {
     cudaSetDevice(h->device);
     void* ptrs[] = {h->d_cols, h->d_bounds, h->d_voc_bytes, h->d_voc_offs, h->d_vtab, h->d_row_off, h->tb.rec, h->dw,
                     h->ds1, h->ds2, h->dg, h->ids, h->h0, h->s, h->zacc, h->logits, h->dz, h->dE, h->splitk, h->colpart, h->head_part,
-                    h->d_loss, h->d_dzsum, h->d_err, h->num_partial, h->num_scratch, h->fused_done, h->claim, h->once_lk, h->sum_h0, h->sum_s, h->sum_lin, h->sum_mf, h->sum_hidden, h->sum_dnn, h->sum_logits, h->sum_limits, h->sum_stats, h->sum_buckets, h->up_partial, h->w0_partial, h->tc_w, h->head_gpart, h->d_slot_col, h->d_slot_j, h->d_field_slot0, h->inv_cnt, h->uidx,
+                    h->d_loss, h->d_dzsum, h->d_err, h->num_partial, h->num_scratch, h->fused_done, h->claim, h->once_lk, h->sum_h0, h->sum_s, h->sum_lin, h->sum_mf, h->sum_hidden, h->sum_dnn, h->sum_logits, h->sum_limits, h->sum_stats, h->sum_buckets, h->d_metrics, h->metric_parts, h->up_partial, h->w0_partial, h->tc_w, h->head_gpart, h->d_slot_col, h->d_slot_j, h->d_field_slot0, h->inv_cnt, h->uidx,
                     h->req_rows, h->d_counts};
     for (void* p : ptrs) if (p) cudaFree(p);
     free_ws(h->ws);
@@ -2127,6 +2130,85 @@ extern "C" int dfm_forward(dfm_handle* h, const dfm_raw_batch* b, float* logits_
     return DFM_OK;
 }
 
+// ----------------------------------------------------------------- EVAL metrics (metrics.cuh)
+static_assert(sizeof(dfm_metric_state) == (1 + metrics::NI + metrics::ND) * 8, "dfm_metric_state is n, NI int64, ND float64");
+static_assert(offsetof(dfm_metric_state, bin_weight) == (1 + metrics::NI) * 8, "float64 fields follow the int64 fields");
+
+// the state is allocated, and zeroed, by the first metrics call on the handle
+static int metrics_ws(dfm_handle* h) {
+    if (h->d_metrics) return DFM_OK;
+    if (dalloc(h, &h->d_metrics, 1) || dalloc(h, &h->metric_parts, metrics::MAX_BLOCKS)) return DFM_ERR_CUDA;
+    CK(cudaMemset(h->d_metrics, 0, sizeof(dfm_metric_state)));
+    return DFM_OK;
+}
+
+static int metrics_launch(dfm_handle* h, const float* logits, const float* labels, const float* weights, int64_t n, cudaStream_t st) {
+    if (n == 0) return DFM_OK;
+    const int grid = (int)std::min<int64_t>((n + metrics::TILE - 1) / metrics::TILE, metrics::MAX_BLOCKS);
+    metrics::metrics_accumulate_kernel<<<grid, metrics::THREADS, 0, st>>>(logits, labels, h->weighted ? weights : nullptr, n,
+                                                                          h->squared ? 1 : 0, h->metric_parts);
+    metrics::metrics_reduce_kernel<<<1, metrics::REDUCE_THREADS, 0, st>>>(
+        h->metric_parts, grid, n, reinterpret_cast<long long*>(h->d_metrics), &h->d_metrics->bin_weight[0][0]);
+    h->launches += 2;
+    CK(cudaGetLastError());
+    return DFM_OK;
+}
+
+static int check_eval_batch(dfm_handle* h, const dfm_raw_batch* b) {
+    if (h->world > 1) FAIL(DFM_ERR_UNSUPPORTED, "row-sharded handle: accumulate the dfm_shard_forward / dfm_xchg_forward logits with dfm_metrics_accumulate");
+    if (b && !b->labels) FAIL(DFM_ERR_INVALID_ARG, "labels are required for an evaluation");
+    if (b && h->weighted && !b->weights) FAIL(DFM_ERR_INVALID_ARG, "weights are required for an evaluation of a weighted model");
+    return check_batch(h, b, false);
+}
+
+extern "C" int dfm_metrics_reset(dfm_handle* h, void* stream) {
+    if (!h) return DFM_ERR_INVALID_ARG;
+    CK(cudaSetDevice(h->device));
+    int rc = metrics_ws(h);
+    if (rc) return rc;
+    CK(cudaMemsetAsync(h->d_metrics, 0, sizeof(dfm_metric_state), stream ? (cudaStream_t)stream : h->stream));
+    return DFM_OK;
+}
+
+extern "C" int dfm_metrics_accumulate(dfm_handle* h, const float* logits, const float* labels, const float* weights, int64_t n,
+                                      void* stream) {
+    if (!h) return DFM_ERR_INVALID_ARG;
+    if (n < 0) FAIL(DFM_ERR_INVALID_ARG, "n < 0");
+    if (n > 0 && (!logits || !labels)) FAIL(DFM_ERR_INVALID_ARG, "logits and labels are required");
+    if (n > 0 && h->weighted && !weights) FAIL(DFM_ERR_INVALID_ARG, "weights are required for an evaluation of a weighted model");
+    CK(cudaSetDevice(h->device));
+    int rc = metrics_ws(h);
+    if (rc) return rc;
+    return metrics_launch(h, logits, labels, weights, n, stream ? (cudaStream_t)stream : h->stream);
+}
+
+extern "C" int dfm_evaluate(dfm_handle* h, const dfm_raw_batch* b, void* stream) {
+    if (!h) return DFM_ERR_INVALID_ARG;
+    int rc = check_eval_batch(h, b);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    if ((rc = metrics_ws(h))) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    BatchPtrs bp = make_ptrs(h, b);
+    bp.labels = nullptr; bp.weights = nullptr;
+    if ((rc = ensure_alpha(h, h->step))) return rc;
+    launch_transform<4>(h, bp, b->batch_size, false, h->ids, st);
+    DISPATCH_K(h, rc = eval_forward<KK>(h, bp, b->batch_size, nullptr, nullptr, st));      // logits -> h->logits
+    if (rc) return rc;
+    return metrics_launch(h, h->logits, b->labels, b->weights, b->batch_size, st);
+}
+
+extern "C" int dfm_metrics_read(dfm_handle* h, dfm_metric_state* out, void* stream) {
+    if (!h || !out) return DFM_ERR_INVALID_ARG;
+    CK(cudaSetDevice(h->device));
+    int rc = metrics_ws(h);
+    if (rc) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    CK(cudaMemcpyAsync(out, h->d_metrics, sizeof(dfm_metric_state), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return DFM_OK;
+}
+
 // ---- layer_summary side outputs (summary.cuh; trainers/model_utils.py:4-6 and its call sites in trainers/deep_fm.py)
 static std::vector<double> summary_limits() {      // core/lib/histogram/histogram.cc InitDefaultBucketsInner
     std::vector<double> pos, out;
@@ -2976,6 +3058,33 @@ extern "C" int dfm_forward_host(dfm_handle* h, const dfm_raw_batch* b, float* lo
     CK(cudaMemcpyAsync(logits_out, h->logits, (size_t)b->batch_size * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
+    return DFM_OK;
+}
+
+extern "C" int dfm_evaluate_host(dfm_handle* h, const dfm_raw_batch* b) {
+    if (!h) return DFM_ERR_INVALID_ARG;
+    int rc = check_eval_batch(h, b);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    if ((rc = metrics_ws(h))) return rc;
+    HostStage& sg = h->stage[0];
+    if (sg.busy) { CK(cudaEventSynchronize(sg.done)); sg.busy = false; }
+    CK(cudaStreamSynchronize(h->stream));
+    BatchPtrs bp;
+    rc = stage_batch(h, b, sg, true, bp, nullptr);          // labels (and weights) staged with the columns
+    if (rc) return rc;
+    CK(cudaEventRecord(sg.copied, h->copy_stream));
+    CK(cudaStreamWaitEvent(h->stream, sg.copied, 0));
+    rc = ensure_alpha(h, h->step);
+    if (rc) return rc;
+    const float* labels = bp.labels;
+    const float* weights = bp.weights;
+    bp.labels = nullptr; bp.weights = nullptr;
+    launch_transform<4>(h, bp, b->batch_size, false, h->ids, h->stream);
+    DISPATCH_K(h, rc = eval_forward<KK>(h, bp, b->batch_size, nullptr, nullptr, h->stream));
+    if (rc) return rc;
+    if ((rc = metrics_launch(h, h->logits, labels, weights, b->batch_size, h->stream))) return rc;
+    CK(cudaStreamSynchronize(h->stream));        // the host buffers may be reused as soon as this returns
     return DFM_OK;
 }
 

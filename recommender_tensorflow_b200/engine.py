@@ -628,6 +628,45 @@ class DeepFMEngine:
         self._check(self.lib.dfm_forward_host(self.h, C.byref(pb.raw), out.ctypes.data_as(C.c_void_p)))
         return out
 
+    # ------------------------------------------------------------------ EVAL metrics streamed on the device
+    def metrics_reset(self, stream=None):
+        """zero this handle's metric state"""
+        self._check(self.lib.dfm_metrics_reset(self.h, C.c_void_p(stream) if stream else None))
+
+    def evaluate_batch(self, features, labels=None, weights=None, stream=None):
+        """Add one EVAL batch to the metric state: the forward pass and the accumulation run on the device, nothing is
+        copied back.  A device PackedBatch carries its labels (and weights) and goes through dfm_evaluate, which only
+        enqueues; the next decode into the same reader buffers must be ordered after it on the stream (GpuCsvReader's
+        decode / decode_lines synchronise the engine first unless given a stream).  Host features are packed with
+        labels / weights and go through dfm_evaluate_host."""
+        pb = features if isinstance(features, PackedBatch) else self.pack(features, labels, weights=weights)
+        if pb.on_device:
+            self._check(self.lib.dfm_evaluate(self.h, C.byref(pb.raw), C.c_void_p(stream) if stream else None))
+        else:
+            self._check(self.lib.dfm_evaluate_host(self.h, C.byref(pb.raw)))
+
+    def metrics_accumulate(self, logits, labels, weights=None, stream=None):
+        """Add a batch whose logits were already computed on the device, e.g. by a row-sharded forward pass.  logits,
+        labels, weights: cuda float32 tensors [B] or raw device pointers (labels / weights of a device PackedBatch are
+        pb.raw.labels / pb.raw.weights); weights are read on a weighted engine only, and required there."""
+        def ptr(x):
+            return C.c_void_p(x.data_ptr() if hasattr(x, "data_ptr") else x) if x is not None else None
+        self._check(self.lib.dfm_metrics_accumulate(self.h, ptr(logits), ptr(labels), ptr(weights), int(logits.numel()),
+                                                    C.c_void_p(stream) if stream else None))
+
+    def metrics_state(self, stream=None):
+        """The raw metric state as numpy arrays (see trainers/model_utils.py: combine_metric_states, finish_metrics);
+        synchronises the stream, then reports any sticky device error of the evaluated batches."""
+        st = _lib.MetricState()
+        self._check(self.lib.dfm_metrics_read(self.h, C.byref(st), C.c_void_p(stream) if stream else None))
+        self.sync()
+        return {"head": self.head, "weighted": self.weighted, "n": np.int64(st.n),
+                "bin_count": np.ctypeslib.as_array(st.bin_count).copy(),
+                "cls": np.array([st.tp, st.fp, st.fn, st.correct], dtype=np.int64),
+                "bin_weight": np.ctypeslib.as_array(st.bin_weight).copy(),
+                "w_cls": np.array([st.w_tp, st.w_fp, st.w_fn, st.w_correct], dtype=np.float64),
+                "sums": np.array([st.sum_w, st.sum_wy, st.sum_wpred, st.sum_wloss], dtype=np.float64)}
+
     # ------------------------------------------------------------------ layer_summary side outputs
     def summary_names(self):
         """TF name scopes of the tensors trainers/deep_fm.py passes to layer_summary, in the library's order."""

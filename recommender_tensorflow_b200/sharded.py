@@ -19,6 +19,42 @@ co-running kernels that wait on each other).
 import numpy as np
 
 
+def _metric_arrays(state):
+    """a metric state as one int64 and one float64 vector (what the ranks all-gather)"""
+    ints = np.concatenate([[state["n"]], np.ravel(state["bin_count"]), state["cls"]]).astype(np.int64)
+    return ints, np.concatenate([np.ravel(state["bin_weight"]), state["w_cls"], state["sums"]]).astype(np.float64)
+
+
+def _metric_state(ints, floats, head, weighted):
+    nb = (ints.size - 5) // 2
+    return {"head": head, "weighted": weighted, "n": np.int64(ints[0]), "bin_count": ints[1:1 + 2 * nb].reshape(2, nb),
+            "cls": ints[1 + 2 * nb:], "bin_weight": floats[:2 * nb].reshape(2, nb), "w_cls": floats[2 * nb:2 * nb + 4],
+            "sums": floats[2 * nb + 4:]}
+
+
+def _evaluate_collective(trainer, batches, steps):
+    """EVAL on one rank of a process group: each local device batch (labels and weights inside) runs the trainer's
+    predict_logits, whose logits are accumulated on the device (dfm_metrics_accumulate); the ranks' metric states are
+    then all-gathered and combined in rank order, so every rank returns the same dict.  Every rank must pass the same
+    number of batches (the forward passes exchange rows)."""
+    from .trainers.model_utils import combine_metric_states, finish_metrics
+    torch, dist, eng = trainer.torch, trainer.dist, trainer.eng
+    st = torch.cuda.current_stream().cuda_stream
+    eng.metrics_reset(st)
+    for n, pb in enumerate(batches):
+        if steps is not None and n >= steps:
+            break
+        eng.metrics_accumulate(trainer.predict_logits(pb), pb.raw.labels, pb.raw.weights, st)
+    dev = "cuda:%d" % eng.device
+    ints, floats = (torch.from_numpy(a).to(dev) for a in _metric_arrays(eng.metrics_state(st)))
+    all_i = torch.empty((trainer.W, ints.numel()), dtype=torch.int64, device=dev)
+    all_f = torch.empty((trainer.W, floats.numel()), dtype=torch.float64, device=dev)
+    dist.all_gather_into_tensor(all_i, ints, group=trainer.group)
+    dist.all_gather_into_tensor(all_f, floats, group=trainer.group)
+    all_i, all_f = all_i.cpu().numpy(), all_f.cpu().numpy()
+    return finish_metrics(combine_metric_states(_metric_state(all_i[r], all_f[r], eng.head, eng.weighted) for r in range(trainer.W)))
+
+
 def split_sizes(counts, width=1):
     return [int(c) * width for c in counts]
 
@@ -151,6 +187,12 @@ class ShardedTrainer:
         eng.shard_forward(pb, self.rowbuf, logits, st)
         return logits
 
+    @_on_real_stream
+    def evaluate(self, batches, steps=None):
+        """EVAL metrics of the head over this rank's device batches, combined over all ranks (the same dict on every
+        rank).  steps: stop after that many batches."""
+        return _evaluate_collective(self, batches, steps)
+
 
 class XchgTrainer:
     """One process per GPU.  The exchanges are fused into the kernels: every rank's exchange region (fixed-capacity id /
@@ -218,6 +260,12 @@ class XchgTrainer:
         eng.xchg_serve(False, st)
         eng.xchg_forward(pb, logits, st)
         return logits
+
+    @_on_real_stream
+    def evaluate(self, batches, steps=None):
+        """EVAL metrics of the head over this rank's device batches, combined over all ranks with one all_gather at the
+        end (the same dict on every rank).  steps: stop after that many batches."""
+        return _evaluate_collective(self, batches, steps)
 
 
 class VirtualCluster:
@@ -315,6 +363,24 @@ class VirtualCluster:
 
     def predict_logits(self, pbs):
         """EVAL / PREDICT: logits of all ranks' batches, concatenated in rank order (numpy)."""
+        return self.torch.cat(self._rank_logits(pbs)).cpu().numpy()
+
+    def evaluate(self, batches, steps=None):
+        """EVAL metrics of the head: batches yields one list of device PackedBatches (labels and weights inside) per
+        step, one per rank.  Each rank accumulates its logits on the device (dfm_metrics_accumulate); the states are
+        combined in rank order on the host.  steps: stop after that many steps."""
+        from .trainers.model_utils import combine_metric_states, finish_metrics
+        for e in self.engs:
+            e.metrics_reset()
+        for n, pbs in enumerate(batches):
+            if steps is not None and n >= steps:
+                break
+            for e, pb, lg in zip(self.engs, pbs, self._rank_logits(pbs)):
+                e.metrics_accumulate(lg, pb.raw.labels, pb.raw.weights)
+        return finish_metrics(combine_metric_states(e.metrics_state() for e in self.engs))
+
+    def _rank_logits(self, pbs):
+        """logits of each rank's batch: cuda tensors, computed and synchronised"""
         torch = self.torch
         dev = "cuda:%d" % self.engs[0].device
         rw = self.engs[0].row_width
@@ -353,7 +419,7 @@ class VirtualCluster:
                 e.shard_forward(pb, rbc, lg)
                 e.sync()
                 outs.append(lg)
-        return torch.cat(outs).cpu().numpy()
+        return outs
 
     def state(self, names_with_slots):
         """Global arrays reassembled from the shards (dense variables from rank 0)."""

@@ -16,7 +16,7 @@ import numpy as np
 from ..engine import DeepFMEngine, PackedBatch
 from .ml_100k import FEATURE_DTYPES, ModeKeys, get_feature_columns, get_input_fn
 from .model_utils import (check_regression_head, get_binary_metrics, get_binary_predictions, get_optimizer,
-                          get_regression_metrics, get_regression_predictions, get_weights, weight_column_key)
+                          get_regression_metrics, get_regression_predictions, get_weights, weight_column_key, finish_metrics)
 
 EstimatorSpec = namedtuple("EstimatorSpec", ["mode", "loss", "train_op", "predictions", "eval_metric_ops", "global_step"])
 _ENGINE_KEY = "_b200_engine"
@@ -204,6 +204,32 @@ class Estimator:
         if not ys:
             raise ValueError("evaluate(): input_fn yielded no batches")
         m = eval_metrics(np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
+        m["global_step"] = self.engine.global_step
+        return m
+
+    def evaluate_streaming(self, input_fn, steps=None):
+        """evaluate() with the metrics streamed on the device (DESIGN.md §8.6): every batch's forward pass and metric
+        accumulation run on the GPU, nothing per example is copied back or kept on the host.  Same metric names plus
+        global_step; the AUCs use TF's float32 predictions and thresholds, so they can differ from evaluate()'s float64
+        ones for predictions at a threshold.  steps: stop after that many batches.  With get_gpu_input_fn(...,
+        device_labels=True) the labels and weights stay on the device."""
+        weight_column = self.params.get("weight_column")
+        _head(self.params)
+        n = 0
+        for feats, labels in input_fn():
+            if steps is not None and n >= steps:
+                break
+            if self.engine is None:
+                self.params[_ENGINE_KEY] = _build_engine(self.params, _batch_size(feats))
+            self._maybe_restore()
+            if n == 0:
+                self.engine.metrics_reset()
+            weights = None if isinstance(feats, PackedBatch) else get_weights(feats, weight_column, _batch_size(feats))
+            self.engine.evaluate_batch(feats, labels, weights)
+            n += 1
+        if not n:
+            raise ValueError("evaluate_streaming(): input_fn yielded no batches")
+        m = finish_metrics(self.engine.metrics_state())
         m["global_step"] = self.engine.global_step
         return m
 

@@ -10,7 +10,7 @@ import numpy as np
 
 from ..engine import DeepFMEngine, PackedBatch, default_optimizer
 from .ml_100k import FEATURE_DTYPES, ModeKeys
-from .model_utils import (check_regression_head, get_binary_metrics, get_binary_predictions, get_regression_metrics,
+from .model_utils import (check_regression_head, finish_metrics, get_binary_metrics, get_binary_predictions, get_regression_metrics,
                           get_regression_predictions, get_weights, weight_column_key)
 
 _DNN_LEARNING_RATE = 0.001
@@ -95,6 +95,23 @@ class _CannedBase:
             if self.weight_column is not None:
                 ws.append(self._weights(feats, zs[-1].shape[0]))
         m = self._head_fns()[1](np.concatenate(ys), np.concatenate(zs), np.concatenate(ws) if ws else None)
+        m["global_step"] = self.engine.global_step
+        return m
+
+    def evaluate_streaming(self, input_fn, steps=None):
+        """evaluate() with the metrics streamed on the device (DESIGN.md §8.6): same metric names plus global_step; the
+        AUCs use TF's float32 predictions and thresholds.  steps: stop after that many batches."""
+        self._maybe_restore()
+        self.engine.metrics_reset()
+        n = 0
+        for feats, labels in input_fn():
+            if steps is not None and n >= steps:
+                break
+            self.engine.evaluate_batch(feats, labels, self._weights(feats))
+            n += 1
+        if not n:
+            raise ValueError("evaluate_streaming(): input_fn yielded no batches")
+        m = finish_metrics(self.engine.metrics_state())
         m["global_step"] = self.engine.global_step
         return m
 

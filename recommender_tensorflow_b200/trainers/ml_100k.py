@@ -157,7 +157,8 @@ def _train_index_stream(n_rows, cap, rng):
         yield from buf
 
 
-def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutoff=5, seed=None, weight_column=None):
+def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutoff=5, seed=None, weight_column=None,
+                     device_labels=False):
     """get_input_fn with tf.decode_csv moved to the GPU (SURVEY.md §8f rank 2): the host only selects whole records
     (same shuffle algorithm and RNG stream as get_input_fn, so the same seed gives the same batches); the file itself
     is uploaded once and stays in HBM, a batch travels as 4 bytes per record (its line number); `GpuCsvReader` splits,
@@ -166,7 +167,8 @@ def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutof
     float32 labels are read back for the metrics.  A record is one text line, as with tf.data.TextLineDataset (a
     quoted field cannot contain a line break).  weight_column (a field key or numeric_column of a weighted engine): the
     batches carry that field as their per-example weights; outside TRAIN its host copy is the batch's `weights`
-    attribute, for the weighted metrics."""
+    attribute, for the weighted metrics.  device_labels=True: yield (PackedBatch, None) in every mode, with nothing read
+    back - for evaluate_streaming, which takes the labels and weights from the batch on the device."""
     from ..csv_reader import GpuCsvReader
     from .model_utils import weight_column_key
     wkey = weight_column_key(weight_column)
@@ -185,7 +187,7 @@ def get_gpu_input_fn(csv_path, engine, mode=ModeKeys.TRAIN, batch_size=32, cutof
 
         def emit(idx):
             pb = reader.decode_lines(np.asarray(idx, dtype=np.int32) + 1)    # +1: line 0 is the header
-            if mode == ModeKeys.TRAIN:
+            if mode == ModeKeys.TRAIN or device_labels:
                 return pb, None
             if wkey is not None:
                 pb.weights = reader.weights()
